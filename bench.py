@@ -8,6 +8,7 @@
   --trainable-emb               textual_embedding_trainable (conv input gradient + word-table scatter; F_train = 3 x fwd)
   --scaling weak|strong         weak: B rows per rank (default); strong: the workload's B split over the ranks
   --no-extras                   skip the sub-records (drop-in protocol timing, per-kernel probes, C2, C4)
+  --dump-outputs DIR            write what the last timed step computed as DIR/<name>.npy (rank 0; see dump_outputs)
 
 A "step" is one LSTUR training step (forward + backward + Keras-Adam) over one batch of B
 impressions per rank; value = impressions/s over all ranks.
@@ -146,6 +147,42 @@ def timed_ms(torch, fn):
     e1.record()
     torch.cuda.synchronize()
     return r, e0.elapsed_time(e1)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_WORD_ROWS = 8192
+
+
+def last_step_outputs(torch, eng, batch):
+    """What a caller of the timed train step holds after its last step, copied to the host: the loss it returned, the
+    probabilities of its forward, every dense weight after the Adam update, and the rows of the embedding tables the step
+    updated (the batch's users; with a trainable word table, a seeded sample of the batch's tokens).  The tables themselves
+    (up to 1M x 200 floats) are too large to write whole."""
+    rows = lambda table, ids: table[torch.as_tensor(ids, dtype=torch.int64, device=eng.device)].cpu().numpy()
+    out = dict(loss=eng.view('loss').cpu().numpy().copy(), probs=eng.view('probs').reshape(eng.B, eng.C).cpu().numpy().copy())
+    out.update(('weight_' + k, v) for k, v in eng._unflatten(eng.dense).items())
+    if eng.user_emb is not None:
+        users = np.unique(batch['user'])
+        out['user_emb_row_ids'] = users.astype(np.float64)
+        out['user_emb_rows'] = rows(eng.user_emb, users)
+    if eng.trainable_word_emb:
+        tokens = np.unique(rows(eng.doc_tokens, np.concatenate([batch['hist_doc'].ravel(), batch['cand_doc'].ravel()])))
+        if tokens.size > DUMP_WORD_ROWS:
+            tokens = np.sort(np.random.default_rng(0).choice(tokens, DUMP_WORD_ROWS, replace=False))
+        out['word_emb_row_ids'] = tokens.astype(np.float64)
+        out['word_emb_rows'] = rows(eng.word_emb, tokens)
+    return out
+
+
+def dump_outputs(dirname, arrays):
+    """DIR/<name>.npy for every array, float32 or float64, at most DUMP_LIMIT_BYTES in all."""
+    arrays = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError('--dump-outputs: %d bytes exceed the %d byte limit' % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(dirname, k + '.npy'), v)
 
 
 def extra_records(torch, lib, sh, eng, dbs, batches, tok, P, precision, pk, args, B, live_frac=1.0):
@@ -303,7 +340,14 @@ def main():
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-extras', action='store_true')
     ap.add_argument('--cpu-sample', type=int, default=64)
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the loss, probabilities, updated weights and updated table rows of the last timed step '
+                         'as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes what the CUDA path computed (--impl ours)')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
 
     from mnexp_b200 import synth
@@ -393,6 +437,8 @@ def main():
     value = B * world * args.steps / (ms_total / 1e3)
     probe_ms = float(np.mean([eng.elapsed_ms(a, b) for a, b in probes]))
     loss_last = eng.loss()
+    # taken before the e2e and extra passes below train the engine further
+    outputs = last_step_outputs(torch, eng, batches[(args.steps - 1) % n_batches]) if args.dump_outputs and rank == 0 else None
 
     # ---- e2e: host (pinned) batches in, loss out, every step
     e2e = None
@@ -461,6 +507,8 @@ def main():
                             user_adam='row-sparse (documented deviation from dense Keras-Adam)', hist_pad_frac=round(pad_frac, 3)),
                 roofline=roofline, cpu_baseline=cpu, e2e=e2e, gpu_launches=launches, clocks=clocks, loss=loss_last,
                 host_enqueue_ms_per_step=host_enqueue_ms, extra=extra)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line))
     if world > 1:
         dist.barrier()
