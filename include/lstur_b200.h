@@ -96,15 +96,11 @@ int lstur_token_gather(int N, int L, int n_docs, const int* doc_tokens, const in
 int lstur_embed_gather_pad(int N, int L, int E, int V, int KS, const float* word_emb, const int* tokens, float* Xp,
                            float dropout, unsigned seed, cudaStream_t stream);
 
-int lstur_embed_gather_pad_tcrng(int N, int L, int E, int V, int KS, int Ep, const float* word_emb, const int* tokens,
-                                 float* Xp, float dropout, unsigned seed, cudaStream_t stream);
-
 /* Tensor-core news encoder (tcgen05/TMEM): Embedding + Dropout + Conv1D(F,3,'same',relu) + pad mask + Masking +
  * Dropout + SimpleAttentionMaskSupport in ONE kernel (task/paper.py:141-158, models.py:474-489).
  * emb_16: (V, lstur_tc_padded_e(E)) 16-bit table from lstur_pack_word_emb_16; wimg: lstur_tc_wimg_elems(E,F)
  * 16-bit elements from lstur_pack_conv_w_tc.  c_out_16 (n_titles,L,F) receives the attention input (saved for
  * backward).  fp16 != 0: IEEE half operands (10-bit mantissa, meets the 1e-3 parity bound); 0: bfloat16. */
-int lstur_conv_tc_available(void);
 int lstur_tc_set_trace(void* dev_buf);   /* profiling hook: clock64 stamps of CTA 0's warp roles; NULL disables */
 int lstur_tc_supported(int L, int E, int F, int KS);
 int lstur_tc_slot(int L);                /* rows of a title slot in the tensor-core kernels: 32 (L <= 31) or 64 (L <= 63) */
@@ -198,11 +194,6 @@ int lstur_attn_pool_bwd(int N, int L, int Lrows, int F, const float* Cd, long lo
                         const float* w_in, const float* d_pooled, long long lddp, const float* att_w, float* dPre,
                         long long dpre_title_stride, float dropout, float* d_att_w, float* d_conv_b, float* d_att_b,
                         int accumulate, float* partials, size_t partial_bytes, cudaStream_t stream);
-int lstur_attn_pool_bwd_16(int fp16, int N, int L, int Lrows, int F, const void* Cd_16, long long title_stride,
-                             const float* a_in, const float* w_in, const float* d_pooled, long long lddp,
-                             const float* att_w, float* dPre, long long dpre_title_stride, float dropout,
-                             float* d_att_w, float* d_conv_b, float* d_att_b, int accumulate, float* partials,
-                             size_t partial_bytes, cudaStream_t stream);
 int lstur_colsum(long long rows, int cols, const float* in, long long ld, float* out, int accumulate,
                  float* workspace, size_t workspace_bytes, cudaStream_t stream);
 
@@ -214,14 +205,15 @@ int lstur_hist_mask_apply(int rows, int L, int D, const int* tokens, float* H, l
 int lstur_row_gather(int B, int D, int n_rows, const float* table, const int* ids, const float* scale, float* out,
                      long long ldo, cudaStream_t stream);
 
-/* keras GRU recurrence (task/paper.py:596-613); XW = H.Wx + b is a GEMM done by the caller. */
+/* keras GRU recurrence (task/paper.py:596-613); XW = H.Wx + b is a GEMM done by the caller.  lstur_gru_fwd/bwd run the
+ * cluster kernels when lstur_gru_cluster_supported(), else the streaming kernels, which ignore row_order. */
 int lstur_transpose(int rows, int cols, const float* in, float* out, cudaStream_t stream);
 int lstur_gru_fwd(int B, int W, int G, const float* XW, const float* gm, const float* h0, long long ldh0,
                   const float* Wh, int rec_act, float* hT, long long ldo, float* Z, float* R, float* HH, float* HP,
-                  float* RH, cudaStream_t stream);
+                  float* RH, const int* row_order, cudaStream_t stream);
 int lstur_gru_bwd(int B, int W, int G, const float* gm, const float* Z, const float* R, const float* HH,
                   const float* HP, const float* WhT, int rec_act, const float* dhT, long long lddh, float* dA,
-                  float* dh0, long long lddh0, cudaStream_t stream);
+                  float* dh0, long long lddh0, const int* row_order, cudaStream_t stream);
 /* The two implementations behind lstur_gru_fwd/bwd.  _cluster: recurrent weights resident in the shared memory of a
  * thread-block cluster for the whole launch, state exchanged through distributed shared memory (gru_cl.cu);
  * row_order (B) optionally permutes the batch rows inside the kernel (length-sorted tiles skip padded steps) or NULL.

@@ -8,8 +8,6 @@
 // carries the same arithmetic in its epilogue.
 #include <cuda_fp16.h>
 
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace lstur {
@@ -65,27 +63,11 @@ attn_pool_fwd_kernel(int N, int L, int F, float* __restrict__ C, long long title
 // Backward of the block above.  Grid-strided over titles; each CTA keeps
 // per-thread partial sums of d(ka), d(conv bias) and d(ba) and writes them to
 // partials[cta][2F+1] (reduced afterwards in a fixed order -> deterministic).
-//   dPre = d(loss)/d(conv pre-activation) incl. ReLU/pad/Masking/Dropout gates.
-__device__ __forceinline__ float ldc(const float* p, long long i) { return p[i]; }
-__device__ __forceinline__ float ldc(const __nv_bfloat16* p, long long i) { return __bfloat162float(p[i]); }
-__device__ __forceinline__ float ldc(const __half* p, long long i) { return __half2float(p[i]); }
-
-// OUT = 0: dPre as fp32 rows (title stride dpre_title_stride, rows L..Lrows-1 zeroed).
-// OUT = 1/2: dPre as bf16/fp16 K-block images for the tensor-core wgrad (conv_tc.cu): one block per 32-row title
-//   slot n, [half h = f / (F/2)][64-column group g][32 rows][128 B]; with fl = f - h*F/2 the element lives at
-//   ((h*ngh + fl/64)*4096 + t*128 + ((((fl%64)/8) ^ (t%8)) << 4) + (fl%8)*2  — MN-major SWIZZLE_128B, one half per CTA of
-//   the wgrad's CTA pair.  ngh = ceil(F/2/64).
-__device__ __forceinline__ void store_dpre_img(void* img, int out_mode, int ngh, int Fh, int n, int t, int f, float v) {
-  const int h = f >= Fh ? 1 : 0, fl = f - h * Fh;
-  const long long byte = (long long)n * ((long long)2 * ngh * 4096) + (long long)(h * ngh + (fl >> 6)) * 4096 + t * 128 +
-                         ((((fl & 63) >> 3) ^ (t & 7)) << 4) + (fl & 7) * 2;
-  if (out_mode == 2) *reinterpret_cast<__half*>((char*)img + byte) = __float2half_rn(fminf(fmaxf(v, -65504.f), 65504.f));
-  else *reinterpret_cast<__nv_bfloat16*>((char*)img + byte) = __float2bfloat16_rn(v);
-}
-
-template <int FPT, typename CT, int OUT>
+//   dPre = d(loss)/d(conv pre-activation) incl. ReLU/pad/Masking/Dropout gates, as fp32 rows (title stride
+//   dpre_title_stride, rows L..Lrows-1 zeroed).
+template <int FPT>
 __global__ void __launch_bounds__(ATT_THREADS)
-attn_pool_bwd_kernel(int N, int L, int Lrows, int F, const CT* __restrict__ Cd, long long title_stride,
+attn_pool_bwd_kernel(int N, int L, int Lrows, int F, const float* __restrict__ Cd, long long title_stride,
                      const float* __restrict__ a_in, const float* __restrict__ w_in, const float* __restrict__ dp,
                      long long lddp, const float* __restrict__ ka, float* __restrict__ dPre,
                      long long dpre_title_stride, float inv_keep, float* __restrict__ partials) {
@@ -95,12 +77,12 @@ attn_pool_bwd_kernel(int N, int L, int Lrows, int F, const CT* __restrict__ Cd, 
 #pragma unroll
   for (int i = 0; i < FPT; ++i) dka[i] = dbc[i] = 0.f;
   for (int n = blockIdx.x; n < N; n += gridDim.x) {
-    const CT* Cn = Cd + (long long)n * title_stride;
+    const float* Cn = Cd + (long long)n * title_stride;
     const float* dpn = dp + (long long)n * lddp;
     float* dPn = dPre + (long long)n * dpre_title_stride;
     for (int t = warp; t < L; t += ATT_THREADS / 32) {
       float dot = 0.f;
-      for (int f = lane; f < F; f += 32) dot = fmaf(ldc(Cn, (long long)t * F + f), dpn[f], dot);
+      for (int f = lane; f < F; f += 32) dot = fmaf(Cn[(long long)t * F + f], dpn[f], dot);
       dot = warp_sum(dot);
       if (lane == 0) {
         sdw[t] = dot;
@@ -121,18 +103,14 @@ attn_pool_bwd_kernel(int N, int L, int Lrows, int F, const CT* __restrict__ Cd, 
       if (f < F) {
         const float dpf = dpn[f], kaf = ka[f];
         for (int t = 0; t < L; ++t) {
-          float c = ldc(Cn, (long long)t * F + f);
+          float c = Cn[(long long)t * F + f];
           float g = fmaf(sw[t], dpf, sdz[t] * kaf);
           float dpre = c > 0.f ? g * inv_keep : 0.f;
-          if (OUT == 0) dPn[(long long)t * F + f] = dpre;
-          else store_dpre_img(dPre, OUT, ((F >> 1) + 63) >> 6, F >> 1, n, t, f, dpre);
+          dPn[(long long)t * F + f] = dpre;
           dka[i] = fmaf(sdz[t], c, dka[i]);
           dbc[i] += dpre;
         }
-        for (int t = L; t < Lrows; ++t) {
-          if (OUT == 0) dPn[(long long)t * F + f] = 0.f;
-          else store_dpre_img(dPre, OUT, ((F >> 1) + 63) >> 6, F >> 1, n, t, f, 0.f);
-        }
+        for (int t = L; t < Lrows; ++t) dPn[(long long)t * F + f] = 0.f;
       }
     }
     if (tid == 0)
@@ -231,15 +209,19 @@ __device__ __forceinline__ uint4 pack8<__nv_bfloat16>(const float* v) {
 }
 
 constexpr int IMG_THREADS = 256;     // 64 chunk columns x 4 row groups
-// SLOT = rows of a title slot of the image (32 for L <= 31, 64 for L <= 63).  img_scale: power-of-two loss scale of the
-// 16-bit dPre values (gradients of a mean over a large global batch would otherwise sit in fp16's subnormal range);
-// the consumers (conv weight / input gradient) divide it out, and the d conv_b partial sums are unscaled on the way out.
+// SLOT = rows of a title slot of the image (32 for L <= 31, 64 for L <= 63).  The image holds one block per title slot n,
+// [half h = f / (F/2)][64-column group][SLOT rows][128 B]; with fl = f - h*F/2 the 16-bit element lives at byte
+//   n*2*ngh*SLOT*128 + (h*ngh + fl/64)*SLOT*128 + t*128 + ((((fl%64)/8) ^ (t%8)) << 4) + (fl%8)*2
+// (MN-major SWIZZLE_128B, one half per CTA of the weight gradient's CTA pair; ngh = ceil(F/2/64)).
+// img_scale: power-of-two loss scale of the 16-bit dPre values (gradients of a mean over a large global batch would
+// otherwise sit in fp16's subnormal range); the consumers (conv weight / input gradient) divide it out, and the d conv_b
+// partial sums are unscaled on the way out.
 template <typename CT, int SLOT>
 __global__ void __launch_bounds__(IMG_THREADS)
 attn_bwd_img_kernel(int N, int L, int F, const CT* __restrict__ Cd, const float* __restrict__ a_in,
                     const float* __restrict__ w_in, const float* __restrict__ dp, long long lddp,
                     const float* __restrict__ ka, uint8_t* __restrict__ img, float inv_keep, float img_scale,
-                    float* __restrict__ partials, int nbuf, const int* __restrict__ n_dev,
+                    float* __restrict__ partials, const int* __restrict__ n_dev,
                     const int* __restrict__ title_idx) {
   if (n_dev) N = min(N, __ldg(n_dev));          // compacted title list: live titles only (lstur_compact_titles)
   extern __shared__ __align__(16) uint8_t att_smem[];
@@ -247,9 +229,8 @@ attn_bwd_img_kernel(int N, int L, int F, const CT* __restrict__ Cd, const float*
   // Two title buffers: the (contiguous, L*F*2-byte) saved C of the NEXT title is fetched with one bulk copy while the
   // current one is processed; its d_pooled row and attention weights are prefetched into registers.
   const size_t buf_bytes = (size_t)SLOT * nchunk * 16;
-  // nbuf = 2: the next title is fetched while the current one is processed; nbuf = 1: one buffer, more CTAs per SM
-  float* sdp = reinterpret_cast<float*>(att_smem + nbuf * buf_bytes);   // [F]
-  float* ska = sdp + F;                                              // [F]
+  float* sdp = reinterpret_cast<float*>(att_smem + 2 * buf_bytes);   // [F]
+  float* ska = sdp + F;                                           // [F]
   float* sred = reinterpret_cast<float*>(att_smem);                  // [3][64][16] reduction scratch, after the title loop
   __shared__ float sdw[SLOT], sdz[SLOT], sw[SLOT];
   __shared__ __align__(8) unsigned long long s_bar[2];
@@ -301,15 +282,11 @@ attn_bwd_img_kernel(int N, int L, int F, const CT* __restrict__ Cd, const float*
   uint32_t phase[2] = {0, 0};
   int it = 0;
   for (int n = blockIdx.x; n < N; n += gridDim.x, ++it) {
-    const int b = nbuf == 2 ? (it & 1) : 0;
+    const int b = it & 1;
     const uint4* sC = reinterpret_cast<const uint4*>(att_smem + b * buf_bytes);  // [L][nchunk]
     __syncthreads();   // previous title fully consumed: its buffer, sdp and sw may be overwritten
     const int n_next = n + gridDim.x;
-    if (nbuf == 2) {
-      if (tid == 0 && n_next < N) fetch_title(n_next, b ^ 1);
-    } else if (it > 0) {
-      if (tid == 0) fetch_title(n, 0);
-    }
+    if (tid == 0 && n_next < N) fetch_title(n_next, b ^ 1);
 #pragma unroll
     for (int i = 0; i < DPR; ++i) {
       const int f = tid + i * IMG_THREADS;
@@ -491,24 +468,11 @@ extern "C" int lstur_attn_pool_fwd(int N, int L, int F, float* C, long long titl
   return LSTUR_OK;
 }
 
-// CTAs of the attention-backward kernels: 4 per SM (shared memory: two 25.6 KB title buffers + 3.2 KB per CTA at F=400;
-// the final reduction scratch aliases the title buffers)
-static int attn_bwd_nbuf() {
-  static int nbuf = 0;
-  if (!nbuf) {
-    const char* e = getenv("LSTUR_ATTN_NBUF");
-    nbuf = (e && atoi(e) == 1) ? 1 : 2;
-  }
-  return nbuf;
-}
+// CTAs of the attention-backward kernels: one per title, at most 4 per SM of a 148-SM B200 (shared memory: two 25.6 KB
+// title buffers + 3.2 KB per CTA at F=400; the final reduction scratch aliases the title buffers), and at least one
 extern "C" int lstur_attn_bwd_grid(int N) {
-  static int per_sm = 0;
-  if (!per_sm) {
-    const char* e = getenv("LSTUR_ATTN_CTAS_PER_SM");
-    per_sm = e ? atoi(e) : 4;
-    if (per_sm < 1 || per_sm > 16) per_sm = 4;
-  }
-  return N < 148 * per_sm ? (N > 0 ? N : 1) : 148 * per_sm;
+  constexpr int max_ctas = 148 * 4;
+  return N < max_ctas ? (N > 0 ? N : 1) : max_ctas;
 }
 
 extern "C" int lstur_colsum(long long rows, int cols, const float* in, long long ld, float* out, int accumulate,
@@ -530,11 +494,11 @@ extern "C" int lstur_colsum(long long rows, int cols, const float* in, long long
 
 // partials must hold lstur_attn_bwd_grid(N) * (2F+1) floats; after the call
 // d_att_w[F], d_conv_b[F], d_att_b[1] are written (or accumulated).
-static int attn_pool_bwd_impl(int c_is_bf16, int out_mode, int N, int L, int Lrows, int F, const void* Cd_, long long title_stride,
-                              const float* a_in, const float* w_in, const float* d_pooled, long long lddp,
-                              const float* att_w, float* dPre, long long dpre_title_stride, float dropout,
-                              float* d_att_w, float* d_conv_b, float* d_att_b, int accumulate, float* partials,
-                              size_t partial_bytes, cudaStream_t stream) {
+extern "C" int lstur_attn_pool_bwd(int N, int L, int Lrows, int F, const float* Cd, long long title_stride,
+                                   const float* a_in, const float* w_in, const float* d_pooled, long long lddp,
+                                   const float* att_w, float* dPre, long long dpre_title_stride, float dropout,
+                                   float* d_att_w, float* d_conv_b, float* d_att_b, int accumulate, float* partials,
+                                   size_t partial_bytes, cudaStream_t stream) {
   LSTUR_REQUIRE(N >= 0 && L > 0 && L <= ATT_MAX_L && Lrows >= L && F > 0 && F <= 8 * ATT_THREADS, "lstur_attn_pool_bwd");
   int grid = lstur_attn_bwd_grid(N);
   size_t need = (size_t)grid * (2 * F + 1) * sizeof(float);
@@ -549,50 +513,19 @@ static int attn_pool_bwd_impl(int c_is_bf16, int out_mode, int N, int L, int Lro
   }
   float inv_keep = 1.f / (1.f - dropout);
   int fpt = cdiv(F, ATT_THREADS);
-#define LAUNCH_T(FPT_, CT_, OUT_)                                                                                  \
-  attn_pool_bwd_kernel<FPT_, CT_, OUT_><<<grid, ATT_THREADS, 0, stream>>>(N, L, Lrows, F, (const CT_*)Cd_, title_stride, \
-                                                                          a_in, w_in, d_pooled, lddp, att_w, dPre,  \
-                                                                          dpre_title_stride, inv_keep, partials)
-#define LAUNCH(FPT_)                                              \
-  do {                                                            \
-    if (c_is_bf16 == 1 && out_mode == 0) LAUNCH_T(FPT_, __nv_bfloat16, 0); \
-    else if (c_is_bf16 == 2 && out_mode == 0) LAUNCH_T(FPT_, __half, 0);   \
-    else if (c_is_bf16 == 1) LAUNCH_T(FPT_, __nv_bfloat16, 1);    \
-    else if (c_is_bf16 == 2) LAUNCH_T(FPT_, __half, 2);           \
-    else LAUNCH_T(FPT_, float, 0);                                \
-  } while (0)
+#define LAUNCH(FPT_)                                                                                                  \
+  attn_pool_bwd_kernel<FPT_><<<grid, ATT_THREADS, 0, stream>>>(N, L, Lrows, F, Cd, title_stride, a_in, w_in, d_pooled, lddp, \
+                                                               att_w, dPre, dpre_title_stride, inv_keep, partials)
   if (fpt <= 1) LAUNCH(1);
   else if (fpt <= 2) LAUNCH(2);
   else if (fpt <= 4) LAUNCH(4);
   else LAUNCH(8);
 #undef LAUNCH
-#undef LAUNCH_T
   LSTUR_CHECK_LAUNCH("lstur_attn_pool_bwd");
   attn_bwd_reduce_kernel<<<cdiv(2 * F + 1, 32), 256, 0, stream>>>(grid, F, partials, d_att_w, d_conv_b, d_att_b,
                                                                      accumulate, 1.f);
   LSTUR_CHECK_LAUNCH("lstur_attn_pool_bwd(reduce)");
   return LSTUR_OK;
-}
-
-extern "C" int lstur_attn_pool_bwd(int N, int L, int Lrows, int F, const float* Cd, long long title_stride,
-                                   const float* a_in, const float* w_in, const float* d_pooled, long long lddp,
-                                   const float* att_w, float* dPre, long long dpre_title_stride, float dropout,
-                                   float* d_att_w, float* d_conv_b, float* d_att_b, int accumulate, float* partials,
-                                   size_t partial_bytes, cudaStream_t stream) {
-  return attn_pool_bwd_impl(0, 0, N, L, Lrows, F, Cd, title_stride, a_in, w_in, d_pooled, lddp, att_w, dPre,
-                            dpre_title_stride, dropout, d_att_w, d_conv_b, d_att_b, accumulate, partials, partial_bytes,
-                            stream);
-}
-
-// Same, with the attention input saved as 16-bit floats by the tensor-core forward (fp16 != 0: half, else bf16).
-extern "C" int lstur_attn_pool_bwd_16(int fp16, int N, int L, int Lrows, int F, const void* Cd_bf16, long long title_stride,
-                                        const float* a_in, const float* w_in, const float* d_pooled, long long lddp,
-                                        const float* att_w, float* dPre, long long dpre_title_stride, float dropout,
-                                        float* d_att_w, float* d_conv_b, float* d_att_b, int accumulate,
-                                        float* partials, size_t partial_bytes, cudaStream_t stream) {
-  return attn_pool_bwd_impl(fp16 ? 2 : 1, 0, N, L, Lrows, F, Cd_bf16, title_stride, a_in, w_in, d_pooled, lddp, att_w, dPre,
-                            dpre_title_stride, dropout, d_att_w, d_conv_b, d_att_b, accumulate, partials, partial_bytes,
-                            stream);
 }
 
 // Tensor-core backward: same arithmetic, dPre emitted as 16-bit K-block images for lstur_conv_wgrad_tc /
@@ -616,15 +549,14 @@ extern "C" int lstur_attn_pool_bwd_img(int fp16, int N, int L, int F, const void
     return LSTUR_OK;
   }
   const float inv_keep = 1.f / (1.f - dropout);
-  const int nbuf = attn_bwd_nbuf();
   const int slot = L <= 31 ? 32 : 64;
-  size_t smem = (size_t)nbuf * slot * (F / 8) * 16 + (size_t)2 * F * sizeof(float);
+  size_t smem = (size_t)2 * slot * (F / 8) * 16 + (size_t)2 * F * sizeof(float);   // two title buffers + d_pooled + att_w
   if (smem < (size_t)3 * 64 * 16 * sizeof(float)) smem = (size_t)3 * 64 * 16 * sizeof(float);   // the final reduction scratch aliases the title buffers
 #define IMG_LAUNCH(CT_, SLOT_)                                                                                          \
   do {                                                                                                                  \
     if (smem > 48 * 1024) cudaFuncSetAttribute(attn_bwd_img_kernel<CT_, SLOT_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
     attn_bwd_img_kernel<CT_, SLOT_><<<grid, IMG_THREADS, smem, stream>>>(N, L, F, (const CT_*)Cd_16, a_in, w_in, d_pooled, lddp, \
-                                                                         att_w, (uint8_t*)dpre_img, inv_keep, img_scale, partials, nbuf, \
+                                                                         att_w, (uint8_t*)dpre_img, inv_keep, img_scale, partials,       \
                                                                          n_titles_dev, title_idx);                       \
   } while (0)
   if (fp16 && slot == 32) IMG_LAUNCH(__half, 32);

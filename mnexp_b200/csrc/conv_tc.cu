@@ -132,9 +132,7 @@ struct FwdParams {
   uint32_t drop_addend;           // quad_addend(threshold)
   float inv_keep;
   uint32_t seed_x, seed_c;
-  int dbg;                        // experiments (LSTUR_FWD_DBG): 1 = epilogue only hands the accumulator back, 2 = producers do not
-                                  // store, 16 = producers neither load nor hash, 32 = the weight loader only signals
-  int nstages;                    // depth of the weight-stage ring (<= MAX_STAGES)
+  int nstages;                    // depth of the weight-stage ring (2 .. DEF_STAGES)
   long long* trace;               // optional: wait cycles of pair 0's MMA issuer (tools/perf_fwd.py)
   uint8_t* xmask;                 // optional (n_titles, L, Ep/8): keep bits of the X-dropout, one byte per 16-byte piece, so
                                   // the weight-gradient kernel need not replay the hash (bit j / 4+j: low / high half of word j)
@@ -153,8 +151,7 @@ struct FwdParams {
 // Shared memory: an A ring with one slot per 32-column chunk of the tile (EC slots of 9 KB, filled once per tile, read by
 // both feature passes) and a B ring of weight stages (this CTA's rows of one (pass, chunk): 3 taps x n0h x 64 B).
 constexpr int MAX_CHUNKS = 16;                // A slots / barrier slots
-constexpr int MAX_STAGES = 8;                 // B stages / barrier slots; the launcher picks the depth (FwdParams::nstages)
-constexpr int DEF_STAGES = 3;
+constexpr int DEF_STAGES = 3;                 // B stages (<= 8 barrier slots); fewer where shared memory runs out
 // rows per CTA of feature pass 0 (pass 1 takes the other Fh - n0h): half of Fh rounded up to a multiple of 8, at most 128
 __host__ __device__ constexpr int conv_n0h(int Fh) { return ((Fh + 15) / 16) * 8 > 128 ? 128 : ((Fh + 15) / 16) * 8; }
 
@@ -163,7 +160,6 @@ struct EpiCtx {
   const float* s_bias;            // conv bias x conv-dropout keep scale (ReLU is positively homogeneous)
   const float* s_ka;
   uint32_t thr, base_lo, inner0, inner1;   // conv-dropout stream of this thread's token row (thr = quad_addend)
-  int dbg;
 };
 
 // Epilogue pass 1 for NC accumulator columns of one token row -> features [f0, f0+NC): scale + bias + ReLU (+ pad-token
@@ -264,7 +260,7 @@ __device__ __forceinline__ void epi_pass1_chunk(const EpiCtx& ec, const RowIO& i
       z = fmaf(hi16<FP16>(p1), k4.w, z);
     }
   }
-  if (!(ec.dbg & 8)) io.store(packed, f0, NC / 8);
+  io.store(packed, f0, NC / 8);
 }
 // Input-gradient epilogue for NC accumulator columns of one token row: scale, round to 16 bits (saturating), store.
 template <bool FP16, int NC>
@@ -406,15 +402,11 @@ __global__ void __launch_bounds__(THREADS, 1) news_conv_tc_kernel(const FwdParam
           const size_t row0 = (size_t)crank * Fh + (fp ? n0h : 0);
           for (int c = 0; c < EC; ++c) {
             mbar_wait(bar_b_empty + 8 * s, ph ^ 1, 1);
-            if (p.dbg & 32) {
-              mbar_arrive(bar_b_full + 8 * s);
-            } else {
-              mbar_expect_tx(bar_b_full + 8 * s, TAPS * rows_bytes);
+            mbar_expect_tx(bar_b_full + 8 * s, TAPS * rows_bytes);
 #pragma unroll
-              for (int j = 0; j < TAPS; ++j)
-                bulk_g2s(b_base + s * b_stage_bytes + j * b_tap_bytes,
-                         (const uint8_t*)p.wimg + ((size_t)(c * TAPS + j) * F + row0) * ROWB, rows_bytes, bar_b_full + 8 * s);
-            }
+            for (int j = 0; j < TAPS; ++j)
+              bulk_g2s(b_base + s * b_stage_bytes + j * b_tap_bytes,
+                       (const uint8_t*)p.wimg + ((size_t)(c * TAPS + j) * F + row0) * ROWB, rows_bytes, bar_b_full + 8 * s);
             if (++s == NB) { s = 0; ph ^= 1; }
           }
         }
@@ -513,7 +505,7 @@ __global__ void __launch_bounds__(THREADS, 1) news_conv_tc_kernel(const FwdParam
 #pragma unroll
       for (int i = 0; i < 2; ++i) {
         v[i] = make_uint4(0, 0, 0, 0);
-        if (ids[i] != kNoToken && !(p.dbg & 16)) {
+        if (ids[i] != kNoToken) {
           if (DG) {
             const int n = ids[i] / SLOT, t = ids[i] % SLOT, half = c / p.cph, ch = c % p.cph;
             const uint8_t* src = p.dimg + ((long long)n * 2 * p.ngh + half * p.ngh + (ch >> 1)) * (SLOT * 128) + t * 128 +
@@ -543,7 +535,7 @@ __global__ void __launch_bounds__(THREADS, 1) news_conv_tc_kernel(const FwdParam
           if (EC == 1) load_ids(tp + n_pairs, ids_next);
           load_rows(ids_next, 0, v_next);
         }
-        if (DROP && !(p.dbg & 16)) {
+        if (DROP) {
           if (c == 0) {   // per tile: pair index of column 0 of each of this thread's rows, inner hash of its high word
 #pragma unroll
             for (int i = 0; i < 2; ++i) {
@@ -579,7 +571,6 @@ __global__ void __launch_bounds__(THREADS, 1) news_conv_tc_kernel(const FwdParam
         if (lane == 0) mbar_wait(bar_a_empty + 8 * c, ph ^ 1, 5);   // one poller per warp: both passes of the previous tile read it
         __syncwarp();
         const uint32_t slot_addr = a_base + c * A_STAGE_BYTES;
-        if (!(p.dbg & 2))
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
           const int r = pw * SLOT + 8 * (2 * rh + i) + rsub;
@@ -639,7 +630,6 @@ __global__ void __launch_bounds__(THREADS, 1) news_conv_tc_kernel(const FwdParam
     ec.s_bias = s_bias;
     ec.s_ka = s_ka;
     ec.thr = p.drop_addend;
-    ec.dbg = p.dbg;
     int par = 0;
     for (int tp = pair; tp < n_tp; tp += n_pairs) {
       const int n = (2 * tp + (int)crank) * TPT + slot, t = t0 + lane;
@@ -661,10 +651,8 @@ __global__ void __launch_bounds__(THREADS, 1) news_conv_tc_kernel(const FwdParam
       for (int fp = 0; fp < NP; ++fp) {
         mbar_wait(bar_t_full + 8 * fp, pht, 6);
         tc_fence_after();
-        if (!(p.dbg & 1)) {
-          if (fp == 0) epi_pass1_segment<FP16, DROP>(ec, io, trow, half * n0h, f_beg, n0h, tk != 0, z, vmax);
-          else epi_pass1_segment<FP16, DROP>(ec, io, trow, 2 * n0h + half * n1h, f_beg + n0h, n1h, tk != 0, z, vmax);
-        }
+        epi_pass1_segment<FP16, DROP>(ec, io, trow, fp ? 2 * n0h + half * n1h : half * n0h, fp ? f_beg + n0h : f_beg, fp ? n1h : n0h,
+                                      tk != 0, z, vmax);
         tc_fence_before();
         __syncwarp();
         if (lane == 0) {
@@ -673,7 +661,6 @@ __global__ void __launch_bounds__(THREADS, 1) news_conv_tc_kernel(const FwdParam
         }
       }
       pht ^= 1;
-      if (p.dbg & 1) continue;
       const int row = q * 32 + lane;
       s_z[(par * 2 + half) * 128 + row] = z;
       s_any[(par * 2 + half) * 128 + row] = vmax != 0u ? 1 : 0;
@@ -705,7 +692,6 @@ __global__ void __launch_bounds__(THREADS, 1) news_conv_tc_kernel(const FwdParam
       // reduce-scatter (7 shuffles per 32 features): no shared-memory staging on this pass.
       // SLOT == 64: the two warps of a title split the 32-feature chunks between them (even / odd) and each sums all 64
       // rows (the neighbour's rows and weights become visible through a second barrier), so no cross-warp reduction.
-      if (p.dbg & 4) continue;
       // pooled rows go to the title's ORIGINAL index when the kernel runs over a compacted title list
       const int n_out = (p.title_idx && n < n_titles) ? __ldg(p.title_idx + n) : n;
       constexpr int NRH = SLOT / 32;                 // 32-row halves of a title
@@ -821,8 +807,6 @@ struct WgradParams {
   uint32_t drop_thr16, drop_addend, seed_x;   // quad-stream threshold (0 = no dropout) and its mask addend
   float scale;
   long long* trace;           // optional: accumulated wait cycles of CTA (0,0)'s roles (tools/perf_conv.py)
-  int dbg;                    // experiments (LSTUR_WGRAD_DBG): 2 = skip all MMAs, 4 = skip bulk copies, 8 = producers only signal,
-                              // 16 = no proxy fence, 32 = no st.shared (timing only)
   const uint8_t* xmask;       // optional keep bits written by the forward (FwdParams::xmask); null: replay the hash
   const int* n_dev;           // optional device count of titles (K blocks) to process (<= n_kblocks): compacted title list
 };
@@ -901,17 +885,13 @@ __global__ void __launch_bounds__(WG_THREADS, 1) conv_wgrad_tc_kernel(const Wgra
         long long t0 = tracing ? clock64() : 0;
         mbar_wait(bar_empty + 8 * s, ph ^ 1, 11);
         if (tracing) { twl += clock64() - t0; p.trace[5] = twl; }
-        if (p.dbg & 4) {
-          mbar_arrive(bar_full + 8 * s);
-        } else {
-          mbar_expect_tx(bar_full + 8 * s, b_stage_bytes);
+        mbar_expect_tx(bar_full + 8 * s, b_stage_bytes);
 #pragma unroll
-          for (int t = 0; t < WG_TPS; ++t) {
-            // a title past the end re-reads the last valid block: finite values, multiplied by the zero A rows
-            const int kb = max(0, min(kb_beg + sb * WG_TPS + t, n_kblocks - 1));
-            const uint8_t* src = (const uint8_t*)p.dpre_img + ((size_t)kb * 2 + crank) * b_tile_bytes;
-            bulk_g2s(b_base + s * b_stage_bytes + t * b_tile_bytes, src, b_tile_bytes, bar_full + 8 * s);
-          }
+        for (int t = 0; t < WG_TPS; ++t) {
+          // a title past the end re-reads the last valid block: finite values, multiplied by the zero A rows
+          const int kb = max(0, min(kb_beg + sb * WG_TPS + t, n_kblocks - 1));
+          const uint8_t* src = (const uint8_t*)p.dpre_img + ((size_t)kb * 2 + crank) * b_tile_bytes;
+          bulk_g2s(b_base + s * b_stage_bytes + t * b_tile_bytes, src, b_tile_bytes, bar_full + 8 * s);
         }
         if (++s == WG_STAGES) { s = 0; ph ^= 1; }
       }
@@ -930,19 +910,17 @@ __global__ void __launch_bounds__(WG_THREADS, 1) conv_wgrad_tc_kernel(const Wgra
         if (tracing) tw += clock64() - t0;
         tc_fence_after();
         if (leader) {
-          if (!(p.dbg & 2)) {
 #pragma unroll
-            for (int t = 0; t < WG_TPS; ++t) {
-              const uint32_t a_addr = a_base + s * a_stage_bytes + t * WG_A_TILE_BYTES;
-              const uint32_t b_addr = b_base + s * b_stage_bytes + t * b_tile_bytes;
+          for (int t = 0; t < WG_TPS; ++t) {
+            const uint32_t a_addr = a_base + s * a_stage_bytes + t * WG_A_TILE_BYTES;
+            const uint32_t b_addr = b_base + s * b_stage_bytes + t * b_tile_bytes;
 #pragma unroll
-              for (int kk = 0; kk < WG_KTOK / 16; ++kk) {
-                const uint64_t ad = make_desc_mn128(a_addr + kk * 2048, WG_GROUP_BYTES);
-                umma_f16_2cta(tmem_base, ad, make_desc_mn128(b_addr + kk * 2048, WG_GROUP_BYTES), idesc0, accum);
-                if (n1h > 0)
-                  umma_f16_2cta(tmem_base + 2 * n0h, ad, make_desc_mn128(b_addr + b1_off + kk * 2048, WG_GROUP_BYTES), idesc1, accum);
-                accum = 1;
-              }
+            for (int kk = 0; kk < WG_KTOK / 16; ++kk) {
+              const uint64_t ad = make_desc_mn128(a_addr + kk * 2048, WG_GROUP_BYTES);
+              umma_f16_2cta(tmem_base, ad, make_desc_mn128(b_addr + kk * 2048, WG_GROUP_BYTES), idesc0, accum);
+              if (n1h > 0)
+                umma_f16_2cta(tmem_base + 2 * n0h, ad, make_desc_mn128(b_addr + b1_off + kk * 2048, WG_GROUP_BYTES), idesc1, accum);
+              accum = 1;
             }
           }
           umma_commit_2cta(bar_empty + 8 * s, 3);
@@ -1016,16 +994,14 @@ __global__ void __launch_bounds__(WG_THREADS, 1) conv_wgrad_tc_kernel(const Wgra
     auto stage_step = [&](int sb, uint4& cur, uint4& nxt, uint32_t mcur, uint32_t& mnxt) {
       const int kb0 = kb_beg + sb * WG_TPS;
       long long tA = tracing ? clock64() : 0;
-      if (!(p.dbg & 8)) {
-        nxt = load_row(idn);                                // stage sb+2
-        mnxt = load_mask(kb0 + 2 * WG_TPS + tsel);
-        idn = load_id(kb0 + 3 * WG_TPS + tsel);             // stage sb+3
-        if (use_mask) {
-          const uint4 lm = mask_lut[mcur];
-          cur.x &= lm.x; cur.y &= lm.y; cur.z &= lm.z; cur.w &= lm.w;
-        } else if (p.drop_thr16 && piece_ok) {
-          drop_piece(kb0 + tsel, cur);
-        }
+      nxt = load_row(idn);                                // stage sb+2
+      mnxt = load_mask(kb0 + 2 * WG_TPS + tsel);
+      idn = load_id(kb0 + 3 * WG_TPS + tsel);             // stage sb+3
+      if (use_mask) {
+        const uint4 lm = mask_lut[mcur];
+        cur.x &= lm.x; cur.y &= lm.y; cur.z &= lm.z; cur.w &= lm.w;
+      } else if (p.drop_thr16 && piece_ok) {
+        drop_piece(kb0 + tsel, cur);
       }
       long long t0 = tracing ? clock64() : 0;
       if (tracing) tseg[0] += t0 - tA;
@@ -1033,22 +1009,20 @@ __global__ void __launch_bounds__(WG_THREADS, 1) conv_wgrad_tc_kernel(const Wgra
       __syncwarp();
       if (tracing) twait += clock64() - t0;
       long long tB = tracing ? clock64() : 0;
-      if (!(p.dbg & 8)) {
-        if (piece_ok) {
-          const uint32_t tile = a_base + s * a_stage_bytes + tsel * WG_A_TILE_BYTES;
+      if (piece_ok) {
+        const uint32_t tile = a_base + s * a_stage_bytes + tsel * WG_A_TILE_BYTES;
 #pragma unroll
-          for (int j = 0; j < TAPS; ++j) {     // M row of (tap j, column e0 + i) = j * 40 + (e0 - slice * 40) + i
-            const int m0 = j * WG_ES + q * 8;
-            const int rr = (r + 1 - j) & (WG_KTOK - 1);
-            const uint32_t addr = tile + (m0 >> 6) * WG_GROUP_BYTES + rr * 128 + ((((m0 & 63) >> 3) ^ (rr & 7)) << 4);
-            asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(cur.x), "r"(cur.y), "r"(cur.z), "r"(cur.w) : "memory");
-          }
+        for (int j = 0; j < TAPS; ++j) {     // M row of (tap j, column e0 + i) = j * 40 + (e0 - slice * 40) + i
+          const int m0 = j * WG_ES + q * 8;
+          const int rr = (r + 1 - j) & (WG_KTOK - 1);
+          const uint32_t addr = tile + (m0 >> 6) * WG_GROUP_BYTES + rr * 128 + ((((m0 & 63) >> 3) ^ (rr & 7)) << 4);
+          asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(cur.x), "r"(cur.y), "r"(cur.z), "r"(cur.w) : "memory");
         }
-        long long tC = tracing ? clock64() : 0;
-        if (tracing) tseg[1] += tC - tB;
-        fence_proxy_async();
-        if (tracing) tseg[2] += clock64() - tC;
       }
+      long long tC = tracing ? clock64() : 0;
+      if (tracing) tseg[1] += tC - tB;
+      fence_proxy_async();
+      if (tracing) tseg[2] += clock64() - tC;
       long long tD = tracing ? clock64() : 0;
       __syncwarp();
       if (lane == 0) {
@@ -1079,7 +1053,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) conv_wgrad_tc_kernel(const Wgra
     tc_fence_after();
     const int row = q * 32 + lane;
     float* dst = p.partial + ((size_t)split * p.n_slices * TILE_M + (size_t)slice * TILE_M + row) * F;
-    const bool any = n_stage_blocks > 0 && !(p.dbg & 2);
+    const bool any = n_stage_blocks > 0;
     for (int seg = 0; seg < 4; ++seg) {
       const int nseg = seg < 2 ? n0h : n1h;
       const int c_beg = seg < 2 ? seg * n0h : 2 * n0h + (seg - 2) * n1h;
@@ -1129,8 +1103,6 @@ __global__ void wgrad_reduce_kernel(int E, int Ep, int F, int splits, int rows_t
 #include "plan.h"
 
 using namespace lstur;
-
-extern "C" int lstur_conv_tc_available(void) { return 1; }
 
 // Padded embedding width (multiple of the 64-element K block).
 extern "C" int lstur_tc_padded_e(int E) { return (E + tc::EPAD - 1) / tc::EPAD * tc::EPAD; }
@@ -1215,9 +1187,7 @@ size_t tc_conv_smem_bytes(int EC, int F, int nstages) {
 static int tc_launch_conv(const tc::FwdParams& p, int L, bool fp16, bool drop, int mode, int max_ctas, cudaStream_t stream,
                           const char* name) {
   const int F = p.F, slot = lstur_tc_slot(L);
-  static int nst_env = -1;
-  if (nst_env < 0) { const char* e = getenv("LSTUR_FWD_STAGES"); nst_env = e ? atoi(e) : 0; }
-  int nst = nst_env >= 2 && nst_env <= tc::MAX_STAGES ? nst_env : tc::DEF_STAGES;
+  int nst = tc::DEF_STAGES;
   while (nst > 2 && tc_conv_smem_bytes(p.EC, F, nst) > TC_SMEM_LIMIT) --nst;
   if (p.EC > tc::MAX_CHUNKS || tc_conv_smem_bytes(p.EC, F, nst) > TC_SMEM_LIMIT) {
     set_error("%s: K = %d chunks x N = %d does not fit the shared-memory plan of the tensor-core conv kernel", name, p.EC, F);
@@ -1274,7 +1244,6 @@ extern "C" int lstur_news_conv_tc_fwd_m(int n_titles, int L, int E, int F, int V
   p.drop_addend = quad_addend(p.drop_thr16);
   p.inv_keep = 1.f / (1.f - dropout);
   p.seed_x = seed * 2u; p.seed_c = seed * 2u + 1u;
-  p.dbg = getenv("LSTUR_FWD_DBG") ? atoi(getenv("LSTUR_FWD_DBG")) : 0;
   p.xmask = (uint8_t*)xmask_out;
   p.n_dev = n_titles_dev; p.title_idx = title_idx;
   p.trace = (long long*)g_tc_trace_ptr;
@@ -1344,7 +1313,6 @@ extern "C" int lstur_conv_dgrad_tc(int n_titles, int L, int E, int F, const void
   p.out_scale = out_scale;
   p.n_dev = n_titles_dev;
   p.inv_keep = 1.f;
-  p.dbg = 0;
   p.trace = nullptr;
   RC(tc_launch_conv(p, L, fp16 != 0, false, tc::MODE_DGRAD, max_ctas, stream, "lstur_conv_dgrad_tc"));
   return LSTUR_OK;
@@ -1410,7 +1378,6 @@ extern "C" int lstur_conv_wgrad_tc_m(int n_titles, int L, int E, int F, int V, c
   p.seed_x = seed * 2u;
   p.scale = 1.f / ((1.f - dropout) * dpre_scale);
   p.trace = (long long*)g_tc_trace_ptr;
-  p.dbg = getenv("LSTUR_WGRAD_DBG") ? atoi(getenv("LSTUR_WGRAD_DBG")) : 0;
   p.xmask = (const uint8_t*)xmask;
   p.n_dev = n_titles_dev;
   // a stage holds WG_STAGE_ROWS K rows whatever the slot height: A = 2 groups, B = ngh groups of 128-byte rows

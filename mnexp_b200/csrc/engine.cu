@@ -71,9 +71,6 @@ extern "C" int lstur_event_elapsed_ms(void* a, void* b, float* ms) {
   return LSTUR_OK;
 }
 
-// conv tensor-core path (conv_tc.cu)
-extern "C" int lstur_conv_tc_available(void);
-
 namespace {
 
 void add_ws(lstur_plan* p, const char* name, long long count) {
@@ -108,9 +105,9 @@ inline bool arch_hist_att(int a) { return a == LSTUR_ARCH_ATT || a == LSTUR_ARCH
 inline int arch_uc(const lstur_config& c) {
   return (c.arch == LSTUR_ARCH_INI_CON || c.arch == LSTUR_ARCH_INI_CAT || c.arch == LSTUR_ARCH_INI_ADD) ? c.Ue - c.G : c.Ue;
 }
-inline gemm_fn pick_gemm(const lstur_plan* p) {
-  return (p->c.precision == LSTUR_PREC_BF16_TC || p->c.precision == LSTUR_PREC_FP16_TC) ? lstur_gemm_tc : lstur_gemm_f32;
-}
+// the tensor-core precision modes (tcgen05 news encoder, dense GEMMs and, where it fits, GRU recurrence)
+inline bool prec_tc(const lstur_config& c) { return c.precision == LSTUR_PREC_BF16_TC || c.precision == LSTUR_PREC_FP16_TC; }
+inline gemm_fn pick_gemm(const lstur_plan* p) { return prec_tc(p->c) ? lstur_gemm_tc : lstur_gemm_f32; }
 
 }  // namespace
 
@@ -156,7 +153,7 @@ extern "C" int lstur_plan_create(const lstur_config* cfg, lstur_plan** out) {
   LSTUR_REQUIRE(c.arch != LSTUR_ARCH_INI_ADD || c.Ue == 2 * c.G, "lstur_plan_create('inagru' needs Ue == 2G)");
   LSTUR_REQUIRE((c.arch != LSTUR_ARCH_ATT_PAIR && c.arch != LSTUR_ARCH_ALPHA) || c.Ue == c.G, "lstur_plan_create('atgru' / 'algru' need Ue == G)");
   LSTUR_REQUIRE(!dot || U == D, "lstur_plan_create('dot' scorer needs user dim == doc dim)");
-  if ((c.precision == LSTUR_PREC_BF16_TC || c.precision == LSTUR_PREC_FP16_TC) && !lstur_tc_supported(c.L, c.E, c.F, c.KS)) {
+  if (prec_tc(c) && !lstur_tc_supported(c.L, c.E, c.F, c.KS)) {
     set_error("lstur_plan_create: shape (L=%d,E=%d,F=%d,KS=%d) not supported by the tensor-core conv kernel", c.L, c.E, c.F, c.KS);
     return LSTUR_ERR_UNSUPPORTED;
   }
@@ -237,7 +234,8 @@ extern "C" int lstur_plan_create(const lstur_config* cfg, lstur_plan** out) {
   p->dense_count = (p->dense_count + 3) & ~3LL;
 
   // ---- workspace
-  const bool tcp = (c.precision == LSTUR_PREC_BF16_TC || c.precision == LSTUR_PREC_FP16_TC);
+  const bool tcp = prec_tc(c);
+  p->tc_gru = has_gru && tcp && lstur_gru_tc_supported(c.B, c.W, G);
   add_ws(p, "tokens", N * c.L);
   if (!tcp) add_ws(p, "Xp", N * Lp * E);
   if (!tcp) add_ws(p, "Cp", N * Lp * F);
@@ -359,8 +357,7 @@ extern "C" int lstur_plan_create(const lstur_config* cfg, lstur_plan** out) {
   add_ws(p, "probs", B * c.C);
   add_ws(p, "loss_rows", B);
   add_ws(p, "loss", 1);
-  const bool tcp0 = c.precision == LSTUR_PREC_BF16_TC || c.precision == LSTUR_PREC_FP16_TC;
-  if (!tcp0) track_gemm(p, (int)(N * Lp), F, c.KS * E);
+  if (!tcp) track_gemm(p, (int)(N * Lp), F, c.KS * E);
   track_gemm(p, (int)N, Dd, F);
   if (bw) {
     add_ws(p, "d_user_vec", B * c.U);
@@ -493,7 +490,7 @@ int encode_titles(const lstur_plan* p, const lstur_weights* w, void* ws, int n, 
   float* docv = W<float>(p, ws, "doc_vec");
   void* gws = W<void>(p, ws, "gemm_ws");
   const size_t gwsb = p->gemm_ws_bytes;
-  if ((c.precision == LSTUR_PREC_BF16_TC || c.precision == LSTUR_PREC_FP16_TC)) {
+  if (prec_tc(c)) {
     RC(lstur_news_encoder_tc_fwd_internal(p, w, ws, n, training, seed, st));
   } else {
     float* Xp = W<float>(p, ws, "Xp");
@@ -508,7 +505,7 @@ int encode_titles(const lstur_plan* p, const lstur_weights* w, void* ws, int n, 
     RC(lstur_attn_pool_fwd(n, L, F, Cp, (long long)Lp * F, tok, DP(p, w->dense, "att_w"), DP(p, w->dense, "att_b"),
                            pooled, F, W<float>(p, ws, "att_a"), W<float>(p, ws, "att_w"), drop, seed * 2u + 1u, st));
   }
-  if (c.use_dense && W<int>(p, ws, "live_idx") && !getenv("LSTUR_GEMM_ROWS_OFF")) {
+  if (c.use_dense && W<int>(p, ws, "live_idx")) {
     // Dense over the live titles of the compacted list; an all-pad title pools to 0, so its vector is the bias
     RC(lstur_gemm_tc_mrows(0, n, c.Dd, F, pooled, F, DP(p, w->dense, "dense_w"), c.Dd, docv, D, DP(p, w->dense, "dense_b"),
                            LSTUR_GEMM_PRECISE, W<int>(p, ws, "live_idx"), W<int>(p, ws, "n_live"), gws, gwsb, st));
@@ -549,14 +546,12 @@ int user_and_score(const lstur_plan* p, const lstur_weights* w, const lstur_batc
   // 5. GRU (k11-k12)
   if (has_gru) {
     float* XW = W<float>(p, ws, "XW");
-    const bool tc_gru0 = (c.precision == LSTUR_PREC_BF16_TC || c.precision == LSTUR_PREC_FP16_TC) &&
-                         lstur_gru_tc_supported(B, c.W, G) && !getenv("LSTUR_GRU_TC_OFF");
-    int* hl_idx = getenv("LSTUR_GEMM_ROWS_OFF") ? nullptr : W<int>(p, ws, "hist_live_idx");
+    int* hl_idx = W<int>(p, ws, "hist_live_idx");
     if (hl_idx) {   // unmasked (user, step) rows, ascending (the weight gradients of the backward reduce over them too)
       RC(lstur_compact_titles(Nh, 1, reinterpret_cast<const int*>(W<float>(p, ws, "gru_mask")), W<int>(p, ws, "hist_live_scratch"),
                               hl_idx, W<int>(p, ws, "n_hist_live"), W<int>(p, ws, "hist_live_dummy"), st));
     }
-    if (hl_idx && tc_gru0) {
+    if (hl_idx && p->tc_gru) {
       // input projection of the unmasked steps only: the tcgen05 recurrence discards what it computes for a masked step
       // (select, not multiply), so the rows of XW behind masked steps are never used
       RC(lstur_gemm_tc_mrows(0, Nh, 3 * G, D, docv, D, DP(p, w->dense, "gru_wx"), 3 * G, XW, 3 * G, DP(p, w->dense, "gru_b"),
@@ -575,11 +570,8 @@ int user_and_score(const lstur_plan* p, const lstur_weights* w, const lstur_batc
     if (c.arch == LSTUR_ARCH_INI || c.arch == LSTUR_ARCH_NOID || c.arch == LSTUR_ARCH_INI_ADD) hdst = uvec;
     if (cat) { hdst = cat; ldo = G + Uc; }
     if (c.arch == LSTUR_ARCH_ATT_PAIR) { hdst = W<float>(p, ws, "seq2"); ldo = 2 * G; }
-    // tensor-core precision modes run the recurrence on tcgen05 (gru_tc.cu) when its weights fit tensor memory
-    const bool tc_gru = (c.precision == LSTUR_PREC_BF16_TC || c.precision == LSTUR_PREC_FP16_TC) &&
-                        lstur_gru_tc_supported(B, c.W, G) && !getenv("LSTUR_GRU_TC_OFF");
     // tiles of 32 batch rows skip the steps at which all their rows are masked: order the rows by their first live step
-    int* order = getenv("LSTUR_GRU_SORT_OFF") ? nullptr : W<int>(p, ws, "gru_order");
+    int* order = W<int>(p, ws, "gru_order");
     if (order) {
       int* key = W<int>(p, ws, "gru_key");
       int* scr = W<int>(p, ws, "gru_sort_scratch");
@@ -587,21 +579,16 @@ int user_and_score(const lstur_plan* p, const lstur_weights* w, const lstur_batc
       RC(lstur_sort_unique_i32(B, key, order, scr, scr + B, scr + 2 * B + 1, scr + 3 * B + 1, st));
     }
     PROBE_BEGIN(p, LSTUR_PROBE_GRU_FWD, st);
-    if (tc_gru) {
+    if (p->tc_gru) {
       RC(lstur_gru_fwd_tc(B, c.W, G, XW, W<float>(p, ws, "gru_mask"), ini ? u0 : nullptr, c.Ue,
                           DP(p, w->dense, "gru_wh"), c.rec_act, hdst, ldo, bw ? W<float>(p, ws, "Z") : nullptr,
                           bw ? W<float>(p, ws, "R") : nullptr, bw ? W<float>(p, ws, "HH") : nullptr,
                           bw ? W<float>(p, ws, "HP") : nullptr, bw ? W<float>(p, ws, "RH") : nullptr, order, st));
-    } else if (order && lstur_gru_cluster_supported(B, c.W, G)) {
-      RC(lstur_gru_fwd_cluster(B, c.W, G, XW, W<float>(p, ws, "gru_mask"), ini ? u0 : nullptr, c.Ue,
-                               DP(p, w->dense, "gru_wh"), c.rec_act, hdst, ldo, bw ? W<float>(p, ws, "Z") : nullptr,
-                               bw ? W<float>(p, ws, "R") : nullptr, bw ? W<float>(p, ws, "HH") : nullptr,
-                               bw ? W<float>(p, ws, "HP") : nullptr, bw ? W<float>(p, ws, "RH") : nullptr, order, st));
     } else {
       RC(lstur_gru_fwd(B, c.W, G, XW, W<float>(p, ws, "gru_mask"), ini ? u0 : nullptr, c.Ue,
                        DP(p, w->dense, "gru_wh"), c.rec_act, hdst, ldo, bw ? W<float>(p, ws, "Z") : nullptr,
                        bw ? W<float>(p, ws, "R") : nullptr, bw ? W<float>(p, ws, "HH") : nullptr,
-                       bw ? W<float>(p, ws, "HP") : nullptr, bw ? W<float>(p, ws, "RH") : nullptr, st));
+                       bw ? W<float>(p, ws, "HP") : nullptr, bw ? W<float>(p, ws, "RH") : nullptr, order, st));
     }
     PROBE_END(p, LSTUR_PROBE_GRU_FWD, st);
     if (cat) {
@@ -871,13 +858,13 @@ int encoder_backward(const lstur_plan* p, const lstur_weights* w, void* ws, int 
   long long lddp = F;
   if (c.use_dense) {
     // d pooled of the live titles only: the attention backward runs over the compacted list and never reads the other rows
-    if (W<int>(p, ws, "live_idx") && !getenv("LSTUR_GEMM_ROWS_OFF"))
+    if (W<int>(p, ws, "live_idx"))
       RC(lstur_gemm_tc_mrows(1, n, F, c.Dd, d_docv, D, DP(p, w->dense, "dense_w"), c.Dd, d_pooled, F, nullptr, 0,
                              W<int>(p, ws, "live_idx"), W<int>(p, ws, "n_live"), gws, gwsb, st));
     else
       RC(GEMM(0, 1, n, F, c.Dd, d_docv, D, DP(p, w->dense, "dense_w"), c.Dd, d_pooled, F, nullptr, 0, gws, gwsb, st));
     // pooled is zero for the all-pad titles: reduce over the live titles of the compacted list (tensor-core modes)
-    if (W<int>(p, ws, "live_idx") && !getenv("LSTUR_GEMM_ROWS_OFF"))
+    if (W<int>(p, ws, "live_idx"))
       RC(lstur_gemm_tc_tn_rows(F, c.Dd, n, pooled, F, d_docv, D, DG(p, dgrad, "dense_w"), c.Dd, W<int>(p, ws, "live_idx"),
                                W<int>(p, ws, "n_live"), gws, gwsb, st));
     else
@@ -891,7 +878,7 @@ int encoder_backward(const lstur_plan* p, const lstur_weights* w, void* ws, int 
   // the dropout streams are replayed only if the saved forward was a training forward (an inference forward followed by
   // a backward differentiates the inference graph)
   const float bwd_drop = p->last_training ? c.dropout : 0.f;
-  if ((c.precision == LSTUR_PREC_BF16_TC || c.precision == LSTUR_PREC_FP16_TC)) {
+  if (prec_tc(c)) {
     const int fp16 = c.precision == LSTUR_PREC_FP16_TC;
     void* img = W<void>(p, ws, "dpre_img");
     // power-of-two loss scale of the 16-bit dPre image: the gradients carry grad_scale = 1 / global batch, which would
@@ -1146,12 +1133,10 @@ extern "C" int lstur_backward_w(const lstur_plan* p, const lstur_weights* w, con
     float* WhT = W<float>(p, ws, "WhT");
     float* dA = W<float>(p, ws, "dA");
     float* dh0 = W<float>(p, ws, "dh0");
-    const bool tc_gru = (c.precision == LSTUR_PREC_BF16_TC || c.precision == LSTUR_PREC_FP16_TC) &&
-                        lstur_gru_tc_supported(B, c.W, G) && !getenv("LSTUR_GRU_TC_OFF");
     // row order of the last forward (the mask has not changed since)
-    const int* order = getenv("LSTUR_GRU_SORT_OFF") ? nullptr : W<int>(p, ws, "gru_order");
+    const int* order = W<int>(p, ws, "gru_order");
     PROBE_BEGIN(p, LSTUR_PROBE_GRU_BWD, st);
-    if (tc_gru) {
+    if (p->tc_gru) {
       // the kernel also leaves per-(tile, row group) column sums of dA: the bias gradient needs no second pass over dA
       float* dbp = W<float>(p, ws, "gru_db_partial");
       RC(lstur_gru_bwd_tc(B, c.W, G, W<float>(p, ws, "gru_mask"), W<float>(p, ws, "Z"), W<float>(p, ws, "R"),
@@ -1160,17 +1145,13 @@ extern "C" int lstur_backward_w(const lstur_plan* p, const lstur_weights* w, con
       RC(lstur_colsum(lstur_gru_tc_db_rows(B), 3 * G, dbp, 3 * G, DG(p, dgrad, "gru_b"), 0, cws, cwsb, st));
     } else {
       RC(lstur_transpose(G, 3 * G, DP(p, w->dense, "gru_wh"), WhT, st));
-      if (order && lstur_gru_cluster_supported(B, c.W, G))
-        RC(lstur_gru_bwd_cluster(B, c.W, G, W<float>(p, ws, "gru_mask"), W<float>(p, ws, "Z"), W<float>(p, ws, "R"),
-                                 W<float>(p, ws, "HH"), W<float>(p, ws, "HP"), WhT, c.rec_act, dhT, lddh, dA, dh0, G, order, st));
-      else
       RC(lstur_gru_bwd(B, c.W, G, W<float>(p, ws, "gru_mask"), W<float>(p, ws, "Z"), W<float>(p, ws, "R"),
-                       W<float>(p, ws, "HH"), W<float>(p, ws, "HP"), WhT, c.rec_act, dhT, lddh, dA, dh0, G, st));
+                       W<float>(p, ws, "HH"), W<float>(p, ws, "HP"), WhT, c.rec_act, dhT, lddh, dA, dh0, G, order, st));
       RC(lstur_colsum(Nh, 3 * G, dA, 3 * G, DG(p, dgrad, "gru_b"), 0, cws, cwsb, st));
     }
     PROBE_END(p, LSTUR_PROBE_GRU_BWD, st);
     int* hl_idx = W<int>(p, ws, "hist_live_idx");
-    if (hl_idx && !getenv("LSTUR_GEMM_ROWS_OFF")) {
+    if (hl_idx) {
       // dA is zero on masked steps: the weight gradients reduce over the unmasked (user, step) rows only (half of them with
       // the left-padded histories of short click logs)
       int* hl_n = W<int>(p, ws, "n_hist_live");       // built by the forward (user_and_score)
@@ -1187,7 +1168,7 @@ extern "C" int lstur_backward_w(const lstur_plan* p, const lstur_weights* w, con
                       nullptr, 0, gws, gwsb, st));
     }
     // dH = dA . Wx^T  (rows of masked steps are zero because dA is zero there)
-    if (hl_idx && !getenv("LSTUR_GEMM_ROWS_OFF")) {
+    if (hl_idx) {
       cudaMemsetAsync(d_docv, 0, (size_t)Nh * D * sizeof(float), st);
       RC(lstur_gemm_tc_mrows(1, Nh, D, 3 * G, dA, 3 * G, DP(p, w->dense, "gru_wx"), 3 * G, d_docv, D, nullptr, 0, hl_idx,
                              W<int>(p, ws, "n_hist_live"), gws, gwsb, st));

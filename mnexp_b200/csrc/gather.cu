@@ -26,7 +26,7 @@ __global__ void token_gather_kernel(int N, int L, int n_docs, const int* __restr
 // One warp per padded row; float4 vectorised when E % 4 == 0.
 __global__ void embed_gather_pad_kernel(int N, int L, int E, int V, int KS, const float* __restrict__ word_emb,
                                         const int* __restrict__ tok, float* __restrict__ Xp, uint32_t drop_thr,
-                                        float inv_keep, uint32_t seed, int Ep) {
+                                        float inv_keep, uint32_t seed) {
   long long row = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   int lane = threadIdx.x & 31;
   const int Lp = L + KS - 1;
@@ -41,17 +41,6 @@ __global__ void embed_gather_pad_kernel(int N, int L, int E, int V, int KS, cons
   id = (id < 0 || id >= V) ? 0 : id;
   const float* src = word_emb + (long long)id * E;
   const uint64_t base = ((uint64_t)n * L + t) * (uint64_t)E;
-  if (Ep > 0) {
-    // tensor-core dropout stream (conv_tc.cu): one 32-bit draw per element PAIR of the Ep-padded row, 16-bit thresholds
-    const uint64_t pbase = ((uint64_t)n * L + t) * (uint64_t)Ep;
-    for (int e = lane; e < E; e += 32) {
-      float v = __ldg(src + e);
-      uint32_t h = rng_u32(seed, (pbase + e) >> 1);
-      uint32_t h16 = (e & 1) ? (h >> 16) : (h & 0xffffu);
-      dst[e] = h16 >= drop_thr ? v * inv_keep : 0.f;
-    }
-    return;
-  }
   if ((E & 3) == 0) {
     for (int e = lane * 4; e < E; e += 128) {
       float4 v = __ldg((const float4*)(src + e));
@@ -332,23 +321,8 @@ extern "C" int lstur_embed_gather_pad(int N, int L, int E, int V, int KS, const 
   if (N == 0) return LSTUR_OK;
   long long rows = (long long)N * (L + KS - 1);
   embed_gather_pad_kernel<<<cdiv(rows * 32, 256), 256, 0, stream>>>(
-      N, L, E, V, KS, word_emb, tokens, Xp, dropout > 0.f ? dropout_threshold(dropout) : 0u, 1.f / (1.f - dropout), seed, 0);
+      N, L, E, V, KS, word_emb, tokens, Xp, dropout > 0.f ? dropout_threshold(dropout) : 0u, 1.f / (1.f - dropout), seed);
   LSTUR_CHECK_LAUNCH("lstur_embed_gather_pad");
-  return LSTUR_OK;
-}
-
-// Same gather, replaying the dropout stream of the tensor-core forward (pair-indexed draws over rows padded to Ep).
-extern "C" int lstur_embed_gather_pad_tcrng(int N, int L, int E, int V, int KS, int Ep, const float* word_emb,
-                                            const int* tokens, float* Xp, float dropout, unsigned seed,
-                                            cudaStream_t stream) {
-  LSTUR_REQUIRE(N >= 0 && L > 0 && E > 0 && KS >= 1 && Ep >= E && dropout >= 0.f && dropout < 1.f,
-                "lstur_embed_gather_pad_tcrng");
-  if (N == 0) return LSTUR_OK;
-  long long rows = (long long)N * (L + KS - 1);
-  embed_gather_pad_kernel<<<cdiv(rows * 32, 256), 256, 0, stream>>>(
-      N, L, E, V, KS, word_emb, tokens, Xp, dropout > 0.f ? (uint32_t)(dropout * 65536.0f) : 0u, 1.f / (1.f - dropout),
-      seed, dropout > 0.f ? Ep : 0);
-  LSTUR_CHECK_LAUNCH("lstur_embed_gather_pad_tcrng");
   return LSTUR_OK;
 }
 

@@ -694,7 +694,6 @@ __global__ void gemm_tc_splitk_reduce_kernel(int M, int N, int splits, const flo
 
 using namespace lstur;
 
-static bool g_gemm_async = true;     // LSTUR_GEMM_ASYNC=0 selects the register-staged kernel everywhere (A/B testing)
 static void gemm_tc_tiling(int M, int N, int K, int* ntile, int* splits, int max_nt = 256) {
   int nparts = (N + max_nt - 1) / max_nt;
   int nt = ((N + nparts - 1) / nparts + 15) & ~15;
@@ -765,18 +764,12 @@ static int gemm_tc_impl(int transA, int transB, int M, int N, int K, const float
   if (M == 0 || N == 0) return LSTUR_OK;
   tc::GemmParams p;
   int splits;
-  static bool env_read = false;
-  if (!env_read) {
-    const char* e = getenv("LSTUR_GEMM_ASYNC");
-    if (e && atoi(e) == 0) g_gemm_async = false;
-    env_read = true;
-  }
   // cp.async staging needs every 16-byte chunk of an operand row to be aligned and entirely inside or outside the matrix
   const bool rows16 = (lda % 4 == 0) && (ldb % 4 == 0) && ((((uintptr_t)A) & 15) == 0) && ((((uintptr_t)B) & 15) == 0) &&
                       ((transA ? M : K) % 4 == 0) && ((transB ? K : N) % 4 == 0);
   // Measured at the LSTUR shapes (tools/perf_gemm.py): the cp.async ring wins for the long-K weight-gradient GEMMs
   // (A transposed, split-K: 192 -> 106 us), the register-staged kernel with its wider N tile for the short-K ones.
-  const bool use_async = g_gemm_async && rows16 && K > 0 && transA;
+  const bool use_async = rows16 && K > 0 && transA;
   gemm_tc_tiling(M, N, K, &p.ntile, &splits, use_async ? tc::GA_NT : 256);
   size_t need = splits > 1 ? (size_t)splits * M * N * sizeof(float) : 0;
   if (need > workspace_bytes || (need && !workspace)) splits = 1;
@@ -814,10 +807,8 @@ static int gemm_tc_impl(int transA, int transB, int M, int N, int K, const float
   if (midx && mcount && !use_async && !transA && splits == 1) { p.midx = midx; p.mcount = mcount; }   // else: every row (a superset)
   // Large-M GEMMs against a small weight matrix (GRU input projection and its input gradient, scorer Dense layers):
   // pack B once per call into stage-layout fp16 tiles; the CTAs then fetch it with bulk copies.
-  static int img_mode = -1;
-  if (img_mode < 0) { const char* e = getenv("LSTUR_GEMM_BIMG"); img_mode = (e && atoi(e) == 0) ? 0 : 1; }
   const size_t img_bytes = (size_t)p.tiles_n * p.nkb_total * (split3 ? 2 : 1) * tc::G_BIMG_TILE;
-  if (img_mode && !use_async && !transA && splits == 1 && M >= 1024 && K > 0 && workspace && img_bytes <= workspace_bytes) {
+  if (!use_async && !transA && splits == 1 && M >= 1024 && K > 0 && workspace && img_bytes <= workspace_bytes) {
     dim3 pg((unsigned)p.nkb_total, (unsigned)p.tiles_n);
     uint8_t* img = (uint8_t*)workspace;
     if (transB) {

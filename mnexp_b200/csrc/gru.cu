@@ -344,18 +344,19 @@ extern "C" int lstur_gru_bwd_streaming(int B, int W, int G, const float* gm, con
 }
 
 // Dispatchers: shared-memory-resident cluster kernels (gru_cl.cu) when the shape fits, else the streaming kernels.
+// row_order (optional) is honoured by the cluster kernels only; the streaming kernels process the rows in order.
 extern "C" int lstur_gru_fwd(int B, int W, int G, const float* XW, const float* gm, const float* h0, long long ldh0,
                              const float* Wh, int rec_act, float* hT, long long ldo, float* Z, float* R, float* HH,
-                             float* HP, float* RH, cudaStream_t stream) {
+                             float* HP, float* RH, const int* row_order, cudaStream_t stream) {
   if (lstur_gru_cluster_supported(B, W, G))
-    return lstur_gru_fwd_cluster(B, W, G, XW, gm, h0, ldh0, Wh, rec_act, hT, ldo, Z, R, HH, HP, RH, nullptr, stream);
+    return lstur_gru_fwd_cluster(B, W, G, XW, gm, h0, ldh0, Wh, rec_act, hT, ldo, Z, R, HH, HP, RH, row_order, stream);
   return lstur_gru_fwd_streaming(B, W, G, XW, gm, h0, ldh0, Wh, rec_act, hT, ldo, Z, R, HH, HP, RH, stream);
 }
 
 extern "C" int lstur_gru_bwd(int B, int W, int G, const float* gm, const float* Z, const float* R, const float* HH,
                              const float* HP, const float* WhT, int rec_act, const float* dhT, long long lddh,
-                             float* dA, float* dh0, long long lddh0, cudaStream_t stream) {
+                             float* dA, float* dh0, long long lddh0, const int* row_order, cudaStream_t stream) {
   if (lstur_gru_cluster_supported(B, W, G))
-    return lstur_gru_bwd_cluster(B, W, G, gm, Z, R, HH, HP, WhT, rec_act, dhT, lddh, dA, dh0, lddh0, nullptr, stream);
+    return lstur_gru_bwd_cluster(B, W, G, gm, Z, R, HH, HP, WhT, rec_act, dhT, lddh, dA, dh0, lddh0, row_order, stream);
   return lstur_gru_bwd_streaming(B, W, G, gm, Z, R, HH, HP, WhT, rec_act, dhT, lddh, dA, dh0, lddh0, stream);
 }

@@ -20,6 +20,7 @@ struct lstur_plan {
   size_t ws_bytes = 0;
   long long dense_count = 0;
   size_t gemm_ws_bytes = 0;
+  bool tc_gru = false;      // the GRU recurrence runs on tcgen05 (gru_tc.cu): tensor-core precision, lstur_gru_tc_supported
   // optional CUDA events recorded around one kernel of the step (bench.py roofline probe)
   int probe_id = 0;
   cudaEvent_t probe_start = nullptr, probe_stop = nullptr;

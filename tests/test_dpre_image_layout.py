@@ -1,4 +1,4 @@
-"""The 16-bit dPre image layout of the tensor-core backward (csrc/attn.cu, store_dpre_img): the image builder the
+"""The 16-bit dPre image layout of the tensor-core backward (csrc/attn.cu, attn_bwd_img_kernel): the image builder the
 consumer tests use (test_gpu_tc.dpre_image) and the decoder the producer tests use
 (test_gpu_tc_backward.decode_dpre_image) are exact inverses.  CPU only."""
 import numpy as np

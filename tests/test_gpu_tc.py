@@ -186,7 +186,7 @@ def test_engine_fp16_tc_forward_and_grads(lib, shape, arch, relu_open):
 
 
 def dpre_image(dpre, fp16=1):
-    """numpy restatement of the K-block image layout documented in csrc/attn.cu (store_dpre_img)."""
+    """numpy restatement of the K-block image layout documented in csrc/attn.cu (attn_bwd_img_kernel)."""
     N, L, F = dpre.shape
     Fh = F // 2
     ngh = (Fh + 63) // 64
