@@ -255,11 +255,21 @@ int lstur_score_softmax_ce(int B, int C, int D, const float* u, long long ldu, c
 int lstur_score_sigmoid(long long n_pairs, int C, int D, const float* u, long long ldu, const float* d, long long ldd,
                         float* out, int apply_sigmoid, cudaStream_t stream);
 
-/* Device-side batch assembly: train_gen + Window + Impression.negative_samples (task/paper.py:7-18, 396-405;
- * task/seq2vec.py:17-53).  A sample is a click (global index into stream_docs) that has an earlier click of the same
- * user; idx (B) picks samples out of sample_click.  user_out (B), hist_doc_out (B,W) = the last W clicks before it,
- * left-padded with 0 (bit-exact with Window), cand_doc_out (B,1+K) = [the click, K negatives drawn with replacement from
- * neg_docs[neg_off[c] .. neg_off[c+1]) by the counter-based RNG]. */
+/* Device-side sample assembly: train_gen / valid_gen + Window + Impression.negative_samples (task/paper.py:7-18,
+ * 387-441, 669-694; task/seq2vec.py:17-53).  Every user's clicks form one stream (stream_docs[stream_off[u] ..
+ * stream_off[u+1])); a sample s is a click c = sample_click[s] (global stream index); idx (B) picks the batch's samples.
+ *   user_out (B)          click_user[c]
+ *   hist_doc_out (B,W)    the W stream entries before hist_end, left-padded with 0 (bit-exact with Window);
+ *                         hist_end = sample_hist_end[s], or c when sample_hist_end is NULL (the training rule).
+ *                         click_time non-NULL (int32 seconds since the Days Window's zero, 2000-01-01): a slot j keeps
+ *                         its doc only if click_time[j] + expire_seconds >= click_time[c] (64-bit sum), else doc 0.
+ *   cand_doc_out (B,1+K)  [the click, K negatives drawn with replacement from neg_docs[neg_off[c] .. neg_off[c+1])]:
+ *                         negative k of row b = neg_docs[n0 + rng_u32(seed, (row0 + b) * K + k) % n]. */
+int lstur_assemble_samples(int B, int W, int K, const int* sample_click, const int* sample_hist_end, const int* idx,
+                           const int* click_user, const int* click_time, long long expire_seconds, const int* stream_off,
+                           const int* stream_docs, const int* neg_off, const int* neg_docs, unsigned seed, long long row0,
+                           int* user_out, int* hist_doc_out, int* cand_doc_out, cudaStream_t stream);
+/* lstur_assemble_samples(sample_hist_end = NULL, click_time = NULL, row0 = 0): training samples, no time window. */
 int lstur_assemble_batch(int B, int W, int K, const int* sample_click, const int* idx, const int* click_user,
                          const int* stream_off, const int* stream_docs, const int* neg_off, const int* neg_docs,
                          unsigned seed, int* user_out, int* hist_doc_out, int* cand_doc_out, cudaStream_t stream);

@@ -153,32 +153,40 @@ __global__ void scale_rows_kernel(int B, int D, const float* __restrict__ scale,
 }
 
 
-// Device-side batch assembly (train_gen + Window + Impression.negative_samples, task/paper.py:7-18, 396-405,
-// task/seq2vec.py:17-53): a training sample is a click c of user u with at least one earlier click; its history is the
-// last W clicks before c (left-padded with doc 0), its positive the click itself, its negatives K draws WITH replacement
-// from the negatives shown in the click's impression.  One thread per output element.
-__global__ void assemble_batch_kernel(int B, int W, int K, const int* __restrict__ sample_click, const int* __restrict__ idx,
-                                      const int* __restrict__ click_user, const int* __restrict__ stream_off,
-                                      const int* __restrict__ stream_docs, const int* __restrict__ neg_off,
-                                      const int* __restrict__ neg_docs, uint32_t seed, int* __restrict__ user_out,
-                                      int* __restrict__ hist_out, int* __restrict__ cand_out) {
+// Device-side sample assembly (train_gen / valid_gen + Window + Impression.negative_samples, task/paper.py:7-18,
+// 387-441, 669-694; task/seq2vec.py:17-53).  Sample s = idx[b] is the click c = sample_click[s] of user u; its history is
+// the W stream entries before hist_end (hist_end = sample_hist_end[s], or c when that table is NULL), left-padded with
+// doc 0.  With click_time, a history slot j keeps its doc only while click_time[j] + expire >= click_time[c] (the Days
+// Window's expiry, summed in 64 bits; times need not be monotonic along the stream).  The positive is the click itself,
+// the negatives K draws WITH replacement from the negatives shown in the click's impression, counter-based on the global
+// row row0 + b.  One thread per output element.
+__global__ void assemble_samples_kernel(int B, int W, int K, const int* __restrict__ sample_click,
+                                        const int* __restrict__ sample_hist_end, const int* __restrict__ idx,
+                                        const int* __restrict__ click_user, const int* __restrict__ click_time,
+                                        long long expire, const int* __restrict__ stream_off,
+                                        const int* __restrict__ stream_docs, const int* __restrict__ neg_off,
+                                        const int* __restrict__ neg_docs, uint32_t seed, long long row0,
+                                        int* __restrict__ user_out, int* __restrict__ hist_out, int* __restrict__ cand_out) {
   const int T = W + 1 + K;
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)B * T) return;
   const int b = (int)(i / T), e = (int)(i % T);
-  const int c = sample_click[idx[b]];
+  const int s = idx[b];
+  const int c = sample_click[s];
   const int u = click_user[c];
   const int off = stream_off[u];
   if (e < W) {
-    const int j = c - W + e;
-    hist_out[(long long)b * W + e] = j >= off ? stream_docs[j] : 0;
+    const int j = (sample_hist_end ? sample_hist_end[s] : c) - W + e;
+    int d = j >= off ? stream_docs[j] : 0;
+    if (click_time && j >= off && (long long)click_time[j] + expire < (long long)click_time[c]) d = 0;
+    hist_out[(long long)b * W + e] = d;
     if (e == 0) user_out[b] = u;
   } else if (e == W) {
     cand_out[(long long)b * (1 + K)] = stream_docs[c];
   } else {
     const int k = e - W - 1;
     const int n0 = neg_off[c], n = neg_off[c + 1] - n0;
-    const uint32_t r = rng_u32(seed, (uint64_t)b * K + k);
+    const uint32_t r = rng_u32(seed, (uint64_t)(row0 + b) * K + k);
     cand_out[(long long)b * (1 + K) + 1 + k] = n > 0 ? neg_docs[n0 + (int)(r % (uint32_t)n)] : 0;
   }
 }
@@ -383,16 +391,26 @@ extern "C" int lstur_scale_rows(int B, int D, const float* scale, float* x, long
   return LSTUR_OK;
 }
 
+extern "C" int lstur_assemble_samples(int B, int W, int K, const int* sample_click, const int* sample_hist_end,
+                                      const int* idx, const int* click_user, const int* click_time, long long expire_seconds,
+                                      const int* stream_off, const int* stream_docs, const int* neg_off, const int* neg_docs,
+                                      unsigned seed, long long row0, int* user_out, int* hist_doc_out, int* cand_doc_out,
+                                      cudaStream_t stream) {
+  LSTUR_REQUIRE(B >= 0 && W > 0 && K >= 0 && row0 >= 0, "lstur_assemble_samples");
+  LSTUR_REQUIRE(B == 0 || (sample_click && idx && click_user && stream_off && stream_docs && neg_off && neg_docs && user_out &&
+                           hist_doc_out && cand_doc_out), "lstur_assemble_samples");
+  if (B == 0) return LSTUR_OK;
+  const long long n = (long long)B * (W + 1 + K);
+  assemble_samples_kernel<<<cdiv(n, 256), 256, 0, stream>>>(B, W, K, sample_click, sample_hist_end, idx, click_user,
+                                                            click_time, expire_seconds, stream_off, stream_docs, neg_off,
+                                                            neg_docs, seed, row0, user_out, hist_doc_out, cand_doc_out);
+  LSTUR_CHECK_LAUNCH("lstur_assemble_samples");
+  return LSTUR_OK;
+}
+
 extern "C" int lstur_assemble_batch(int B, int W, int K, const int* sample_click, const int* idx, const int* click_user,
                                     const int* stream_off, const int* stream_docs, const int* neg_off, const int* neg_docs,
                                     unsigned seed, int* user_out, int* hist_doc_out, int* cand_doc_out, cudaStream_t stream) {
-  LSTUR_REQUIRE(B >= 0 && W > 0 && K >= 0, "lstur_assemble_batch");
-  LSTUR_REQUIRE(B == 0 || (sample_click && idx && click_user && stream_off && stream_docs && neg_off && neg_docs && user_out &&
-                           hist_doc_out && cand_doc_out), "lstur_assemble_batch");
-  if (B == 0) return LSTUR_OK;
-  const long long n = (long long)B * (W + 1 + K);
-  assemble_batch_kernel<<<cdiv(n, 256), 256, 0, stream>>>(B, W, K, sample_click, idx, click_user, stream_off, stream_docs,
-                                                          neg_off, neg_docs, seed, user_out, hist_doc_out, cand_doc_out);
-  LSTUR_CHECK_LAUNCH("lstur_assemble_batch");
-  return LSTUR_OK;
+  return lstur_assemble_samples(B, W, K, sample_click, nullptr, idx, click_user, nullptr, 0, stream_off, stream_docs, neg_off,
+                                neg_docs, seed, 0, user_out, hist_doc_out, cand_doc_out, stream);
 }

@@ -8,11 +8,15 @@
   get_layer(name), get_weights / set_weights, summary()         task/test_pipeline.py:28,87; utils.py:70,79
 
 Inputs are host numpy arrays in the reference's order: [user(B,) , clicked(B,W,L), cand_0(B,L) .. cand_K(B,L)]
-(user omitted for the classes without a user-ID embedding), target (B,1+K) one-hot.
+(user omitted for the classes without a user-ID embedding), target (B,1+K) one-hot.  train_on_batch / fit_generator /
+evaluate / evaluate_generator of the softmax family also take batches assembled on the device (assemble.DeviceBatch,
+the task handlers' device_train / device_valid): doc ids go to the engine as they are, the target is the positive in
+column 0, and vertical ids come from the engine's doc_vert table.
 """
 import numpy as np
 import torch
 
+from .assemble import DeviceBatch
 from .engine import LsturEngine
 
 
@@ -57,6 +61,7 @@ class _Core:
         self.predict_rows = predict_rows
         self.step_seed = 0
         self.freeze_encoder = False     # --enable-pretrain-encoder without --pretrain-encoder-trainable (task/paper.py:103-106)
+        self.doc_vert = None            # (n_docs,) vertical of every document: vertical ids of device-assembled batches
 
     def precision(self):
         p = getattr(self.cfg, 'precision', 'auto')
@@ -79,7 +84,8 @@ class _Core:
                 dropout=c.dropout, lr=c.learning_rate, recurrent_activation=c.recurrent_activation,
                 precision=self.precision(), doc_tokens=self.doc_tokens, training=True,
                 sparse_user_adam=bool(c.sparse_user_adam), score_model=self.score_model,
-                trainable_word_emb=bool(getattr(c, 'textual_embedding_trainable', False)), **self.head_kw())
+                trainable_word_emb=bool(getattr(c, 'textual_embedding_trainable', False)), doc_vert=self.doc_vert,
+                **self.head_kw())
             if old is not None:
                 self.train_engine.adopt_state_from(old)
             self.train_engine.freeze_encoder = self.freeze_encoder
@@ -151,6 +157,38 @@ class _Core:
             user = np.zeros(clicked.shape[0], dtype=np.int32)
         return user, clicked, cand, verts
 
+    def device_inputs(self, batch, n_cand, with_label=True):
+        """assemble.DeviceBatch -> engine batch dict: the doc ids as they are (user zeroed for the classes without a
+        user-ID embedding, as split_inputs does), the target = the positive in column 0."""
+        if self.loss == 'bce':
+            raise ValueError('device-assembled batches feed the softmax family only')
+        B = batch.B
+        assert batch.cand_doc.shape[1] == n_cand, 'the batch has %d candidates per row, the model %d' % (batch.cand_doc.shape[1], n_cand)
+        dev = batch.hist_doc.device
+        cache = self.__dict__.setdefault('_device_consts', {})
+        user = batch.user
+        if not self.has_user:
+            if ('zeros', B) not in cache:
+                cache[('zeros', B)] = torch.zeros(B, dtype=torch.int32, device=dev)
+            user = cache[('zeros', B)]
+        db = dict(user=user, hist_doc=batch.hist_doc, cand_doc=batch.cand_doc)
+        if with_label:
+            if ('label', B, n_cand) not in cache:
+                lab = torch.zeros((B, n_cand), dtype=torch.float32, device=dev)
+                lab[:, 0] = 1.0
+                cache[('label', B, n_cand)] = lab
+            db['label'] = cache[('label', B, n_cand)]
+        return db
+
+    def device_user_scale(self, B, device):
+        """dgru's Dropout(0.5, noise_shape=(None, 1)) multipliers drawn on the device (0 or 2 per row), from a generator
+        seeded once from numpy's global state."""
+        g = self.__dict__.get('_scale_gen')
+        if g is None:
+            g = self.__dict__['_scale_gen'] = torch.Generator(device=device)
+            g.manual_seed(int(np.random.randint(1 << 31)))
+        return (torch.rand(B, device=device, generator=g) >= 0.5).to(torch.float32) * 2.0
+
 
 class Model:
     """`model` (train=True: probabilities over the 1+K candidates) or `test_model` (sigmoid of one candidate)."""
@@ -175,26 +213,33 @@ class Model:
         assert self.is_train, 'test_model is not compiled for training'
         core = self.core
         C = core.n_train_cand()
-        user, clicked, cand, verts = core.split_inputs(x, C)
-        eng = core.engine_train(clicked.shape[0])
-        eng.lr = core.optimizer.lr.value
-        batch = dict(user=user, hist_tok=core.stage_tokens('hist', clicked, slot), cand_tok=core.stage_tokens('cand', cand, slot),
-                     label=np.asarray(y, dtype=np.float32).reshape(len(clicked), C))
-        if verts is not None:
-            batch['hist_vert'], batch['cand_vert'] = verts
-        if core.arch == 'dgru':     # Dropout(0.5, noise_shape=(None, 1)) on the user vector (task/paper.py:609)
-            batch['user_scale'] = (np.random.random(clicked.shape[0]) >= 0.5).astype(np.float32) * 2.0
-        if copy_stream is None:
-            db = eng.to_device_batch(batch, non_blocking=True)
-        else:       # upload on a side stream: it runs under the previous step's kernels; this step waits for it
-            main = torch.cuda.current_stream()
-            with torch.cuda.stream(copy_stream):
+        if isinstance(x, DeviceBatch):      # assembled on the device: nothing to stage or upload
+            eng = core.engine_train(x.B)
+            eng.lr = core.optimizer.lr.value
+            db = core.device_inputs(x, C)
+            if core.arch == 'dgru':
+                db['user_scale'] = core.device_user_scale(x.B, eng.device)
+        else:
+            user, clicked, cand, verts = core.split_inputs(x, C)
+            eng = core.engine_train(clicked.shape[0])
+            eng.lr = core.optimizer.lr.value
+            batch = dict(user=user, hist_tok=core.stage_tokens('hist', clicked, slot), cand_tok=core.stage_tokens('cand', cand, slot),
+                         label=np.asarray(y, dtype=np.float32).reshape(len(clicked), C))
+            if verts is not None:
+                batch['hist_vert'], batch['cand_vert'] = verts
+            if core.arch == 'dgru':     # Dropout(0.5, noise_shape=(None, 1)) on the user vector (task/paper.py:609)
+                batch['user_scale'] = (np.random.random(clicked.shape[0]) >= 0.5).astype(np.float32) * 2.0
+            if copy_stream is None:
                 db = eng.to_device_batch(batch, non_blocking=True)
-                ready = torch.cuda.Event()
-                ready.record(copy_stream)
-            main.wait_event(ready)
-            for t in db.values():
-                t.record_stream(main)
+            else:       # upload on a side stream: it runs under the previous step's kernels; this step waits for it
+                main = torch.cuda.current_stream()
+                with torch.cuda.stream(copy_stream):
+                    db = eng.to_device_batch(batch, non_blocking=True)
+                    ready = torch.cuda.Event()
+                    ready.record(copy_stream)
+                main.wait_event(ready)
+                for t in db.values():
+                    t.record_stream(main)
         nv = eng.B if n_valid is None else int(n_valid)      # rows beyond nv are padding with an all-zero target (fit)
         dp = core.dp(eng)
         if dp is None:
@@ -228,7 +273,8 @@ class Model:
         done.synchronize()
         return [float(res[0]), float(res[1])]
 
-    def train_on_batch(self, x, y):
+    def train_on_batch(self, x, y=None):
+        """x, y: host inputs and targets, or x = an assemble.DeviceBatch (no y)."""
         return self._finish_train(self._enqueue_train(x, y))
 
     def fit_generator(self, generator, steps_per_epoch, epochs=1, initial_epoch=0, verbose=0, **_):
@@ -246,7 +292,7 @@ class Model:
             tot = np.zeros(len(self.metrics_names))
             pending = None
             for step in range(steps_per_epoch):
-                x, y = next(generator)
+                x, y = _unpack(next(generator))
                 if not pipelined:
                     tot += self.train_on_batch(x, y)
                     continue
@@ -354,9 +400,35 @@ class Model:
 
     predict_on_batch = predict
 
-    def evaluate(self, x, y, batch_size=None, verbose=0, **_):
-        y = np.asarray(y[0] if isinstance(y, (list, tuple)) else y, dtype=np.float64)
-        p = self.predict(x).astype(np.float64)
+    def _predict_device(self, batch):
+        """probabilities (B, 1+K) of an assemble.DeviceBatch through the same inference engine and row chunks as predict
+        on host arrays (pad rows = doc 0, the all-zero title)."""
+        core = self.core
+        if not self.is_train:
+            raise ValueError('device-assembled batches carry 1+K candidates: evaluate them with `model`, not test_model')
+        C = core.n_train_cand()
+        src = core.device_inputs(batch, C, with_label=False)
+        eng = core.engine_infer(C)
+        R, n = eng.B, batch.B
+        outs = []
+        for s in range(0, n, R):
+            m = min(R, n - s)
+            db = {}
+            for k, v in src.items():
+                t = torch.zeros((R,) + tuple(v.shape[1:]), dtype=v.dtype, device=v.device)
+                t[:m] = v[s:s + m]
+                db[k] = t
+            outs.append(eng.forward(db, training=False)[:m].cpu().numpy().copy())
+        return np.concatenate(outs)
+
+    def evaluate(self, x, y=None, batch_size=None, verbose=0, **_):
+        if isinstance(x, DeviceBatch):
+            p = self._predict_device(x).astype(np.float64)
+            y = np.zeros(p.shape, dtype=np.float64)
+            y[:, 0] = 1.0
+        else:
+            y = np.asarray(y[0] if isinstance(y, (list, tuple)) else y, dtype=np.float64)
+            p = self.predict(x).astype(np.float64)
         if self.core.loss == 'bce':              # Seq2Vec.loss + utils.auc_roc
             from . import metrics
             K, yy, q = float(self.core.cfg.negative_samples), y.reshape(-1), p.reshape(-1)
@@ -372,7 +444,7 @@ class Model:
     def evaluate_generator(self, generator, steps, verbose=0, **_):
         tot = np.zeros(len(self.metrics_names))
         for _ in range(steps):
-            x, y = next(generator)
+            x, y = _unpack(next(generator))
             tot += self.evaluate(x, y)
         return list(tot / max(1, steps))
 
@@ -448,14 +520,23 @@ class VertSupModel(Model):
         acc = float((probs.argmax(1) == db['label'].argmax(1)).float().mean())
         n = eng.B * (eng.W + eng.C)
         vp = eng.view('vs_probs').reshape(n, eng.aux_nv)
-        lab = torch.cat([db['hist_vert'].reshape(-1), db['cand_vert'].reshape(-1)])
+        if 'hist_vert' in db:
+            lab = torch.cat([db['hist_vert'].reshape(-1), db['cand_vert'].reshape(-1)])
+        else:                       # device batch: the verticals of its documents
+            lab = eng.doc_vert[torch.cat([db['hist_doc'].reshape(-1), db['cand_doc'].reshape(-1)]).long()]
         vacc = float((vp.argmax(1) == lab).float().mean())
         main, aux = eng.loss(), eng.aux_loss()
         return [main + eng.aux_gain * aux, main, aux, acc, vacc]
 
-    def train_on_batch(self, x, y):
+    def train_on_batch(self, x, y=None):
         core = self.core
         C = core.n_train_cand()
+        if isinstance(x, DeviceBatch):
+            eng = core.engine_train(x.B)
+            eng.lr = core.optimizer.lr.value
+            db = core.device_inputs(x, C)
+            eng.train_step(db)
+            return self._metrics(eng, db)
         user, clicked, cand, _ = core.split_inputs(x, C)
         eng = core.engine_train(clicked.shape[0])
         eng.lr = core.optimizer.lr.value
@@ -466,9 +547,14 @@ class VertSupModel(Model):
         eng.train_step(db)
         return self._metrics(eng, db)
 
-    def evaluate(self, x, y, batch_size=None, verbose=0, **_):
+    def evaluate(self, x, y=None, batch_size=None, verbose=0, **_):
         core = self.core
         C = core.n_train_cand()
+        if isinstance(x, DeviceBatch):
+            eng = core.engine_train(x.B)
+            db = core.device_inputs(x, C)
+            eng.forward(db, training=False)
+            return self._metrics(eng, db)
         user, clicked, cand, _ = core.split_inputs(x, C)
         eng = core.engine_train(clicked.shape[0])
         hv, cv = self._vert_ids(y[1], clicked.shape[1])
@@ -554,6 +640,11 @@ class VertModel:
             x, y = next(generator)
             tot += self.evaluate(x, y)
         return list(tot / max(1, steps))
+
+
+def _unpack(item):
+    """a generator's item -> (x, y): an assemble.DeviceBatch carries its own target"""
+    return (item, None) if isinstance(item, DeviceBatch) else item
 
 
 class _InputLayer:

@@ -48,11 +48,15 @@ def _with_captured_evaluations(log, fn, *args):
         utils.logging_evaluation = orig
 
 
-def train(config, on_build=None):
-    """main.py:56-96.  on_build(handler) runs once after the first build_model (tests load reference weights there)."""
+def train(config, on_build=None, device_batches=False):
+    """main.py:56-96.  on_build(handler) runs once after the first build_model (tests load reference weights there).
+    device_batches: feed the handler's device_train / device_valid (batches assembled on the GPU, softmax-family handlers;
+    their sampling differs from the host generators', mnexp_b200/assemble.py) where the loop feeds train / valid."""
     log = _Log()
     handler = task.get(config)
-    training_data = handler.train
+    if device_batches and not hasattr(handler, 'device_train'):
+        raise NotImplementedError('%s has no device-assembled batches (the softmax-family handlers have)' % config.task)
+    training_data = handler.device_train if device_batches else handler.train
     for epoch in range(config.epochs):
         logging.info('[+] start epoch {}'.format(epoch))
         model = handler.build_model(epoch)
@@ -63,7 +67,8 @@ def train(config, on_build=None):
         if hasattr(handler, 'callback'):
             _with_captured_evaluations(log, handler.callback, epoch)
         try:
-            evaluations = model.evaluate_generator(handler.valid, handler.validation_step, verbose=2)
+            valid = handler.device_valid if device_batches else handler.valid
+            evaluations = model.evaluate_generator(valid, handler.validation_step, verbose=2)
             log.evaluation(dict(zip(model.metrics_names, evaluations)))
         except Exception:           # the reference swallows evaluation failures the same way (main.py:82-88)
             pass

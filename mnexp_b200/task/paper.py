@@ -237,6 +237,52 @@ class Seq2VecPaperSoftmax(Seq2VecPaper):
                         for pos in impression.pos:
                             self._w_push(ch, pos, impression)
 
+    # ---- device-assembled batches (mnexp_b200/assemble.py): an opt-in alternative to `train` / `valid` with its own
+    # sampling — a device permutation per epoch instead of the 100·B shuffle pool, counter-based negatives instead of
+    # np.random.choice — over the same samples, windows and candidates ------------------------------------------------
+    DEVICE_SEED = 0         # the same on every data-parallel rank: the ranks draw one permutation and take disjoint rows
+
+    def _w_device(self):
+        """The time window of `_new_window` as build_tables wants it: None (no expiry) here, (time_of, seconds) for Days."""
+        return None
+
+    def _device_batcher(self, split):
+        from .. import assemble
+        import torch.distributed as tdist
+        if getattr(self, '_device_tables', None) is None:       # (host tables, their device copies): built once
+            self._device_tables = (assemble.build_tables(self.data, self.config.window_size, self._w_device()), None)
+        rank, world = 0, 1
+        if split == 'train' and tdist.is_available() and tdist.is_initialized():
+            rank, world = tdist.get_rank(), tdist.get_world_size()
+        c = self.config
+        host, dev = self._device_tables
+        bt = assemble.DeviceBatcher(self.data, c.batch_size, c.window_size, c.negative_samples, seed=self.DEVICE_SEED,
+                                    split=split, rank=rank, world=world, window=self._w_device(), tables=host,
+                                    device_tables=dev)
+        self._device_tables = (host, bt.t)
+        return bt
+
+    @property
+    def device_train(self):
+        """Endless generator of assembled training batches (assemble.DeviceBatch) for model.fit_generator; under
+        torch.distributed every rank yields its own disjoint share of each global batch."""
+        return self._device_batcher('train').batches()
+
+    @property
+    def device_valid(self):
+        """Endless generator of assembled validation batches for model.evaluate_generator, in valid_gen order from the
+        first sample on."""
+        return self._device_batcher('valid').batches()
+
+    def device_doc_vert(self):
+        """(doc_count,) int32 vertical of every document (doc 0 and ids absent from DocMeta -> 0): the engine's doc_vert
+        table, from which device batches take their vertical ids."""
+        tab = np.zeros(self.doc_count, dtype=np.int32)
+        for i, d in self.docs.items():
+            if i:
+                tab[i] = getattr(d, 'vertical', 0)
+        return tab
+
     def test_gen(self):
         def __gen__(_user, _clicked, _impression):
             for p in _impression.pos:
@@ -400,6 +446,10 @@ class _DaysWindowMixin:
     def _w_push(self, ch, pos, impression):
         ch.push(pos, impression.time)
 
+    def _w_device(self):
+        zero = self.Window.zero
+        return (lambda imp: (imp.time - zero) // timedelta(seconds=1)), timedelta(days=self.config.days) // timedelta(seconds=1)
+
 
 class Seq2VecPaperSoftmaxDays(_DaysWindowMixin, Seq2VecPaperSoftmax):
     """task/paper.py:668-750."""
@@ -463,6 +513,7 @@ class Seq2VecPaperSoftmaxDaysIdVert(Seq2VecPaperSoftmaxDaysId):
     def _build_model(self):
         super(Seq2VecPaperSoftmaxDaysIdVert, self)._build_model()
         self._core.has_vert = True
+        self._core.doc_vert = self.device_doc_vert()     # vertical ids of device batches (host batches carry their own)
 
 
 def _to_categorical(ids, num_classes):
@@ -524,6 +575,7 @@ class Seq2VecPaperSoftmaxDaysIdVertSup(Seq2VecPaperSoftmaxDaysId):
 
     def _build_model(self):
         super(Seq2VecPaperSoftmaxDaysIdVertSup, self)._build_model()
+        self._core.doc_vert = self.device_doc_vert()     # vertical labels of device batches (host batches carry their own)
         layers = self.model.layers
         self.model = keras_like.VertSupModel(self._core, name='model')
         self.model.layers.update(layers)
@@ -538,6 +590,11 @@ class Seq2VecPaperSoftmaxDaysIdVertAlt(Seq2VecPaperSoftmaxDaysId):
         super(Seq2VecPaperSoftmaxDaysIdVertAlt, self).__init__(config)
         self.round = self.config.round
         self.config.epochs *= self.round
+
+    def _device_batcher(self, split):
+        # the vertical epochs train VertModel on title batches, which device-assembled click batches cannot feed
+        raise NotImplementedError('device-assembled batches do not cover the alternating vertical model of '
+                                  'Seq2VecPaperSoftmaxDaysIdVertAlt: train it from handler.train / handler.valid')
 
     def _load_docs(self):
         super(Seq2VecPaperSoftmaxDaysIdVertAlt, self)._load_docs()
