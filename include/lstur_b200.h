@@ -254,6 +254,12 @@ int lstur_score_softmax_ce(int B, int C, int D, const float* u, long long ldu, c
                            cudaStream_t stream);
 int lstur_score_sigmoid(long long n_pairs, int C, int D, const float* u, long long ldu, const float* d, long long ldd,
                         float* out, int apply_sigmoid, cudaStream_t stream);
+/* Ragged test head over impressions of different sizes: out[j] = sigmoid(u[pair_row[j]] . d[pair_doc[j]]) (d[j] when
+ * pair_doc is NULL), one warp per pair.  lstur_csr_rows: CSR offsets (n_rows + 1) -> row_of[j - offsets[0]] = the row
+ * whose range [offsets[r], offsets[r+1]) holds j. */
+int lstur_score_sigmoid_ragged(long long n_pairs, int D, const int* pair_row, const float* u, long long ldu,
+                               const int* pair_doc, const float* d, long long ldd, float* out, cudaStream_t stream);
+int lstur_csr_rows(int n_rows, const int* offsets, int* row_of, cudaStream_t stream);
 
 /* Device-side sample assembly: train_gen / valid_gen + Window + Impression.negative_samples (task/paper.py:7-18,
  * 387-441, 669-694; task/seq2vec.py:17-53).  Every user's clicks form one stream (stream_docs[stream_off[u] ..
@@ -275,10 +281,10 @@ int lstur_assemble_batch(int B, int W, int K, const int* sample_click, const int
                          unsigned seed, int* user_out, int* hist_doc_out, int* cand_doc_out, cudaStream_t stream);
 
 /* Pieces of the 'dnn' / 'ddot' scorers (task/paper.py:448-455) and of 'niavg' (models.py:422-441) around the GEMMs:
- * pair rows [u[b] ‖ d[(b,c)]] and their gradient split (du summed over the C candidates in a fixed order), the output
+ * pair rows [u[b] ‖ d[(b,c)]] (b = i / C, or pair_row[i] when pair_row is non-NULL) and their gradient split (du summed over the C candidates in a fixed order), the output
  * Dense(1), its backward (dhid, and dl*hid whose column sums are d w2), tanh and its backward, the masked mean. */
 int lstur_pair_concat(long long n_pairs, int C, int U, int D, const float* u, long long ldu, const float* d,
-                      long long ldd, float* out, cudaStream_t stream);
+                      long long ldd, float* out, const int* pair_row, cudaStream_t stream);
 int lstur_pair_split(int B, int C, int U, int D, const float* dcat, float* du, long long lddu, float* dd, long long lddd,
                      cudaStream_t stream);
 int lstur_rowdot_bias(long long n, int H, const float* h, const float* w, const float* bias, float* out,
@@ -531,6 +537,18 @@ int lstur_encode_titles(const lstur_plan* plan, const lstur_weights* weights, vo
                         float* doc_vec_out, long long ldo, cudaStream_t stream);
 int lstur_forward_docvecs(const lstur_plan* plan, const lstur_weights* weights, const lstur_batch* batch, void* workspace,
                           const float* doc_vec_table, long long ld, int n_rows, cudaStream_t stream);
+/* Ranking of whole impressions (the evaluation pass of Seq2VecPaperSoftmax.callback, task/paper.py:497-524) against
+ * cached document vectors doc_vec_table (n_rows, document-vector width), on an inference plan (save_for_backward = 0).
+ * Impression i: user[i], history hist_doc[i, 0..W), candidates cand_doc[cand_off[i] .. cand_off[i+1]).
+ * scores_out[j] = sigmoid(score(user vector of j's impression, doc_vec_table[cand_doc[j]])) with the plan's scorer ('dot',
+ * 'dnn', 'ddot'): the test head's value, as LsturEngine.score_sigmoid after lstur_forward.  The user encoder runs once per
+ * impression, on chunks of at most B impressions and B*C pairs; an impression of more than B*C candidates is
+ * LSTUR_ERR_ARG.  A history slot is masked when its document's title is all zero tokens (weights->doc_tokens required),
+ * as lstur_forward masks it; a candidate keeps its row of the table.  cand_off (n_impr + 1 ints) is HOST memory: the
+ * chunks are cut on the host and each chunk's offsets copied to the device.  Every other array is on the device. */
+int lstur_score_impressions(const lstur_plan* plan, const lstur_weights* weights, void* workspace, int n_impr,
+                            const int* user, const int* hist_doc, const int* cand_off, const int* cand_doc,
+                            const float* doc_vec_table, int n_rows, float* scores_out, cudaStream_t stream);
 
 #ifdef __cplusplus
 }

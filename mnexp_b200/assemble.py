@@ -31,7 +31,11 @@ def build_tables(data, W=None, window=None):
     impression's negatives (neg_off / neg_docs, per click) and, with a window, its impression's time (click_time).
     sample_click: training samples in train_gen order.  valid_click / valid_hist_end: validation samples in valid_gen
     order (every positive of every validation impression of a user with both splits) and the stream index of the first
-    click of their impression (valid_gen pushes an impression's clicks only after yielding all of them)."""
+    click of their impression (valid_gen pushes an impression's clicks only after yielding all of them).
+    eval_*: one entry per validation impression of a user with both splits, in test_gen order — eval_first_click (the
+    stream index of its first click: its history is the W stream entries before it, its user and time those of that
+    click), eval_npos (its positives), eval_cand_off (n + 1) / eval_cand_docs (CSR: its positives in file order, then all
+    its negatives in file order, as test_gen yields them)."""
     imps = [(u, s, imp) for u, (ih, iv) in enumerate(data) for s, part in ((0, ih), (1, iv)) for imp in part]
     i64 = lambda a: np.asarray(a, dtype=np.int64)
     imp_user = i64([u for u, _, _ in imps])
@@ -81,10 +85,24 @@ def build_tables(data, W=None, window=None):
     valid_click = c[valid]
     valid_hist_end = imp_first[click_imp[valid]]
 
+    # evaluation impressions (test_gen order): every validation impression of a user with both splits; its candidates
+    # are its positives in file order, then all its negatives in file order
+    ev = np.nonzero((imp_split == 1) & has_both[imp_user])[0]
+    eval_first_click, eval_npos, ev_nneg = imp_first[ev], imp_npos[ev], imp_nneg[ev]
+    eval_cand_off = np.concatenate([[0], np.cumsum(eval_npos + ev_nneg)])
+    eval_cand_docs = np.zeros(int(eval_cand_off[-1]), dtype=np.int64)
+    dst0 = eval_cand_off[:-1]
+    for n, src, src0, dst in ((eval_npos, stream_docs, eval_first_click, dst0), (ev_nneg, neg_flat, imp_neg0[ev], dst0 + eval_npos)):
+        k = np.repeat(np.arange(len(ev)), n)                       # the impression of every entry
+        j = np.arange(len(k)) - np.repeat(np.cumsum(n) - n, n)     # its index within the impression's positives / negatives
+        eval_cand_docs[dst[k] + j] = src[src0[k] + j]
+
     i32 = lambda a: np.ascontiguousarray(a, dtype=np.int32)
     out = dict(stream_off=i32(stream_off), stream_docs=i32(stream_docs if len(stream_docs) else [0]), click_user=i32(click_user),
                neg_off=i32(neg_off), neg_docs=i32(neg_docs if len(neg_docs) else [0]), sample_click=i32(sample_click),
-               valid_click=i32(valid_click), valid_hist_end=i32(valid_hist_end))
+               valid_click=i32(valid_click), valid_hist_end=i32(valid_hist_end), eval_first_click=i32(eval_first_click),
+               eval_npos=i32(eval_npos), eval_cand_off=i32(eval_cand_off),
+               eval_cand_docs=i32(eval_cand_docs if len(eval_cand_docs) else [0]))
     if click_time is not None:
         assert click_time.size == 0 or (click_time.min() >= -2 ** 31 and click_time.max() < 2 ** 31), 'times beyond int32 seconds'
         out['click_time'] = i32(click_time)

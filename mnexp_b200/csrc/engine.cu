@@ -423,6 +423,11 @@ extern "C" int lstur_plan_create(const lstur_config* cfg, lstur_plan** out) {
     if (con_dense) track_gemm(p, G + Uc, c.U, (int)B);
   }
   if (has_rnn) track_gemm(p, (int)Nh, NG * G, D);
+  if (!bw) {   // lstur_score_impressions: one chunk's users, rebased candidate offsets and pair -> impression rows
+    add_ws(p, "ev_user", B);
+    add_ws(p, "ev_off", B + 1);
+    add_ws(p, "ev_pair_row", p->Nc);
+  }
   add_ws(p, "gemm_ws", (long long)(p->gemm_ws_bytes / 4) + 4);
   {
     int cols = NG * G > D ? NG * G : D;
@@ -519,8 +524,8 @@ int encode_titles(const lstur_plan* p, const lstur_weights* w, void* ws, int n, 
   return LSTUR_OK;
 }
 
-// User encoder + scorer + loss (k10-k14) on doc_vec / gru_mask already in the workspace.
-int user_and_score(const lstur_plan* p, const lstur_weights* w, const lstur_batch* b, void* ws, cudaStream_t st) {
+// User encoder (k10-k12) on the history rows of doc_vec / gru_mask already in the workspace -> user_vec (B, U).
+int user_vector(const lstur_plan* p, const lstur_weights* w, const lstur_batch* b, void* ws, cudaStream_t st) {
   const lstur_config& c = p->c;
   const int Nh = p->Nh, D = p->D, G = c.G, B = c.B;
   const bool bw = c.save_for_backward != 0;
@@ -637,6 +642,19 @@ int user_and_score(const lstur_plan* p, const lstur_weights* w, const lstur_batc
   } else {
     cudaMemcpyAsync(uvec, u0, (size_t)B * c.Ue * 4, cudaMemcpyDeviceToDevice, st);
   }
+  return LSTUR_OK;
+}
+
+// User encoder + scorer + loss (k10-k14) on doc_vec / gru_mask already in the workspace.
+int user_and_score(const lstur_plan* p, const lstur_weights* w, const lstur_batch* b, void* ws, cudaStream_t st) {
+  const lstur_config& c = p->c;
+  const int Nh = p->Nh, D = p->D, B = c.B;
+  const gemm_fn GEMM = pick_gemm(p);
+  float* docv = W<float>(p, ws, "doc_vec");
+  void* gws = W<void>(p, ws, "gemm_ws");
+  const size_t gwsb = p->gemm_ws_bytes;
+  float* uvec = W<float>(p, ws, "user_vec");
+  RC(user_vector(p, w, b, ws, st));
   // 6. score + softmax + loss (k13-k14)
   const float* cand = docv + (size_t)Nh * D;
   const bool bce = c.loss_model == LSTUR_LOSS_WEIGHTED_BCE;
@@ -654,7 +672,7 @@ int user_and_score(const lstur_plan* p, const lstur_weights* w, const lstur_batc
     float* hid = W<float>(p, ws, "sc_hid");
     float* raw = W<float>(p, ws, "sc_raw");
     float* ones = W<float>(p, ws, "sc_ones");
-    RC(lstur_pair_concat(p->Nc, c.C, c.U, D, uvec, c.U, cand, D, sc_cat, st));
+    RC(lstur_pair_concat(p->Nc, c.C, c.U, D, uvec, c.U, cand, D, sc_cat, nullptr, st));
     RC(GEMM(0, 0, p->Nc, c.Hs, K2, sc_cat, K2, DP(p, w->dense, "sh_w"), c.Hs, hid, c.Hs, DP(p, w->dense, "sh_b"),
             LSTUR_GEMM_RELU | LSTUR_GEMM_PRECISE, gws, gwsb, st));
     RC(lstur_rowdot_bias(p->Nc, c.Hs, hid, DP(p, w->dense, "so_w"), DP(p, w->dense, "so_b"), raw, st));
@@ -837,6 +855,111 @@ extern "C" int lstur_forward_docvecs(const lstur_plan* p, const lstur_weights* w
   return user_and_score(p, w, b, ws, st);
 }
 
+// Ranking of whole impressions against cached document vectors (the validation / test pass of Seq2VecPaperSoftmax.callback,
+// task/paper.py:497-524): impression i has the user user[i], the history hist_doc[i, :W] and the candidates
+// cand_doc[cand_off[i] .. cand_off[i+1]); scores_out[j] = sigmoid(score(user vector of j's impression, doc_vec_table[cand_doc[j]]))
+// with the plan's own scorer, the value of the test head.  The user encoder runs once per impression, on chunks of at
+// most B impressions and B*C pairs.  cand_off is HOST memory (the chunks are cut on the host; each chunk's offsets are
+// copied to the device); every other array is on the device.  A history slot is masked when its document's title is all
+// zero tokens (weights->doc_tokens), as in lstur_forward; a candidate keeps its table row whatever its title.
+extern "C" int lstur_score_impressions(const lstur_plan* p, const lstur_weights* w, void* ws, int n_impr, const int* user,
+                                       const int* hist_doc, const int* cand_off, const int* cand_doc,
+                                       const float* doc_vec_table, int n_rows, float* scores_out, cudaStream_t st) {
+  LSTUR_REQUIRE(p && w && ws && w->dense && w->doc_tokens && n_impr >= 0, "lstur_score_impressions");
+  LSTUR_REQUIRE(n_impr == 0 || (user && hist_doc && cand_off && cand_doc && doc_vec_table && n_rows > 0 && scores_out),
+                "lstur_score_impressions");
+  const lstur_config& c = p->c;
+  LSTUR_REQUIRE(c.save_for_backward == 0, "lstur_score_impressions(needs an inference plan: save_for_backward = 0)");
+  LSTUR_REQUIRE(c.loss_model == LSTUR_LOSS_SOFTMAX_CE, "lstur_score_impressions(the softmax-family test head)");
+  const int Nh = p->Nh, Nc = p->Nc, D = p->D, B = c.B, L = c.L;
+  for (int i = 0; i < n_impr; ++i) {
+    const int n = cand_off[i + 1] - cand_off[i];
+    if (n < 0) {
+      set_error("lstur_score_impressions: cand_off decreases at impression %d", i);
+      return LSTUR_ERR_ARG;
+    }
+    if (n > Nc) {
+      set_error("lstur_score_impressions: impression %d has %d candidates, more than one chunk of the plan holds "
+                "(B*C = %d*%d = %d): build the plan with more rows or candidates", i, n, B, c.C, Nc);
+      return LSTUR_ERR_ARG;
+    }
+  }
+  if (n_impr == 0) return LSTUR_OK;
+  const gemm_fn GEMM = pick_gemm(p);
+  void* gws = W<void>(p, ws, "gemm_ws");
+  const size_t gwsb = p->gemm_ws_bytes;
+  float* docv = W<float>(p, ws, "doc_vec");
+  float* cand = docv + (size_t)Nh * D;
+  float* uvec = W<float>(p, ws, "user_vec");
+  int* tok = W<int>(p, ws, "tokens");
+  int* ev_user = W<int>(p, ws, "ev_user");
+  int* ev_off = W<int>(p, ws, "ev_off");
+  int* pair_row = W<int>(p, ws, "ev_pair_row");
+  lstur_batch b;
+  memset(&b, 0, sizeof(b));
+  b.user = ev_user;
+  std::vector<int> off;
+  const_cast<lstur_plan*>(p)->last_training = 0;
+  for (int i0 = 0; i0 < n_impr;) {
+    int i1 = i0;
+    while (i1 < n_impr && i1 - i0 < B && cand_off[i1 + 1] - cand_off[i0] <= Nc) ++i1;
+    const int m = i1 - i0, p0 = cand_off[i0], np = cand_off[i1] - p0;
+    off.assign(cand_off + i0, cand_off + i1 + 1);
+    cudaMemcpyAsync(ev_off, off.data(), (size_t)(m + 1) * 4, cudaMemcpyHostToDevice, st);
+    RC(lstur_csr_rows(m, ev_off, pair_row, st));
+    // users and history rows of the chunk; rows m..B are padding (user 0, all history slots masked)
+    cudaMemsetAsync(ev_user, 0, (size_t)B * 4, st);
+    cudaMemcpyAsync(ev_user, user + i0, (size_t)m * 4, cudaMemcpyDeviceToDevice, st);
+    const long long nh = (long long)m * c.W;
+    RC(lstur_token_gather((int)nh, L, c.n_docs, w->doc_tokens, hist_doc + (size_t)i0 * c.W, tok, st));
+    RC(lstur_row_gather((int)nh, D, n_rows, doc_vec_table, hist_doc + (size_t)i0 * c.W, nullptr, docv, D, st));
+    if (nh < Nh) {
+      cudaMemsetAsync(tok + nh * L, 0, (size_t)(Nh - nh) * L * 4, st);
+      cudaMemsetAsync(docv + nh * D, 0, (size_t)(Nh - nh) * D * 4, st);
+    }
+    RC(lstur_hist_mask_apply(Nh, L, D, tok, docv, D, W<float>(p, ws, "hist_mask"), W<float>(p, ws, "gru_mask"), st));
+    RC(user_vector(p, w, &b, ws, st));
+    float* out = scores_out + p0;
+    const int* cd = cand_doc + p0;
+    if (c.score_model == LSTUR_SCORE_DOT) {
+      RC(lstur_score_sigmoid_ragged(np, D, pair_row, uvec, c.U, cd, doc_vec_table, D, out, st));
+    } else {
+      RC(lstur_row_gather(np, D, n_rows, doc_vec_table, cd, nullptr, cand, D, st));
+      if (c.score_model == LSTUR_SCORE_DNN) {   // [u ‖ d] pair rows -> relu Dense -> Dense(1) -> sigmoid
+        const int K2 = c.U + D;
+        float* sc_cat = W<float>(p, ws, "sc_cat");
+        float* hid = W<float>(p, ws, "sc_hid");
+        float* raw = W<float>(p, ws, "sc_raw");
+        float* ones = W<float>(p, ws, "sc_ones");
+        RC(lstur_pair_concat(np, 1, c.U, D, uvec, c.U, cand, D, sc_cat, pair_row, st));
+        RC(GEMM(0, 0, np, c.Hs, K2, sc_cat, K2, DP(p, w->dense, "sh_w"), c.Hs, hid, c.Hs, DP(p, w->dense, "sh_b"),
+                LSTUR_GEMM_RELU | LSTUR_GEMM_PRECISE, gws, gwsb, st));
+        RC(lstur_rowdot_bias(np, c.Hs, hid, DP(p, w->dense, "so_w"), DP(p, w->dense, "so_b"), raw, st));
+        RC(lstur_fill(B, 1.f, ones, st));
+        RC(lstur_score_sigmoid_ragged(np, 1, pair_row, ones, 1, nullptr, raw, 1, out, st));
+      } else {                                  // Dense(Hs) (+ tanh) on both sides, then dot
+        float* uh = W<float>(p, ws, "sc_uh");
+        float* dh = W<float>(p, ws, "sc_dh");
+        RC(GEMM(0, 0, B, c.Hs, c.U, uvec, c.U, DP(p, w->dense, "su_w"), c.Hs, uh, c.Hs, DP(p, w->dense, "su_b"),
+                LSTUR_GEMM_PRECISE, gws, gwsb, st));
+        RC(GEMM(0, 0, np, c.Hs, D, cand, D, DP(p, w->dense, "sd_w"), c.Hs, dh, c.Hs, DP(p, w->dense, "sd_b"),
+                LSTUR_GEMM_PRECISE, gws, gwsb, st));
+        if (c.score_model == LSTUR_SCORE_DDOT) {
+          RC(lstur_tanh_fwd((long long)B * c.Hs, uh, st));
+          RC(lstur_tanh_fwd((long long)np * c.Hs, dh, st));
+        }
+        RC(lstur_score_sigmoid_ragged(np, c.Hs, pair_row, uh, c.Hs, nullptr, dh, c.Hs, out, st));
+      }
+    }
+    i0 = i1;
+  }
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) {
+    set_error("lstur_score_impressions: %s", cudaGetErrorString(e));
+    return LSTUR_ERR_CUDA;
+  }
+  return LSTUR_OK;
+}
 
 namespace {
 

@@ -77,6 +77,30 @@ __global__ void score_sigmoid_kernel(long long n, int C, int D, const float* __r
   if (lane == 0) out[i] = apply_sigmoid ? 1.f / (1.f + expf(-acc)) : acc;
 }
 
+// Ragged test head: one warp per pair j, out[j] = sigmoid(u[pair_row[j]] . d[pair_doc ? pair_doc[j] : j]); the sum runs
+// in the lane order of score_sigmoid_kernel.
+__global__ void score_sigmoid_ragged_kernel(long long n, int D, const int* __restrict__ pair_row, const float* __restrict__ u,
+                                            long long ldu, const int* __restrict__ pair_doc, const float* __restrict__ d,
+                                            long long ldd, float* __restrict__ out) {
+  const long long j = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (j >= n) return;
+  const float* ub = u + (long long)pair_row[j] * ldu;
+  const float* dj = d + (pair_doc ? (long long)pair_doc[j] : j) * ldd;
+  float acc = 0.f;
+  for (int k = lane; k < D; k += 32) acc = fmaf(ub[k], dj[k], acc);
+  acc = warp_sum(acc);
+  if (lane == 0) out[j] = 1.f / (1.f + expf(-acc));
+}
+// CSR offsets (n_rows + 1, starting anywhere) -> row_of[j - offsets[0]] = the row that pair j belongs to; one warp per row
+__global__ void csr_rows_kernel(int n_rows, const int* __restrict__ offsets, int* __restrict__ row_of) {
+  const int r = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+  const int lane = threadIdx.x & 31;
+  if (r >= n_rows) return;
+  const int base = offsets[0], e = offsets[r + 1] - base;
+  for (int j = offsets[r] - base + lane; j < e; j += 32) row_of[j] = r;
+}
+
 __global__ void mean_kernel(int n, const float* __restrict__ x, float* __restrict__ out) {
   __shared__ float s[32];
   float acc = 0.f;
@@ -151,13 +175,16 @@ __global__ void ranking_metrics_kernel(int n_impr, const int* __restrict__ offse
 // (models.py:422-441): small row-wise kernels around the dense GEMMs.
 
 // out[(b,c)] = [u[b] (U) ‖ d[(b,c)] (D)]
+// pair_row (nullable): the user row of pair i comes from a ragged list (pair_row[i]) instead of i / C
 __global__ void pair_concat_kernel(long long n_pairs, int C, int U, int D, const float* __restrict__ u, long long ldu,
-                                   const float* __restrict__ d, long long ldd, float* __restrict__ out) {
+                                   const float* __restrict__ d, long long ldd, float* __restrict__ out,
+                                   const int* __restrict__ pair_row) {
   const int K = U + D;
   const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) / K;
   const int k = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) % K);
   if (i >= n_pairs) return;
-  out[i * K + k] = k < U ? u[(i / C) * ldu + k] : d[i * ldd + (k - U)];
+  const long long r = pair_row ? (long long)pair_row[i] : i / C;
+  out[i * K + k] = k < U ? u[r * ldu + k] : d[i * ldd + (k - U)];
 }
 // du[b] = sum_c dcat[(b,c), :U] (fixed order);  dd[(b,c)] = dcat[(b,c), U:]
 __global__ void pair_split_kernel(int B, int C, int U, int D, const float* __restrict__ dcat, float* __restrict__ du,
@@ -315,11 +342,29 @@ extern "C" int lstur_ranking_metrics(int n_impr, const int* offsets, const float
   return LSTUR_OK;
 }
 
+extern "C" int lstur_score_sigmoid_ragged(long long n_pairs, int D, const int* pair_row, const float* u, long long ldu,
+                                          const int* pair_doc, const float* d, long long ldd, float* out,
+                                          cudaStream_t stream) {
+  LSTUR_REQUIRE(n_pairs >= 0 && D > 0 && (n_pairs == 0 || (pair_row && u && d && out)), "lstur_score_sigmoid_ragged");
+  if (n_pairs == 0) return LSTUR_OK;
+  score_sigmoid_ragged_kernel<<<cdiv(n_pairs * 32, 256), 256, 0, stream>>>(n_pairs, D, pair_row, u, ldu, pair_doc, d, ldd,
+                                                                            out);
+  LSTUR_CHECK_LAUNCH("lstur_score_sigmoid_ragged");
+  return LSTUR_OK;
+}
+extern "C" int lstur_csr_rows(int n_rows, const int* offsets, int* row_of, cudaStream_t stream) {
+  LSTUR_REQUIRE(n_rows >= 0 && (n_rows == 0 || (offsets && row_of)), "lstur_csr_rows");
+  if (n_rows == 0) return LSTUR_OK;
+  csr_rows_kernel<<<cdiv((long long)n_rows * 32, 256), 256, 0, stream>>>(n_rows, offsets, row_of);
+  LSTUR_CHECK_LAUNCH("lstur_csr_rows");
+  return LSTUR_OK;
+}
+
 extern "C" int lstur_pair_concat(long long n_pairs, int C, int U, int D, const float* u, long long ldu, const float* d,
-                                 long long ldd, float* out, cudaStream_t stream) {
+                                 long long ldd, float* out, const int* pair_row, cudaStream_t stream) {
   LSTUR_REQUIRE(n_pairs >= 0 && C >= 1 && U > 0 && D > 0 && u && d && out, "lstur_pair_concat");
   if (n_pairs == 0) return LSTUR_OK;
-  pair_concat_kernel<<<cdiv(n_pairs * (U + D), 256), 256, 0, stream>>>(n_pairs, C, U, D, u, ldu, d, ldd, out);
+  pair_concat_kernel<<<cdiv(n_pairs * (U + D), 256), 256, 0, stream>>>(n_pairs, C, U, D, u, ldu, d, ldd, out, pair_row);
   LSTUR_CHECK_LAUNCH("lstur_pair_concat");
   return LSTUR_OK;
 }

@@ -359,6 +359,41 @@ class LsturEngine:
         table[0].zero_()
         return table
 
+    def eval_doc_table(self):
+        """Vectors of every document of the token table, as the news encoder gives them (row 0, the pad document, is
+        Dense(0) = the bias), with the vertical columns of the doc_vert / doc_subvert tables in plans that have them:
+        the candidate rows of score_impressions."""
+        n_docs = int(self.doc_tokens.shape[0])
+        ids = torch.arange(n_docs, dtype=torch.int32, device=self.device)
+        table = self.encode_docs(ids)
+        if self.cfg.dv + self.cfg.ds:
+            assert (self.cfg.dv == 0 or self.doc_vert is not None) and (self.cfg.ds == 0 or self.doc_subvert is not None), \
+                'the vertical columns need the doc_vert / doc_subvert tables'
+            _lib.check(self.lib.lstur_vert_concat(
+                n_docs, self.D, self.D - self.cfg.dv - self.cfg.ds, self.cfg.dv, self.cfg.ds, n_docs, self.cfg.n_vert,
+                self.cfg.n_subvert, _ptr(ids), _ptr(self.doc_vert), _ptr(self.doc_subvert),
+                ctypes.c_void_p(self.dense.data_ptr() + 4 * self.layout['vert_emb'][0]) if self.cfg.dv else None,
+                ctypes.c_void_p(self.dense.data_ptr() + 4 * self.layout['subvert_emb'][0]) if self.cfg.ds else None,
+                _ptr(table), None, None, self._stream()))
+        return table
+
+    def score_impressions(self, user, hist_doc, cand_off, cand_doc, table, out=None):
+        """Test-head scores of whole impressions (lstur_score_impressions): user (n,), hist_doc (n, W), cand_doc (pairs,)
+        int32 device tensors, cand_off (n + 1,) host int32 offsets into cand_doc, table = eval_doc_table().  The user
+        encoder runs once per impression.  -> (cand_off[-1],) float32 device tensor of sigmoid scores (entries before
+        cand_off[0] are left as they were in `out`)."""
+        off = np.ascontiguousarray(cand_off, dtype=np.int32)
+        n = len(off) - 1
+        assert table.dtype == torch.float32 and table.is_contiguous() and table.shape[1] == self.D
+        if out is None:
+            out = torch.empty(int(off[-1]) if n >= 0 else 0, dtype=torch.float32, device=self.device)
+        for t in (user, hist_doc, cand_doc):
+            assert t.dtype == torch.int32 and t.is_contiguous() and t.device == self.device
+        _lib.check(self.lib.lstur_score_impressions(self.plan, ctypes.byref(self._w), _ptr(self.ws), n, _ptr(user),
+                                                    _ptr(hist_doc), off.ctypes.data_as(ctypes.c_void_p), _ptr(cand_doc),
+                                                    _ptr(table), int(table.shape[0]), _ptr(out), self._stream()))
+        return out
+
     def forward_docvecs(self, db, table):
         """User encoder + scorer over cached document vectors (TestPipeline.test_user_vec / test_user_doc_score);
         db carries user, hist_doc (B,W), cand_doc (B,C).  Returns the (B, C) softmax probabilities; score_sigmoid()

@@ -48,14 +48,19 @@ def _with_captured_evaluations(log, fn, *args):
         utils.logging_evaluation = orig
 
 
-def train(config, on_build=None, device_batches=False):
+def train(config, on_build=None, device_batches=False, device_eval=False):
     """main.py:56-96.  on_build(handler) runs once after the first build_model (tests load reference weights there).
     device_batches: feed the handler's device_train / device_valid (batches assembled on the GPU, softmax-family handlers;
-    their sampling differs from the host generators', mnexp_b200/assemble.py) where the loop feeds train / valid."""
+    their sampling differs from the host generators', mnexp_b200/assemble.py) where the loop feeds train / valid.
+    device_eval: call handler.device_callback (the same impressions ranked on the GPU; the metrics differ by rounding
+    only) where the loop calls handler.callback; independent of device_batches."""
     log = _Log()
     handler = task.get(config)
     if device_batches and not hasattr(handler, 'device_train'):
         raise NotImplementedError('%s has no device-assembled batches (the softmax-family handlers have)' % config.task)
+    if device_eval and not getattr(handler, 'DEVICE_EVAL', False):
+        raise NotImplementedError('%s has no device evaluation (the softmax-family handlers but ...VertAlt have)' % config.task)
+    callback = getattr(handler, 'device_callback' if device_eval else 'callback', None)
     training_data = handler.device_train if device_batches else handler.train
     for epoch in range(config.epochs):
         logging.info('[+] start epoch {}'.format(epoch))
@@ -64,8 +69,8 @@ def train(config, on_build=None, device_batches=False):
             on_build(handler)
         history = model.fit_generator(training_data, handler.training_step, epochs=epoch + 1, initial_epoch=epoch, verbose=2)
         log.history(history)
-        if hasattr(handler, 'callback'):
-            _with_captured_evaluations(log, handler.callback, epoch)
+        if callback is not None:
+            _with_captured_evaluations(log, callback, epoch)
         try:
             valid = handler.device_valid if device_batches else handler.valid
             evaluations = model.evaluate_generator(valid, handler.validation_step, verbose=2)

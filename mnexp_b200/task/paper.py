@@ -52,6 +52,12 @@ class Seq2VecPaper(Seq2Vec):
     def save_model(self):
         pass                                                 # task/paper.py:254-255
 
+    DEVICE_EVAL = False     # handlers whose epoch-end ranking can run on the GPU (device_callback)
+
+    def device_callback(self, epoch):
+        raise NotImplementedError('%s has no device evaluation (the softmax-family handlers have): use handler.callback'
+                                  % type(self).__name__)
+
     # ---- sigmoid family: one (history, candidate, label) sample per row, weighted BCE (task/paper.py:36-256) ----
     HAS_USER = False
     SCORE = 'dnn'                                            # score_encoder: Dense(relu)([u ‖ d]) -> Dense(1, sigmoid), :222-226
@@ -246,11 +252,26 @@ class Seq2VecPaperSoftmax(Seq2VecPaper):
         """The time window of `_new_window` as build_tables wants it: None (no expiry) here, (time_of, seconds) for Days."""
         return None
 
+    def _host_tables(self):
+        from .. import assemble
+        if getattr(self, '_device_tables', None) is None:       # (host tables, their device copies): built once
+            self._device_tables = (assemble.build_tables(self.data, self.config.window_size, self._w_device()), None)
+        return self._device_tables[0]
+
+    def _uploaded_tables(self):
+        import torch
+        host = self._host_tables()
+        dev = self._device_tables[1]
+        if dev is None:
+            device = torch.device('cuda', torch.cuda.current_device())
+            dev = {k: torch.as_tensor(v).to(device) for k, v in host.items()}
+            self._device_tables = (host, dev)
+        return host, dev
+
     def _device_batcher(self, split):
         from .. import assemble
         import torch.distributed as tdist
-        if getattr(self, '_device_tables', None) is None:       # (host tables, their device copies): built once
-            self._device_tables = (assemble.build_tables(self.data, self.config.window_size, self._w_device()), None)
+        self._host_tables()
         rank, world = 0, 1
         if split == 'train' and tdist.is_available() and tdist.is_initialized():
             rank, world = tdist.get_rank(), tdist.get_world_size()
@@ -273,6 +294,70 @@ class Seq2VecPaperSoftmax(Seq2VecPaper):
         """Endless generator of assembled validation batches for model.evaluate_generator, in valid_gen order from the
         first sample on."""
         return self._device_batcher('valid').batches()
+
+    # ---- device evaluation: the impressions of test_gen ranked on the GPU from news vectors encoded once per pass -----
+    DEVICE_EVAL = True
+
+    def _eval_engine(self):
+        """Inference engine of the device evaluation (shares the live weights): C = the mean impression size (at most the
+        plan's 32), and enough rows that the largest impression fits one chunk of rows * C pairs."""
+        sizes = np.diff(self._host_tables()['eval_cand_off'])
+        C = int(min(32, max(1, np.ceil(sizes.mean())))) if len(sizes) else 1
+        rows = max(int(self.config.batch_size), -(-int(sizes.max(initial=1)) // C))
+        return self._core.engine_infer(C, rows=rows)
+
+    def device_test(self, n):
+        """The first n impressions of test_gen (all of them if there are fewer, as zip(range(n), self.test)) scored on the
+        GPU by test_model's head -> (offsets (m + 1,), scores (offsets[-1],), labels (offsets[-1],)) device tensors; the
+        candidates of impression i are entries offsets[i] .. offsets[i+1] in test_gen order, positives (label 1) first.
+        Every document is encoded once, the user encoder runs once per impression (LsturEngine.score_impressions)."""
+        import ctypes
+        import torch
+        from .. import _lib
+        host, dev = self._uploaded_tables()
+        m = min(int(n), len(host['eval_first_click']))
+        off = host['eval_cand_off'][:m + 1]
+        if getattr(self, '_eval_label', None) is None:
+            sizes = np.diff(host['eval_cand_off'])
+            rank = np.arange(int(host['eval_cand_off'][-1])) - np.repeat(host['eval_cand_off'][:-1], sizes)
+            self._eval_label = torch.as_tensor((rank < np.repeat(host['eval_npos'], sizes)).astype(np.float32)).to(
+                dev['eval_cand_off'].device)
+        eng = self._eval_engine()
+        W = self.config.window_size
+        user = torch.empty(m, dtype=torch.int32, device=eng.device)
+        hist = torch.empty((m, W), dtype=torch.int32, device=eng.device)
+        pos = torch.empty((m, 1), dtype=torch.int32, device=eng.device)
+        idx = torch.arange(m, dtype=torch.int32, device=eng.device)
+        w = self._w_device()
+        p = lambda x: ctypes.c_void_p(None if x is None else x.data_ptr())
+        # the history of impression i: the W stream entries before its first click (K = 0: no negatives are drawn)
+        _lib.check(eng.lib.lstur_assemble_samples(
+            m, W, 0, p(dev['eval_first_click']), p(dev['eval_first_click']), p(idx), p(dev['click_user']),
+            p(dev.get('click_time')), 0 if w is None else int(w[1]), p(dev['stream_off']), p(dev['stream_docs']),
+            p(dev['neg_off']), p(dev['neg_docs']), 0, 0, p(user), p(hist), p(pos), eng._stream()))
+        table = eng.eval_doc_table()
+        scores = eng.score_impressions(user, hist, off, dev['eval_cand_docs'], table)
+        P = int(off[-1])
+        return dev['eval_cand_off'][:m + 1], scores[:P], self._eval_label[:P]
+
+    def _device_rows(self, x):
+        import ctypes
+        import torch
+        from .. import _lib
+        off, scores, labels = self.device_test(x)
+        n = int(off.numel()) - 1
+        out = torch.empty((n, 4), dtype=torch.float32, device=off.device)
+        if n:
+            _lib.check(_lib.load().lstur_ranking_metrics(
+                n, ctypes.c_void_p(off.data_ptr()), ctypes.c_void_p(scores.data_ptr()), ctypes.c_void_p(labels.data_ptr()),
+                ctypes.c_void_p(out.data_ptr()), ctypes.c_void_p(torch.cuda.current_stream(off.device).cuda_stream)))
+        host = self._host_tables()
+        return out.cpu().numpy(), host['eval_npos'][:n].tolist(), np.diff(host['eval_cand_off'][:n + 1]).tolist()
+
+    def device_callback(self, epoch):
+        """callback with the impressions ranked on the GPU (device_test + the device metrics): the same learning-rate
+        decay, model swap, last_evaluation and logged lines; the metrics differ from callback's by rounding only."""
+        self._ranking_callback(epoch, self._device_rows)
 
     def device_doc_vert(self):
         """(doc_count,) int32 vertical of every document (doc 0 and ids absent from DocMeta -> 0): the engine's doc_vert
@@ -367,21 +452,25 @@ class Seq2VecPaperSoftmax(Seq2VecPaper):
             m.layers['doc_encoder'] = self.doc_encoder
             m.layers['user_encoder'] = self.user_encoder
 
-    def callback(self, epoch):
-        """LR decay + per-impression AUC / nDCG@10 / nDCG@5 / MRR on the validation split (task/paper.py:497-524)."""
+    def _host_rows(self, x):
+        # the reference scores one impression at a time on the host (roc_auc_score, utils.ndcg_score / mrr_score);
+        # here the x impressions are ranked in ONE launch of the device kernel (mnexp_b200/metrics.py)
+        preds, trues = [], []
+        for _, (y_pred, y_true) in zip(range(x), self.test):
+            preds.append(np.asarray(y_pred).reshape(-1)); trues.append(np.asarray(y_true).reshape(-1))
+        return metrics.ranking_metrics(preds, trues), [np.sum(y) for y in trues], [len(y) for y in trues]
+
+    def _ranking_callback(self, epoch, rows_of):
+        """LR decay, the model swap, and the two evaluation lines of the first validation_impression impressions (two more
+        of the first testing_impression after the last epoch); rows_of(x) -> ((x, 4) metrics, positives, sizes)."""
         keras_like.backend.set_value(self.model.optimizer.lr,
                                      keras_like.backend.get_value(self.model.optimizer.lr) * self.config.learning_rate_decay)
         self.model, self.test_model = self.test_model, self.model
 
         def __gen__(x):
-            # the reference scores one impression at a time on the host (roc_auc_score, utils.ndcg_score / mrr_score);
-            # here the x impressions are ranked in ONE launch of the device kernel (mnexp_b200/metrics.py)
-            preds, trues = [], []
-            for _, (y_pred, y_true) in zip(range(x), self.test):
-                preds.append(np.asarray(y_pred).reshape(-1)); trues.append(np.asarray(y_true).reshape(-1))
-            m = metrics.ranking_metrics(preds, trues)
-            for i, (row, y_true) in enumerate(zip(m, trues)):
-                yield float(row[0]), float(row[1]), float(row[2]), float(row[3]), np.sum(y_true), len(y_true), i
+            m, pos, size = rows_of(x)
+            for i, (row, p, n) in enumerate(zip(m, pos, size)):
+                yield float(row[0]), float(row[1]), float(row[2]), float(row[3]), p, n, i
 
         values = [np.mean(x) for x in zip(*__gen__(self.config.validation_impression))]
         self.last_evaluation = dict(auc=values[0], ndcgx=values[1], ndcgv=values[2], mrr=values[3])
@@ -393,6 +482,10 @@ class Seq2VecPaperSoftmax(Seq2VecPaper):
             utils.logging_evaluation(dict(auc=values[0], ndcgx=values[1], ndcgv=values[2], mrr=values[3]))
             utils.logging_evaluation(dict(pos=values[4], size=values[5], num=values[6] * 2 + 1))
         self.model, self.test_model = self.test_model, self.model
+
+    def callback(self, epoch):
+        """LR decay + per-impression AUC / nDCG@10 / nDCG@5 / MRR on the validation split (task/paper.py:497-524)."""
+        self._ranking_callback(epoch, self._host_rows)
 
 
 class Seq2VecPaperSoftmaxId(Seq2VecPaperSoftmax):
@@ -595,6 +688,15 @@ class Seq2VecPaperSoftmaxDaysIdVertAlt(Seq2VecPaperSoftmaxDaysId):
         # the vertical epochs train VertModel on title batches, which device-assembled click batches cannot feed
         raise NotImplementedError('device-assembled batches do not cover the alternating vertical model of '
                                   'Seq2VecPaperSoftmaxDaysIdVertAlt: train it from handler.train / handler.valid')
+
+    DEVICE_EVAL = False
+
+    def device_test(self, n):
+        raise NotImplementedError('the device evaluation does not cover Seq2VecPaperSoftmaxDaysIdVertAlt, whose epochs '
+                                  'alternate with the vertical model: evaluate it with handler.callback')
+
+    def device_callback(self, epoch):
+        return self.device_test(self.config.validation_impression)
 
     def _load_docs(self):
         super(Seq2VecPaperSoftmaxDaysIdVertAlt, self)._load_docs()
