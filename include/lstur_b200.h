@@ -217,7 +217,8 @@ int lstur_gru_bwd(int B, int W, int G, const float* gm, const float* Z, const fl
 /* The two implementations behind lstur_gru_fwd/bwd.  _cluster: recurrent weights resident in the shared memory of a
  * thread-block cluster for the whole launch, state exchanged through distributed shared memory (gru_cl.cu);
  * row_order (B) optionally permutes the batch rows inside the kernel (length-sorted tiles skip padded steps) or NULL.
- * _streaming: weights streamed from L2 every step (any G <= 1024). */
+ * _streaming: weights streamed from L2 every step, any G <= 1024 (8 batch rows per CTA where the register file allows one
+ * thread per unit, else 4). */
 int lstur_gru_cluster_supported(int B, int W, int G);
 int lstur_gru_fwd_cluster(int B, int W, int G, const float* XW, const float* gm, const float* h0, long long ldh0,
                           const float* Wh, int rec_act, float* hT, long long ldo, float* Z, float* R, float* HH,
@@ -339,7 +340,8 @@ int lstur_alpha_add_bwd(int rows, int D, const float* alpha, const float* a, lon
 /* softmax + keras.losses.categorical_crossentropy against integer class labels (= one-hot targets): the auxiliary
  * vertical classifier of Seq2VecPaperSoftmaxDaysIdVertSup (task/paper.py:899-902, 973-990) and the vertical model of
  * ...VertAlt (:1128-1136).  logits (n, n_classes); probs / loss_rows / loss_mean / dlogits optional;
- * dlogits = scale * dL_row/dlogits (zero through a saturated clip, like Keras). */
+ * dlogits = scale * dL_row/dlogits (zero through a saturated clip, like Keras).  A label outside [0, n_classes) is read
+ * as class 0. */
 int lstur_softmax_ce_labels(long long n, int n_classes, const float* logits, const int* label, float* probs,
                             float* loss_rows, float* loss_mean, float* dlogits, float scale, cudaStream_t stream);
 /* g[i] = 0 where y[i] <= 0: backward of a relu Dense given its output y */
@@ -350,7 +352,7 @@ int lstur_minmaxnorm(int n, float lo, float hi, float* w, cudaStream_t stream);
 /* keras.layers.LSTM(G)(Masking()(history)) of cook 'ilstm' (task/cook.py:161-163): recurrent part.  XW (B,W,4G) = H.Wx + b
  * precomputed, gate order i,f,c,o; masked steps carry (h, c); output = last h.  SI..STC (B,W,G) saved gates / previous
  * cell / previous state / tanh(c') (all NULL for inference).  Backward yields dA (B,W,4G), zero on masked steps; WhT is
- * Wh transposed (4G, G). */
+ * Wh transposed (4G, G).  Any G <= 1024. */
 int lstur_lstm_fwd(int B, int W, int G, const float* XW, const float* gm, const float* Wh, int rec_act, float* hT,
                    long long ldo, float* SI, float* SF, float* SG, float* SO, float* SCP, float* SHP, float* STC,
                    cudaStream_t stream);

@@ -32,6 +32,12 @@ extern unsigned long long g_launch_count;   // kernels launched through this lib
 
 static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
 
+// Widest CTA a kernel can be launched with on the current device (its register count included); 0 if the query fails.
+static inline int kernel_max_threads(const void* fn) {
+  cudaFuncAttributes a{};
+  return cudaFuncGetAttributes(&a, fn) == cudaSuccess ? a.maxThreadsPerBlock : 0;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -26,10 +26,11 @@ __device__ __forceinline__ float rec_act_grad(float y, int act) {
 }
 
 template <int BT>
-__global__ void gru_fwd_kernel(int B, int W, int G, const float* __restrict__ XW, const float* __restrict__ gm,
-                               const float* __restrict__ h0, long long ldh0, const float* __restrict__ Wh, int act,
-                               float* __restrict__ hT, long long ldo, float* __restrict__ Z, float* __restrict__ R,
-                               float* __restrict__ HH, float* __restrict__ HP, float* __restrict__ RH) {
+__device__ __forceinline__ void gru_fwd_body(int B, int W, int G, const float* __restrict__ XW, const float* __restrict__ gm,
+                                             const float* __restrict__ h0, long long ldh0, const float* __restrict__ Wh,
+                                             int act, float* __restrict__ hT, long long ldo, float* __restrict__ Z,
+                                             float* __restrict__ R, float* __restrict__ HH, float* __restrict__ HP,
+                                             float* __restrict__ RH) {
   extern __shared__ float sm[];
   // rows of the mirrored state are padded to a multiple of 4 floats (zero tail) so that any G keeps the 128-bit reads
   // aligned: G = user_embedding_dim + vertical_embedding_dim = 215 at the reference's defaults (task/paper.py:1204-1208)
@@ -157,11 +158,11 @@ __global__ void gru_fwd_kernel(int B, int W, int G, const float* __restrict__ XW
 // thread k reads WhT[c*G + k] coalesced.  Produces dA = d(loss)/d(pre-activations)
 // (B,W,3G) in gate order z,r,h (zero on masked steps) and dh0.
 template <int BT>
-__global__ void gru_bwd_kernel(int B, int W, int G, const float* __restrict__ gm, const float* __restrict__ Z,
-                               const float* __restrict__ R, const float* __restrict__ HH,
-                               const float* __restrict__ HP, const float* __restrict__ WhT, int act,
-                               const float* __restrict__ dhT, long long lddh, float* __restrict__ dA,
-                               float* __restrict__ dh0, long long lddh0) {
+__device__ __forceinline__ void gru_bwd_body(int B, int W, int G, const float* __restrict__ gm, const float* __restrict__ Z,
+                                             const float* __restrict__ R, const float* __restrict__ HH,
+                                             const float* __restrict__ HP, const float* __restrict__ WhT, int act,
+                                             const float* __restrict__ dhT, long long lddh, float* __restrict__ dA,
+                                             float* __restrict__ dh0, long long lddh0) {
   extern __shared__ float sm[];
   const int Gs = (G + 3) & ~3;      // padded row stride, zero tail (see the forward kernel)
   float* s_dah = sm;                // [BT][Gs]
@@ -287,6 +288,42 @@ __global__ void gru_bwd_kernel(int B, int W, int G, const float* __restrict__ gm
   }
 }
 
+// Two instances of each kernel.  GRU_BT = 8 rows per CTA keeps 8 states per thread in registers, which limits the CTA
+// to fewer threads than the widest G (140 registers: 448 threads forward).  Wider G takes the _wide instance: 4 rows per
+// CTA under __launch_bounds__(1024), so one thread per unit fits for every G <= 1024.
+constexpr int GRU_BT_WIDE = 4;
+
+template <int BT>
+__global__ void gru_fwd_kernel(int B, int W, int G, const float* __restrict__ XW, const float* __restrict__ gm,
+                               const float* __restrict__ h0, long long ldh0, const float* __restrict__ Wh, int act,
+                               float* __restrict__ hT, long long ldo, float* __restrict__ Z, float* __restrict__ R,
+                               float* __restrict__ HH, float* __restrict__ HP, float* __restrict__ RH) {
+  gru_fwd_body<BT>(B, W, G, XW, gm, h0, ldh0, Wh, act, hT, ldo, Z, R, HH, HP, RH);
+}
+__global__ void __launch_bounds__(1024)
+gru_fwd_kernel_wide(int B, int W, int G, const float* __restrict__ XW, const float* __restrict__ gm,
+                    const float* __restrict__ h0, long long ldh0, const float* __restrict__ Wh, int act,
+                    float* __restrict__ hT, long long ldo, float* __restrict__ Z, float* __restrict__ R,
+                    float* __restrict__ HH, float* __restrict__ HP, float* __restrict__ RH) {
+  gru_fwd_body<GRU_BT_WIDE>(B, W, G, XW, gm, h0, ldh0, Wh, act, hT, ldo, Z, R, HH, HP, RH);
+}
+
+template <int BT>
+__global__ void gru_bwd_kernel(int B, int W, int G, const float* __restrict__ gm, const float* __restrict__ Z,
+                               const float* __restrict__ R, const float* __restrict__ HH,
+                               const float* __restrict__ HP, const float* __restrict__ WhT, int act,
+                               const float* __restrict__ dhT, long long lddh, float* __restrict__ dA,
+                               float* __restrict__ dh0, long long lddh0) {
+  gru_bwd_body<BT>(B, W, G, gm, Z, R, HH, HP, WhT, act, dhT, lddh, dA, dh0, lddh0);
+}
+__global__ void __launch_bounds__(1024)
+gru_bwd_kernel_wide(int B, int W, int G, const float* __restrict__ gm, const float* __restrict__ Z,
+                    const float* __restrict__ R, const float* __restrict__ HH, const float* __restrict__ HP,
+                    const float* __restrict__ WhT, int act, const float* __restrict__ dhT, long long lddh,
+                    float* __restrict__ dA, float* __restrict__ dh0, long long lddh0) {
+  gru_bwd_body<GRU_BT_WIDE>(B, W, G, gm, Z, R, HH, HP, WhT, act, dhT, lddh, dA, dh0, lddh0);
+}
+
 __global__ void transpose_kernel(int rows, int cols, const float* __restrict__ in, float* __restrict__ out) {
   __shared__ float tile[32][33];
   int x = blockIdx.x * 32 + threadIdx.x, y0 = blockIdx.y * 32;
@@ -318,12 +355,18 @@ extern "C" int lstur_gru_fwd_streaming(int B, int W, int G, const float* XW, con
   LSTUR_REQUIRE(B >= 0 && W > 0 && G > 0 && G <= 1024, "lstur_gru_fwd_streaming");
   LSTUR_REQUIRE((Z && R && HH && HP && RH) || (!Z && !R && !HH && !HP && !RH), "lstur_gru_fwd_streaming");
   if (B == 0) return LSTUR_OK;
-  int threads = cdiv(G, 32) * 32;
-  size_t smem = (size_t)2 * GRU_BT * ((G + 3) & ~3) * sizeof(float);
-  if (smem > 48 * 1024)
-    cudaFuncSetAttribute(gru_fwd_kernel<GRU_BT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  gru_fwd_kernel<GRU_BT><<<cdiv(B, GRU_BT), threads, smem, stream>>>(B, W, G, XW, gm, h0, ldh0, Wh, rec_act, hT, ldo, Z,
-                                                                      R, HH, HP, RH);
+  static const int narrow_max = kernel_max_threads((const void*)gru_fwd_kernel<GRU_BT>);
+  const int threads = cdiv(G, 32) * 32;
+  const int bt = threads <= narrow_max ? GRU_BT : GRU_BT_WIDE;
+  const void* fn = bt == GRU_BT ? (const void*)gru_fwd_kernel<GRU_BT> : (const void*)gru_fwd_kernel_wide;
+  const size_t smem = (size_t)2 * bt * ((G + 3) & ~3) * sizeof(float);
+  if (smem > 48 * 1024) cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (bt == GRU_BT)
+    gru_fwd_kernel<GRU_BT><<<cdiv(B, bt), threads, smem, stream>>>(B, W, G, XW, gm, h0, ldh0, Wh, rec_act, hT, ldo, Z, R,
+                                                                    HH, HP, RH);
+  else
+    gru_fwd_kernel_wide<<<cdiv(B, bt), threads, smem, stream>>>(B, W, G, XW, gm, h0, ldh0, Wh, rec_act, hT, ldo, Z, R, HH,
+                                                                 HP, RH);
   LSTUR_CHECK_LAUNCH("lstur_gru_fwd_streaming");
   return LSTUR_OK;
 }
@@ -333,12 +376,18 @@ extern "C" int lstur_gru_bwd_streaming(int B, int W, int G, const float* gm, con
                              float* dA, float* dh0, long long lddh0, cudaStream_t stream) {
   LSTUR_REQUIRE(B >= 0 && W > 0 && G > 0 && G <= 1024, "lstur_gru_bwd_streaming");
   if (B == 0) return LSTUR_OK;
-  int threads = cdiv(G, 32) * 32;
-  size_t smem = (size_t)3 * GRU_BT * ((G + 3) & ~3) * sizeof(float);
-  if (smem > 48 * 1024)
-    cudaFuncSetAttribute(gru_bwd_kernel<GRU_BT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  gru_bwd_kernel<GRU_BT><<<cdiv(B, GRU_BT), threads, smem, stream>>>(B, W, G, gm, Z, R, HH, HP, WhT, rec_act, dhT, lddh,
-                                                                      dA, dh0, lddh0);
+  static const int narrow_max = kernel_max_threads((const void*)gru_bwd_kernel<GRU_BT>);
+  const int threads = cdiv(G, 32) * 32;
+  const int bt = threads <= narrow_max ? GRU_BT : GRU_BT_WIDE;
+  const void* fn = bt == GRU_BT ? (const void*)gru_bwd_kernel<GRU_BT> : (const void*)gru_bwd_kernel_wide;
+  const size_t smem = (size_t)3 * bt * ((G + 3) & ~3) * sizeof(float);
+  if (smem > 48 * 1024) cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (bt == GRU_BT)
+    gru_bwd_kernel<GRU_BT><<<cdiv(B, bt), threads, smem, stream>>>(B, W, G, gm, Z, R, HH, HP, WhT, rec_act, dhT, lddh, dA,
+                                                                    dh0, lddh0);
+  else
+    gru_bwd_kernel_wide<<<cdiv(B, bt), threads, smem, stream>>>(B, W, G, gm, Z, R, HH, HP, WhT, rec_act, dhT, lddh, dA, dh0,
+                                                                 lddh0);
   LSTUR_CHECK_LAUNCH("lstur_gru_bwd_streaming");
   return LSTUR_OK;
 }

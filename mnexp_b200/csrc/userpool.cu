@@ -240,11 +240,11 @@ __device__ __forceinline__ float lstm_act_grad(float y, int act) {
 }
 
 template <int BT>
-__global__ void lstm_fwd_kernel(int B, int W, int G, const float* __restrict__ XW, const float* __restrict__ gm,
-                                const float* __restrict__ Wh, int act, float* __restrict__ hT, long long ldo,
-                                float* __restrict__ SI, float* __restrict__ SF, float* __restrict__ SG,
-                                float* __restrict__ SO, float* __restrict__ SCP, float* __restrict__ SHP,
-                                float* __restrict__ STC) {
+__device__ __forceinline__ void lstm_fwd_body(int B, int W, int G, const float* __restrict__ XW, const float* __restrict__ gm,
+                                              const float* __restrict__ Wh, int act, float* __restrict__ hT, long long ldo,
+                                              float* __restrict__ SI, float* __restrict__ SF, float* __restrict__ SG,
+                                              float* __restrict__ SO, float* __restrict__ SCP, float* __restrict__ SHP,
+                                              float* __restrict__ STC) {
   extern __shared__ float sm[];   // [BT][G] previous h
   const int j = threadIdx.x, b0 = blockIdx.x * BT;
   const bool act_j = j < G;
@@ -313,11 +313,11 @@ __global__ void lstm_fwd_kernel(int B, int W, int G, const float* __restrict__ X
 
 // BPTT: dA (B,W,4G) in gate order i,f,c,o (zero on masked steps).  WhT = Wh transposed (4G, G).
 template <int BT>
-__global__ void lstm_bwd_kernel(int B, int W, int G, const float* __restrict__ gm, const float* __restrict__ SI,
-                                const float* __restrict__ SF, const float* __restrict__ SG, const float* __restrict__ SO,
-                                const float* __restrict__ SCP, const float* __restrict__ STC,
-                                const float* __restrict__ WhT, int act, const float* __restrict__ dhT, long long lddh,
-                                float* __restrict__ dA) {
+__device__ __forceinline__ void lstm_bwd_body(int B, int W, int G, const float* __restrict__ gm, const float* __restrict__ SI,
+                                              const float* __restrict__ SF, const float* __restrict__ SG,
+                                              const float* __restrict__ SO, const float* __restrict__ SCP,
+                                              const float* __restrict__ STC, const float* __restrict__ WhT, int act,
+                                              const float* __restrict__ dhT, long long lddh, float* __restrict__ dA) {
   extern __shared__ float sm[];   // [4][BT][G] gate pre-activation gradients of this step
   const int k = threadIdx.x, b0 = blockIdx.x * BT;
   const bool act_k = k < G;
@@ -376,6 +376,42 @@ __global__ void lstm_bwd_kernel(int B, int W, int G, const float* __restrict__ g
       if ((mbits >> i) & 1u) { dh[i] = dhp[i]; dc[i] = dcp[i]; }
     __syncthreads();
   }
+}
+
+// Two instances of each kernel, as for the streaming GRU (gru.cu): LSTM_BT = 8 rows per CTA for the widths its register
+// count can launch with one thread per unit, the _wide one (4 rows, __launch_bounds__(1024)) for every wider G <= 1024.
+constexpr int LSTM_BT_WIDE = 4;
+
+template <int BT>
+__global__ void lstm_fwd_kernel(int B, int W, int G, const float* __restrict__ XW, const float* __restrict__ gm,
+                                const float* __restrict__ Wh, int act, float* __restrict__ hT, long long ldo,
+                                float* __restrict__ SI, float* __restrict__ SF, float* __restrict__ SG,
+                                float* __restrict__ SO, float* __restrict__ SCP, float* __restrict__ SHP,
+                                float* __restrict__ STC) {
+  lstm_fwd_body<BT>(B, W, G, XW, gm, Wh, act, hT, ldo, SI, SF, SG, SO, SCP, SHP, STC);
+}
+__global__ void __launch_bounds__(1024)
+lstm_fwd_kernel_wide(int B, int W, int G, const float* __restrict__ XW, const float* __restrict__ gm,
+                     const float* __restrict__ Wh, int act, float* __restrict__ hT, long long ldo, float* __restrict__ SI,
+                     float* __restrict__ SF, float* __restrict__ SG, float* __restrict__ SO, float* __restrict__ SCP,
+                     float* __restrict__ SHP, float* __restrict__ STC) {
+  lstm_fwd_body<LSTM_BT_WIDE>(B, W, G, XW, gm, Wh, act, hT, ldo, SI, SF, SG, SO, SCP, SHP, STC);
+}
+
+template <int BT>
+__global__ void lstm_bwd_kernel(int B, int W, int G, const float* __restrict__ gm, const float* __restrict__ SI,
+                                const float* __restrict__ SF, const float* __restrict__ SG, const float* __restrict__ SO,
+                                const float* __restrict__ SCP, const float* __restrict__ STC,
+                                const float* __restrict__ WhT, int act, const float* __restrict__ dhT, long long lddh,
+                                float* __restrict__ dA) {
+  lstm_bwd_body<BT>(B, W, G, gm, SI, SF, SG, SO, SCP, STC, WhT, act, dhT, lddh, dA);
+}
+__global__ void __launch_bounds__(1024)
+lstm_bwd_kernel_wide(int B, int W, int G, const float* __restrict__ gm, const float* __restrict__ SI,
+                     const float* __restrict__ SF, const float* __restrict__ SG, const float* __restrict__ SO,
+                     const float* __restrict__ SCP, const float* __restrict__ STC, const float* __restrict__ WhT, int act,
+                     const float* __restrict__ dhT, long long lddh, float* __restrict__ dA) {
+  lstm_bwd_body<LSTM_BT_WIDE>(B, W, G, gm, SI, SF, SG, SO, SCP, STC, WhT, act, dhT, lddh, dA);
 }
 
 }  // namespace lstur
@@ -491,11 +527,18 @@ extern "C" int lstur_lstm_fwd(int B, int W, int G, const float* XW, const float*
   LSTUR_REQUIRE(B >= 0 && W > 0 && G > 0 && G <= 1024 && XW && gm && Wh && hT, "lstur_lstm_fwd");
   LSTUR_REQUIRE((SI && SF && SG && SO && SCP && SHP && STC) || (!SI && !SF && !SG && !SO && !SCP && !SHP && !STC), "lstur_lstm_fwd");
   if (B == 0) return LSTUR_OK;
+  static const int narrow_max = kernel_max_threads((const void*)lstm_fwd_kernel<LSTM_BT>);
   const int threads = cdiv(G, 32) * 32;
-  const size_t smem = (size_t)LSTM_BT * G * sizeof(float);
-  if (smem > 48 * 1024) cudaFuncSetAttribute(lstm_fwd_kernel<LSTM_BT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  lstm_fwd_kernel<LSTM_BT><<<cdiv(B, LSTM_BT), threads, smem, stream>>>(B, W, G, XW, gm, Wh, rec_act, hT, ldo, SI, SF, SG, SO,
-                                                                       SCP, SHP, STC);
+  const int bt = threads <= narrow_max ? LSTM_BT : LSTM_BT_WIDE;
+  const void* fn = bt == LSTM_BT ? (const void*)lstm_fwd_kernel<LSTM_BT> : (const void*)lstm_fwd_kernel_wide;
+  const size_t smem = (size_t)bt * G * sizeof(float);
+  if (smem > 48 * 1024) cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (bt == LSTM_BT)
+    lstm_fwd_kernel<LSTM_BT><<<cdiv(B, bt), threads, smem, stream>>>(B, W, G, XW, gm, Wh, rec_act, hT, ldo, SI, SF, SG, SO,
+                                                                      SCP, SHP, STC);
+  else
+    lstm_fwd_kernel_wide<<<cdiv(B, bt), threads, smem, stream>>>(B, W, G, XW, gm, Wh, rec_act, hT, ldo, SI, SF, SG, SO, SCP,
+                                                                  SHP, STC);
   LSTUR_CHECK_LAUNCH("lstur_lstm_fwd");
   return LSTUR_OK;
 }
@@ -505,11 +548,18 @@ extern "C" int lstur_lstm_bwd(int B, int W, int G, const float* gm, const float*
                               const float* dhT, long long lddh, float* dA, cudaStream_t stream) {
   LSTUR_REQUIRE(B >= 0 && W > 0 && G > 0 && G <= 1024 && gm && SI && SF && SG && SO && SCP && STC && WhT && dhT && dA, "lstur_lstm_bwd");
   if (B == 0) return LSTUR_OK;
+  static const int narrow_max = kernel_max_threads((const void*)lstm_bwd_kernel<LSTM_BT>);
   const int threads = cdiv(G, 32) * 32;
-  const size_t smem = (size_t)4 * LSTM_BT * G * sizeof(float);
-  if (smem > 48 * 1024) cudaFuncSetAttribute(lstm_bwd_kernel<LSTM_BT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  lstm_bwd_kernel<LSTM_BT><<<cdiv(B, LSTM_BT), threads, smem, stream>>>(B, W, G, gm, SI, SF, SG, SO, SCP, STC, WhT, rec_act, dhT,
-                                                                       lddh, dA);
+  const int bt = threads <= narrow_max ? LSTM_BT : LSTM_BT_WIDE;
+  const void* fn = bt == LSTM_BT ? (const void*)lstm_bwd_kernel<LSTM_BT> : (const void*)lstm_bwd_kernel_wide;
+  const size_t smem = (size_t)4 * bt * G * sizeof(float);
+  if (smem > 48 * 1024) cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (bt == LSTM_BT)
+    lstm_bwd_kernel<LSTM_BT><<<cdiv(B, bt), threads, smem, stream>>>(B, W, G, gm, SI, SF, SG, SO, SCP, STC, WhT, rec_act, dhT,
+                                                                      lddh, dA);
+  else
+    lstm_bwd_kernel_wide<<<cdiv(B, bt), threads, smem, stream>>>(B, W, G, gm, SI, SF, SG, SO, SCP, STC, WhT, rec_act, dhT, lddh,
+                                                                  dA);
   LSTUR_CHECK_LAUNCH("lstur_lstm_bwd");
   return LSTUR_OK;
 }
