@@ -475,11 +475,12 @@ void lstur_plan_destroy(lstur_plan* plan);
 int lstur_plan_invalidate_tables(lstur_plan* plan);
 size_t lstur_plan_workspace_bytes(const lstur_plan* plan);
 long long lstur_plan_dense_count(const lstur_plan* plan);
-/* name in {conv_w, conv_b, att_w, att_b, dense_w, dense_b, vert_emb, subvert_emb, gru_wx, gru_wh, gru_b,
- * con_w, con_b}; returns LSTUR_ERR_ARG if the tensor does not exist in this configuration. */
+/* offset (floats) and count of a dense tensor, by the names of LSTUR_DENSE_TENSORS (mnexp_b200/csrc/engine.cu);
+ * returns LSTUR_ERR_ARG if the tensor does not exist in this configuration. */
 int lstur_plan_dense_offset(const lstur_plan* plan, const char* name, long long* offset, long long* count);
-/* named views into the workspace after forward/backward (for tests and the Python shim):
- * tokens, pooled, doc_vec, hist_mask, user_vec, logits, probs, loss, d_user_rows, user_rows, n_user_rows */
+/* named views into the workspace after forward/backward (for tests and the Python shim), by the names of
+ * LSTUR_WS_REGIONS (mnexp_b200/csrc/engine.cu); returns LSTUR_ERR_ARG if the region does not exist in this
+ * configuration.  *ptr = workspace + the region's byte offset, *count = its 4-byte elements. */
 int lstur_plan_view(const lstur_plan* plan, void* workspace, const char* name, void** ptr, long long* count);
 
 /* Measurement hook: record the two CUDA events (cudaEvent_t) around one kernel of the step. */
@@ -506,14 +507,16 @@ int lstur_event_create(void** ev);
 int lstur_event_destroy(void* ev);
 int lstur_event_elapsed_ms(void* start_event, void* stop_event, float* ms);
 
-int lstur_forward(const lstur_plan* plan, const lstur_weights* w, const lstur_batch* b, void* workspace,
+/* Entry points that take a non-const plan record in it what later calls depend on: the seed, mode and title count of
+ * the last forward (the backward replays them) and which word table the workspace holds a 16-bit copy of. */
+int lstur_forward(lstur_plan* plan, const lstur_weights* w, const lstur_batch* b, void* workspace,
                   int training, unsigned seed, cudaStream_t stream);
 /* Vertical model of Seq2VecPaperSoftmaxDaysIdVertAlt (task/paper.py:1128-1136; plan with cls_nv > 0):
  * Dense(cls_nv, softmax)(doc_encoder(title)) + categorical cross-entropy on n <= B*(W+C) titles.  tokens (n,L), labels (n)
  * device ints.  Workspace views afterwards: vc_probs (n, cls_nv), vc_loss_rows (n), vc_loss (1).  The backward fills the
  * whole dense-gradient arena (zero outside vcls_w / vcls_b and the title-encoder tensors) and word_grad when the word table
  * trains; grad_scale = 1 / (global number of titles). */
-int lstur_title_cls_forward(const lstur_plan* plan, const lstur_weights* w, void* workspace, int n, const int* tokens,
+int lstur_title_cls_forward(lstur_plan* plan, const lstur_weights* w, void* workspace, int n, const int* tokens,
                             const int* labels, int training, unsigned seed, cudaStream_t stream);
 int lstur_title_cls_backward(const lstur_plan* plan, const lstur_weights* w, void* workspace, float* dgrad,
                              float* word_grad, float grad_scale, cudaStream_t stream);
@@ -531,13 +534,13 @@ int lstur_backward_w(const lstur_plan* plan, const lstur_weights* w, const lstur
  * (doc_ids on the device, weights->doc_tokens required); lstur_forward_docvecs gathers history / candidate vectors from
  * doc_vec_table (n_rows, ld == document-vector width) — an all-zero row (unknown / pad document) is a masked history
  * slot — and leaves probs / logits / user_vec in the workspace like lstur_forward. */
-int lstur_encode_docs(const lstur_plan* plan, const lstur_weights* weights, void* workspace, int n, const int* doc_ids,
+int lstur_encode_docs(lstur_plan* plan, const lstur_weights* weights, void* workspace, int n, const int* doc_ids,
                       float* doc_vec_out, long long ldo, cudaStream_t stream);
 /* The same encoder on explicit token rows (n, L) instead of document ids: `doc_encoder.predict(titles)`, the layer
  * TestPipeline fetches with get_layer('doc_encoder') (task/test_pipeline.py:27-35, task/paper.py:160). */
-int lstur_encode_titles(const lstur_plan* plan, const lstur_weights* weights, void* workspace, int n, const int* tokens,
+int lstur_encode_titles(lstur_plan* plan, const lstur_weights* weights, void* workspace, int n, const int* tokens,
                         float* doc_vec_out, long long ldo, cudaStream_t stream);
-int lstur_forward_docvecs(const lstur_plan* plan, const lstur_weights* weights, const lstur_batch* batch, void* workspace,
+int lstur_forward_docvecs(lstur_plan* plan, const lstur_weights* weights, const lstur_batch* batch, void* workspace,
                           const float* doc_vec_table, long long ld, int n_rows, cudaStream_t stream);
 /* Ranking of whole impressions (the evaluation pass of Seq2VecPaperSoftmax.callback, task/paper.py:497-524) against
  * cached document vectors doc_vec_table (n_rows, document-vector width), on an inference plan (save_for_backward = 0).
@@ -548,7 +551,7 @@ int lstur_forward_docvecs(const lstur_plan* plan, const lstur_weights* weights, 
  * LSTUR_ERR_ARG.  A history slot is masked when its document's title is all zero tokens (weights->doc_tokens required),
  * as lstur_forward masks it; a candidate keeps its row of the table.  cand_off (n_impr + 1 ints) is HOST memory: the
  * chunks are cut on the host and each chunk's offsets copied to the device.  Every other array is on the device. */
-int lstur_score_impressions(const lstur_plan* plan, const lstur_weights* weights, void* workspace, int n_impr,
+int lstur_score_impressions(lstur_plan* plan, const lstur_weights* weights, void* workspace, int n_impr,
                             const int* user, const int* hist_doc, const int* cand_off, const int* cand_doc,
                             const float* doc_vec_table, int n_rows, float* scores_out, cudaStream_t stream);
 

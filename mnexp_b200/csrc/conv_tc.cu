@@ -1100,8 +1100,6 @@ __global__ void wgrad_reduce_kernel(int E, int Ep, int F, int splits, int rows_t
 }  // namespace lstur
 
 // ======================================================================== host side
-#include "plan.h"
-
 using namespace lstur;
 
 // Padded embedding width (multiple of the 64-element K block).
@@ -1247,41 +1245,8 @@ extern "C" int lstur_news_conv_tc_fwd_m(int n_titles, int L, int E, int F, int V
   p.xmask = (uint8_t*)xmask_out;
   p.n_dev = n_titles_dev; p.title_idx = title_idx;
   p.trace = (long long*)g_tc_trace_ptr;
-  RC(tc_launch_conv(p, L, fp16 != 0, p.drop_thr16 != 0, tc::MODE_FWD, max_ctas, stream, "lstur_news_conv_tc_fwd"));
-  return LSTUR_OK;
+  return tc_launch_conv(p, L, fp16 != 0, p.drop_thr16 != 0, tc::MODE_FWD, max_ctas, stream, "lstur_news_conv_tc_fwd");
 }
-
-extern "C" int lstur_news_encoder_tc_fwd_internal(const lstur_plan* p, const lstur_weights* w, void* ws, int n_titles,
-                                                  int training, unsigned seed, cudaStream_t st) {
-  const lstur_config& c = p->c;
-  void* emb = W<void>(p, ws, "emb_bf16");
-  void* wimg = W<void>(p, ws, "wimg");
-  LSTUR_REQUIRE(emb && wimg, "lstur_news_encoder_tc_fwd_internal");
-  const int fp16 = c.precision == LSTUR_PREC_FP16_TC;
-  if (p->emb16_src != (const void*)w->word_emb || p->emb16_dst != emb) {
-    RC(lstur_pack_word_emb_16(c.V, c.E, w->word_emb, emb, fp16, st));
-    const_cast<lstur_plan*>(p)->emb16_src = w->word_emb;
-    const_cast<lstur_plan*>(p)->emb16_dst = emb;
-  }
-  RC(lstur_pack_conv_w_tc(c.E, c.F, DP(p, w->dense, "conv_w"), wimg, fp16, st));
-  // Live titles only: an all-pad title (left padding of a short history) pools to exactly 0 and back-propagates exactly 0,
-  // so the kernels run over the compacted title list; pooled rows of the dead titles are zeroed here.
-  int* n_live = W<int>(p, ws, "n_live");
-  int* live_idx = W<int>(p, ws, "live_idx");
-  int* tok_c = W<int>(p, ws, "tokens_c");
-  RC(lstur_compact_titles(n_titles, c.L, W<int>(p, ws, "tokens"), W<int>(p, ws, "title_flags"), live_idx, n_live, tok_c, st));
-  cudaMemsetAsync(W<float>(p, ws, "pooled"), 0, (size_t)n_titles * c.F * sizeof(float), st);
-  PROBE_BEGIN(p, LSTUR_PROBE_CONV_FWD, st);
-  // a training forward leaves the X-dropout keep bits for the weight-gradient kernel (workspace region "xmask")
-  void* xm = (training && c.dropout > 0.f && n_titles == p->N) ? W<void>(p, ws, "xmask") : nullptr;
-  RC(lstur_news_conv_tc_fwd_m(n_titles, c.L, c.E, c.F, c.V, tok_c, emb, wimg, DP(p, w->dense, "conv_b"),
-                              DP(p, w->dense, "att_w"), DP(p, w->dense, "att_b"), W<void>(p, ws, "C16"),
-                              W<float>(p, ws, "pooled"), W<float>(p, ws, "att_a"), W<float>(p, ws, "att_w"),
-                              training ? c.dropout : 0.f, seed, fp16, 0, xm, n_live, live_idx, st));
-  PROBE_END(p, LSTUR_PROBE_CONV_FWD, st);
-  return LSTUR_OK;
-}
-
 
 // ---- conv input gradient (word-table training: keras Embedding(trainable=True), task/paper.py:132-138) ----------
 extern "C" int lstur_tc_wgrad_groups(int F);
@@ -1314,8 +1279,7 @@ extern "C" int lstur_conv_dgrad_tc(int n_titles, int L, int E, int F, const void
   p.n_dev = n_titles_dev;
   p.inv_keep = 1.f;
   p.trace = nullptr;
-  RC(tc_launch_conv(p, L, fp16 != 0, false, tc::MODE_DGRAD, max_ctas, stream, "lstur_conv_dgrad_tc"));
-  return LSTUR_OK;
+  return tc_launch_conv(p, L, fp16 != 0, false, tc::MODE_DGRAD, max_ctas, stream, "lstur_conv_dgrad_tc");
 }
 
 // ---- wgrad host side ------------------------------------------------------------------------------
