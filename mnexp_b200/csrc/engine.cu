@@ -294,6 +294,8 @@ extern "C" int lstur_plan_create(const lstur_config* cfg, lstur_plan** out) {
 
   LSTUR_REQUIRE(!c.trainable_word_emb || (c.save_for_backward && c.E % 4 == 0 && c.E <= 512),
                 "lstur_plan_create(trainable word table: training plan, E % 4 == 0, E <= 512)");
+  LSTUR_REQUIRE(!c.save_for_backward || prec_tc(c) || c.F <= 1024,
+                "lstur_plan_create(fp32 training plan: F <= 1024, the limit of the attention backward)");
   lstur_plan* p = new lstur_plan();
   p->c = c;
   p->c.Dd = Dd;

@@ -11,8 +11,10 @@
 // finishes every token whose positions it contains entirely and hands at most two partial rows to the next level.  A
 // step is therefore bit-reproducible, and the heavy tokens of a Zipf vocabulary (one token can own > 10 % of all
 // positions) are spread over many warps instead of serialising on one.
-// Positions whose gradient is identically zero are dropped before the sort: a pad position that has no real token
-// within the conv window (dPre is exactly 0 under the pad mask, task/paper.py:150-155).
+// Positions whose gradient is identically zero are dropped before the sort: a pad position that no conv output over a
+// real token reads (dPre is exactly 0 under the pad mask, task/paper.py:150-155).  With the TF 'SAME' halo,
+// pl = (KS-1)/2, output m reads positions m-pl .. m+KS-1-pl, so position t is live when a token in
+// [t-(KS-1-pl), t+pl] of its title is non-zero: KS-1-pl positions back, pl forward (KS = 4: two back, one forward).
 #include "common.cuh"
 
 namespace lstur {
@@ -25,15 +27,17 @@ constexpr int BATCH = 4;                           // rows whose loads a warp ke
 constexpr int RED_THREADS = 256;                   // 8 warps = 8 work items per block
 
 // ---- keys: token id of every live position, V for dead ones (sorted to the end and ignored) --------------------------
-__global__ void keys_kernel(long long n_pos, int L, int V, const int* __restrict__ tok, int* __restrict__ keys,
-                            int* __restrict__ pos, const int* __restrict__ n_titles_dev) {
+// back / fwd: reach of the conv window on each side (KS-1-pl and pl)
+__global__ void keys_kernel(long long n_pos, int L, int V, int back, int fwd, const int* __restrict__ tok,
+                            int* __restrict__ keys, int* __restrict__ pos, const int* __restrict__ n_titles_dev) {
   long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= n_pos) return;
   const int t = (int)(p % L);
   const bool in_range = !n_titles_dev || p < (long long)__ldg(n_titles_dev) * L;   // compacted title list: rows beyond are unused
   int id = in_range ? tok[p] : 0;
-  const int prev = (in_range && t > 0) ? tok[p - 1] : 0, next = (in_range && t + 1 < L) ? tok[p + 1] : 0;
-  const bool live = (id != 0) || (prev != 0) || (next != 0);
+  bool live = id != 0;
+  if (in_range)
+    for (int s = max(t - back, 0), e = min(t + fwd, L - 1); s <= e && !live; ++s) live = tok[p - t + s] != 0;
   id = (id < 0 || id >= V) ? 0 : id;          // out-of-range ids read row 0, like the forward gather
   keys[p] = live ? id : V;
   pos[p] = (int)p;
@@ -365,14 +369,15 @@ static Ws carve(void* base, long long n, int V, int E) {
 }
 
 template <typename SRC>
-static int run(SRC src, long long n, int L, int V, int E, const int* tokens, const int* n_titles_dev, float scale,
+static int run(SRC src, long long n, int L, int KS, int V, int E, const int* tokens, const int* n_titles_dev, float scale,
                float* d_word_emb, void* workspace, size_t workspace_bytes, cudaStream_t st, const char* name) {
   LSTUR_REQUIRE(n >= 0 && n < (1LL << 31) && L >= 1 && V >= 1 && E >= 4 && E % 4 == 0 && E <= 512 && tokens && d_word_emb, name);
   Ws w = carve(workspace, n, V, E);
   LSTUR_REQUIRE(workspace != nullptr && workspace_bytes >= w.bytes, name);
   cudaMemsetAsync(d_word_emb, 0, (size_t)V * E * sizeof(float), st);
   if (n == 0) return LSTUR_OK;
-  keys_kernel<<<cdiv(n, 256), 256, 0, st>>>(n, L, V, tokens, w.keys_a, w.pos_a, n_titles_dev);
+  const int pl = (KS - 1) / 2;
+  keys_kernel<<<cdiv(n, 256), 256, 0, st>>>(n, L, V, KS - 1 - pl, pl, tokens, w.keys_a, w.pos_a, n_titles_dev);
   LSTUR_CHECK_LAUNCH(name);
   int bits = 1;
   while ((1LL << bits) <= V) ++bits;              // keys are 0 .. V inclusive
@@ -438,8 +443,8 @@ extern "C" int lstur_word_grad_scatter_16(int n_titles, int L, int E, int V, con
                                           size_t workspace_bytes, const int* n_titles_dev, cudaStream_t stream) {
   LSTUR_REQUIRE(n_titles >= 0 && dx16 != nullptr, "lstur_word_grad_scatter_16");
   wg::Src16 s{(const uint16_t*)dx16, (const uint8_t*)xmask, lstur_tc_padded_e(E), fp16};
-  return wg::run(s, (long long)n_titles * L, L, V, E, tokens, n_titles_dev, scale, d_word_emb, workspace, workspace_bytes,
-                 stream, "lstur_word_grad_scatter_16");
+  return wg::run(s, (long long)n_titles * L, L, 3, V, E, tokens, n_titles_dev, scale, d_word_emb, workspace, workspace_bytes,
+                 stream, "lstur_word_grad_scatter_16");     // the tensor-core conv has KS = 3
 }
 
 // fp32 mode: dXp (n_titles, L+KS-1, E) = gradient of the zero-haloed title buffer of lstur_embed_gather_pad; the X-dropout
@@ -449,6 +454,6 @@ extern "C" int lstur_word_grad_scatter_f32(int n_titles, int L, int KS, int E, i
                                            size_t workspace_bytes, cudaStream_t stream) {
   LSTUR_REQUIRE(n_titles >= 0 && dXp != nullptr && KS >= 1 && dropout >= 0.f && dropout < 1.f, "lstur_word_grad_scatter_f32");
   wg::Src32 s{dXp, L, L + KS - 1, (KS - 1) / 2, E, dropout > 0.f ? dropout_threshold(dropout) : 0u, seed};
-  return wg::run(s, (long long)n_titles * L, L, V, E, tokens, nullptr, scale / (1.f - dropout), d_word_emb, workspace,
+  return wg::run(s, (long long)n_titles * L, L, KS, V, E, tokens, nullptr, scale / (1.f - dropout), d_word_emb, workspace,
                  workspace_bytes, stream, "lstur_word_grad_scatter_f32");
 }

@@ -44,11 +44,13 @@ def case(sh, arch='igru', seed=0, relu_open=False):
     return tok, P, b
 
 
+@pytest.mark.parametrize('k', [3, 2, 4, 5])
 @pytest.mark.parametrize('dropout', [0.0, 0.2])
-def test_word_table_gradient_fp32(lib, dropout):
-    """fp32 mode: d word_emb == autograd to <= 5e-5, bit-reproducible run to run"""
+def test_word_table_gradient_fp32(lib, dropout, k):
+    """fp32 mode: d word_emb == autograd to <= 5e-5, bit-reproducible run to run, at filter widths 2 .. 5 (an even
+    width's 'same' halo reaches one more position back than forward)"""
     from mnexp_b200.engine import LsturEngine
-    sh = synth.Shape('wt', 50, 80, 120, L=7, W=5, K=2, B=6, E=12, F=16, U=8)
+    sh = synth.Shape('wt', 50, 80, 120, L=7, W=5, K=2, B=6, E=12, F=16, U=8, k=k)
     tok, P, b = case(sh)
     eng = LsturEngine(P, sh.B, sh.W, 1 + sh.K, sh.L, arch='igru', doc_tokens=tok, dropout=dropout, trainable_word_emb=True)
     db = eng.to_device_batch(b)
