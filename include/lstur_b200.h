@@ -276,6 +276,14 @@ int lstur_assemble_samples(int B, int W, int K, const int* sample_click, const i
                            const int* click_user, const int* click_time, long long expire_seconds, const int* stream_off,
                            const int* stream_docs, const int* neg_off, const int* neg_docs, unsigned seed, long long row0,
                            int* user_out, int* hist_doc_out, int* cand_doc_out, cudaStream_t stream);
+/* Cook's batches from its interned .npz rows (CookModel.fit / _batch, task/cook.py via main.py:147-215 `model.fit`):
+ * row b < m of the batch is sample s = pos[b], rows b >= m (the ragged last batch) repeat pos[0] with an all-zero label
+ * row.  Per sample tables -> outputs: user (n) -> user_out (B), scale (n) -> scale_out (B), hist_doc (n, W) ->
+ * hist_doc_out (B, W), cand_doc (n, C) -> cand_doc_out (B, C), label (n, C) -> label_out (B, C).  A NULL table skips its
+ * output.  1 <= m <= B. */
+int lstur_gather_samples(int B, int m, int W, int C, const int* pos, const int* user, const float* scale,
+                         const int* hist_doc, const int* cand_doc, const float* label, int* user_out, float* scale_out,
+                         int* hist_doc_out, int* cand_doc_out, float* label_out, cudaStream_t stream);
 /* lstur_assemble_samples(sample_hist_end = NULL, click_time = NULL, row0 = 0): training samples, no time window. */
 int lstur_assemble_batch(int B, int W, int K, const int* sample_click, const int* idx, const int* click_user,
                          const int* stream_off, const int* stream_docs, const int* neg_off, const int* neg_docs,
@@ -359,6 +367,27 @@ int lstur_lstm_fwd(int B, int W, int G, const float* XW, const float* gm, const 
 int lstur_lstm_bwd(int B, int W, int G, const float* gm, const float* SI, const float* SF, const float* SG,
                    const float* SO, const float* SCP, const float* STC, const float* WhT, int rec_act, const float* dhT,
                    long long lddh, float* dA, cudaStream_t stream);
+
+/* Row interning of Cook's token rows (ch_title / ch_vert / ch_subvert and cd_title / cd_vert / cd_subvert of the .npz
+ * files, task/cook.py:14-28) into a document table.  Key of row r: tokens[r, 0..L), vert[r], subvert[r] (a NULL column
+ * reads 0).  ids[r] (n): 0 for the all-zero key, else 1, 2, ... in the order of each key's first row; two rows get the same
+ * id iff their keys are equal in every column (a stable radix sort of the positions by the columns, no hashing).
+ * first_row (n + 1 ints): first_row[u] = the first row with id u, for 1 <= u < *n_unique.  *n_unique (HOST int) = 1 +
+ * the number of distinct non-zero keys.  Token values are kept verbatim (ids >= V included).  The call waits for the
+ * stream twice (the columns' value ranges, then the count).  workspace: lstur_intern_workspace_bytes(n, L) bytes.
+ * lstur_intern_table: doc_tokens (n_unique, L), doc_vert, doc_subvert (n_unique, each may be NULL) = the key of
+ * first_row[u], row 0 all zero: doc_tokens[ids[r]] == tokens[r]. */
+size_t lstur_intern_workspace_bytes(long long n, int L);
+int lstur_intern_rows(int n, int L, const int* tokens, const int* vert, const int* subvert, int* ids, int* first_row,
+                      int* n_unique, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+int lstur_intern_table(int n_unique, int L, const int* tokens, const int* vert, const int* subvert, const int* first_row,
+                       int* doc_tokens, int* doc_vert, int* doc_subvert, cudaStream_t stream);
+/* User groups of Cook's test rows (one candidate per row; CookModel.predict over Cook.test(), task/cook.py via main.py:216-
+ * 224): row i starts a group when i == 0 or its user, scale (bitwise; NULL: not compared) or history row hist_doc[i, 0..W)
+ * differs from row i-1's.  starts (n) <- the first rows of the groups in order, *n_groups (HOST int) <- their count; the
+ * call waits for the stream.  workspace: lstur_intern_workspace_bytes(n, 0) bytes. */
+int lstur_group_rows(int n, int W, const int* user, const float* scale, const int* hist_doc, int* starts, int* n_groups,
+                     void* workspace, size_t workspace_bytes, cudaStream_t stream);
 
 /* Per-impression AUC / nDCG@10 / nDCG@5 / MRR (Seq2VecPaperSoftmax.callback, task/paper.py:497-524; utils.py:106-124;
  * sklearn roc_auc_score): offsets (n_impr+1) index scores / labels; out (n_impr, 4); ties ordered by descending index. */
@@ -550,10 +579,14 @@ int lstur_forward_docvecs(lstur_plan* plan, const lstur_weights* weights, const 
  * impression, on chunks of at most B impressions and B*C pairs; an impression of more than B*C candidates is
  * LSTUR_ERR_ARG.  A history slot is masked when its document's title is all zero tokens (weights->doc_tokens required),
  * as lstur_forward masks it; a candidate keeps its row of the table.  cand_off (n_impr + 1 ints) is HOST memory: the
- * chunks are cut on the host and each chunk's offsets copied to the device.  Every other array is on the device. */
+ * chunks are cut on the host and each chunk's offsets copied to the device.  Every other array is on the device.
+ * user_scale / user_scale2 (n_impr floats each, or NULL): the per-impression multipliers of the user embedding that
+ * lstur_batch.user_scale / user_scale2 are in lstur_forward — Cook's test model scales the id embedding by idx_mask
+ * (task/cook.py:139-142), so an out-of-vocabulary user scores with a zero id vector.  NULL: no multiplier. */
 int lstur_score_impressions(lstur_plan* plan, const lstur_weights* weights, void* workspace, int n_impr,
-                            const int* user, const int* hist_doc, const int* cand_off, const int* cand_doc,
-                            const float* doc_vec_table, int n_rows, float* scores_out, cudaStream_t stream);
+                            const int* user, const float* user_scale, const float* user_scale2, const int* hist_doc,
+                            const int* cand_off, const int* cand_doc, const float* doc_vec_table, int n_rows,
+                            float* scores_out, cudaStream_t stream);
 
 #ifdef __cplusplus
 }

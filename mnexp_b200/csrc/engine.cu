@@ -45,7 +45,7 @@ void set_error(const char* fmt, ...) {
   X(float, dA) X(float, dh0) X(float, d_cat) X(float, sc_dhid) X(float, sc_whid) X(float, sc_dcat)                     \
   X(float, sc_dlogit) X(float, sc_scratch) X(float, sc_duh) X(float, sc_ddh) X(int, sorted_pos) X(int, user_rows)      \
   X(int, seg_start) X(int, inverse) X(int, n_user_rows) X(float, d_user_rows) X(float, d_u0) X(int, ev_user)           \
-  X(int, ev_off) X(int, ev_pair_row) X(void, gemm_ws) X(float, colsum_ws)
+  X(float, ev_scale) X(float, ev_scale2) X(int, ev_off) X(int, ev_pair_row) X(void, gemm_ws) X(float, colsum_ws)
 
 // Tensors of the dense-parameter arena, in layout order; lstur_plan_dense_offset serves them by name.
 #define LSTUR_DENSE_TENSORS(X)                                                                                          \
@@ -569,8 +569,10 @@ extern "C" int lstur_plan_create(const lstur_config* cfg, lstur_plan** out) {
     if (con_dense) track_gemm(p, G + Uc, c.U, (int)B);
   }
   if (has_rnn) track_gemm(p, (int)Nh, NG * G, D);
-  if (!bw) {   // lstur_score_impressions: one chunk's users, rebased candidate offsets and pair -> impression rows
+  if (!bw) {   // lstur_score_impressions: one chunk's users and their scales, rebased candidate offsets and pair -> impression rows
     add_ws(p, r.ev_user, B);
+    add_ws(p, r.ev_scale, B);
+    add_ws(p, r.ev_scale2, B);
     add_ws(p, r.ev_off, B + 1);
     add_ws(p, r.ev_pair_row, p->Nc);
   }
@@ -1010,8 +1012,9 @@ extern "C" int lstur_forward_docvecs(lstur_plan* p, const lstur_weights* w, cons
 // copied to the device); every other array is on the device.  A history slot is masked when its document's title is all
 // zero tokens (weights->doc_tokens), as in lstur_forward; a candidate keeps its table row whatever its title.
 extern "C" int lstur_score_impressions(lstur_plan* p, const lstur_weights* w, void* ws, int n_impr, const int* user,
-                                       const int* hist_doc, const int* cand_off, const int* cand_doc,
-                                       const float* doc_vec_table, int n_rows, float* scores_out, cudaStream_t st) {
+                                       const float* user_scale, const float* user_scale2, const int* hist_doc,
+                                       const int* cand_off, const int* cand_doc, const float* doc_vec_table, int n_rows,
+                                       float* scores_out, cudaStream_t st) {
   LSTUR_REQUIRE(p && w && ws && w->dense && w->doc_tokens && n_impr >= 0, "lstur_score_impressions");
   LSTUR_REQUIRE(n_impr == 0 || (user && hist_doc && cand_off && cand_doc && doc_vec_table && n_rows > 0 && scores_out),
                 "lstur_score_impressions");
@@ -1042,6 +1045,10 @@ extern "C" int lstur_score_impressions(lstur_plan* p, const lstur_weights* w, vo
   lstur_batch b;
   memset(&b, 0, sizeof(b));
   b.user = ev_user;
+  float* ev_scale = user_scale ? p->ws.ev_scale(ws) : nullptr;
+  float* ev_scale2 = user_scale2 ? p->ws.ev_scale2(ws) : nullptr;
+  b.user_scale = ev_scale;
+  b.user_scale2 = ev_scale2;
   std::vector<int> off;
   p->last_training = 0;
   for (int i0 = 0; i0 < n_impr;) {
@@ -1054,6 +1061,14 @@ extern "C" int lstur_score_impressions(lstur_plan* p, const lstur_weights* w, vo
     // users and history rows of the chunk; rows m..B are padding (user 0, all history slots masked)
     cudaMemsetAsync(ev_user, 0, (size_t)B * 4, st);
     cudaMemcpyAsync(ev_user, user + i0, (size_t)m * 4, cudaMemcpyDeviceToDevice, st);
+    if (ev_scale) {
+      cudaMemsetAsync(ev_scale, 0, (size_t)B * 4, st);
+      cudaMemcpyAsync(ev_scale, user_scale + i0, (size_t)m * 4, cudaMemcpyDeviceToDevice, st);
+    }
+    if (ev_scale2) {
+      cudaMemsetAsync(ev_scale2, 0, (size_t)B * 4, st);
+      cudaMemcpyAsync(ev_scale2, user_scale2 + i0, (size_t)m * 4, cudaMemcpyDeviceToDevice, st);
+    }
     const long long nh = (long long)m * c.W;
     RC(lstur_token_gather((int)nh, L, c.n_docs, w->doc_tokens, hist_doc + (size_t)i0 * c.W, tok, st));
     RC(lstur_row_gather((int)nh, D, n_rows, doc_vec_table, hist_doc + (size_t)i0 * c.W, nullptr, docv, D, st));

@@ -281,6 +281,33 @@ __global__ void __launch_bounds__(1024) mask_compact_kernel(int N, const int* __
   }
 }
 
+// Rows of a sample table by position (Cook's interned .npz, task/cook.py:60-90): row b of the batch is sample
+// s = pos[b] for b < m and pos[0] for the padding rows b >= m of a ragged last batch, whose label row is zero.  One thread
+// per output element; a NULL table leaves its output alone.
+__global__ void gather_samples_kernel(int B, int m, int W, int C, const int* __restrict__ pos, const int* __restrict__ user,
+                                      const float* __restrict__ scale, const int* __restrict__ hist_doc,
+                                      const int* __restrict__ cand_doc, const float* __restrict__ label,
+                                      int* __restrict__ user_out, float* __restrict__ scale_out, int* __restrict__ hist_out,
+                                      int* __restrict__ cand_out, float* __restrict__ label_out) {
+  const int per = 2 + W + 2 * C;               // user, scale, W history slots, C candidates, C labels
+  const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= (long long)B * per) return;
+  const int b = (int)(e / per), j = (int)(e % per);
+  const long long s = pos[b < m ? b : 0];
+  if (j == 0) {
+    if (user) user_out[b] = user[s];
+  } else if (j == 1) {
+    if (scale) scale_out[b] = scale[s];
+  } else if (j < 2 + W) {
+    if (hist_doc) hist_out[(long long)b * W + j - 2] = hist_doc[s * W + j - 2];
+  } else if (j < 2 + W + C) {
+    if (cand_doc) cand_out[(long long)b * C + j - 2 - W] = cand_doc[s * C + j - 2 - W];
+  } else if (label) {
+    const int c = j - 2 - W - C;
+    label_out[(long long)b * C + c] = b < m ? label[s * C + c] : 0.f;
+  }
+}
+
 }  // namespace lstur
 
 using namespace lstur;
@@ -413,4 +440,18 @@ extern "C" int lstur_assemble_batch(int B, int W, int K, const int* sample_click
                                     unsigned seed, int* user_out, int* hist_doc_out, int* cand_doc_out, cudaStream_t stream) {
   return lstur_assemble_samples(B, W, K, sample_click, nullptr, idx, click_user, nullptr, 0, stream_off, stream_docs, neg_off,
                                 neg_docs, seed, 0, user_out, hist_doc_out, cand_doc_out, stream);
+}
+
+extern "C" int lstur_gather_samples(int B, int m, int W, int C, const int* pos, const int* user, const float* scale,
+                                    const int* hist_doc, const int* cand_doc, const float* label, int* user_out,
+                                    float* scale_out, int* hist_doc_out, int* cand_doc_out, float* label_out,
+                                    cudaStream_t stream) {
+  LSTUR_REQUIRE(B >= 0 && W >= 0 && C >= 0 && (B == 0 || (m >= 1 && m <= B && pos)), "lstur_gather_samples");
+  LSTUR_REQUIRE((!user || user_out) && (!scale || scale_out) && (!hist_doc || hist_doc_out) && (!cand_doc || cand_doc_out) &&
+                (!label || label_out), "lstur_gather_samples");
+  if (B == 0) return LSTUR_OK;
+  gather_samples_kernel<<<cdiv((long long)B * (2 + W + 2 * C), 256), 256, 0, stream>>>(
+      B, m, W, C, pos, user, scale, hist_doc, cand_doc, label, user_out, scale_out, hist_doc_out, cand_doc_out, label_out);
+  LSTUR_CHECK_LAUNCH("lstur_gather_samples");
+  return LSTUR_OK;
 }

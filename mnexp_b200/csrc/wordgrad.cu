@@ -15,13 +15,11 @@
 // real token reads (dPre is exactly 0 under the pad mask, task/paper.py:150-155).  With the TF 'SAME' halo,
 // pl = (KS-1)/2, output m reads positions m-pl .. m+KS-1-pl, so position t is live when a token in
 // [t-(KS-1-pl), t+pl] of its title is non-zero: KS-1-pl positions back, pl forward (KS = 4: two back, one forward).
-#include "common.cuh"
+#include "radix.cuh"
 
 namespace lstur {
 namespace wg {
 
-constexpr int RB = 9, RADIX = 1 << RB;             // radix-sort digit
-constexpr int SORT_THREADS = 256, SORT_ITEMS = 8, SORT_CH = SORT_THREADS * SORT_ITEMS;
 constexpr int R = 64;                              // rows (or piece slots) walked by one warp
 constexpr int BATCH = 4;                           // rows whose loads a warp keeps in flight
 constexpr int RED_THREADS = 256;                   // 8 warps = 8 work items per block
@@ -57,21 +55,6 @@ __global__ void __launch_bounds__(SORT_THREADS) radix_hist_kernel(const int* __r
   }
   __syncthreads();
   for (int b = threadIdx.x; b < RADIX; b += SORT_THREADS) ghist[(long long)b * nblk + blockIdx.x] = h[b];
-}
-
-__device__ __forceinline__ int block_inclusive_scan_256(int v, int* sm /* 8 ints */) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const int u = __shfl_up_sync(0xffffffffu, v, o);
-    if (lane >= o) v += u;
-  }
-  if (lane == 31) sm[warp] = v;
-  __syncthreads();
-  int add = 0;
-  for (int w = 0; w < warp; ++w) add += sm[w];
-  __syncthreads();
-  return v + add;
 }
 
 // row b of ghist (the digit's counts per block) -> exclusive prefix over the blocks; bintot[b] = the digit's total
@@ -150,6 +133,30 @@ __global__ void __launch_bounds__(SORT_THREADS) radix_scatter_kernel(const int* 
       pos_out[dst] = ps[r];
     }
   }
+}
+
+int radix_sort_pairs(int** keys, int** pos, int** keys_tmp, int** pos_tmp, long long n, int bits, int* ghist, int* bintot,
+                     cudaStream_t st, const char* name) {
+  if (n <= 0) return LSTUR_OK;
+  const int nblk = (int)sort_blocks(n);
+  for (int shift = 0; shift < bits; shift += RB) {
+    radix_hist_kernel<<<nblk, SORT_THREADS, 0, st>>>(*keys, n, shift, nblk, ghist);
+    LSTUR_CHECK_LAUNCH(name);
+    radix_rowscan_kernel<<<RADIX, 256, 0, st>>>(ghist, nblk, bintot);
+    LSTUR_CHECK_LAUNCH(name);
+    radix_scatter_kernel<<<nblk, SORT_THREADS, 0, st>>>(*keys, *pos, *keys_tmp, *pos_tmp, n, shift, nblk, ghist, bintot);
+    LSTUR_CHECK_LAUNCH(name);
+    int* t = *keys; *keys = *keys_tmp; *keys_tmp = t;
+    t = *pos; *pos = *pos_tmp; *pos_tmp = t;
+  }
+  return LSTUR_OK;
+}
+
+int exclusive_scan_rows(int* rows, int n_rows, int len, int* totals, cudaStream_t st, const char* name) {
+  if (n_rows <= 0) return LSTUR_OK;
+  radix_rowscan_kernel<<<n_rows, 256, 0, st>>>(rows, len, totals);
+  LSTUR_CHECK_LAUNCH(name);
+  return LSTUR_OK;
 }
 
 // ---- segments of the sorted keys: seg_beg[v] / seg_end[v] (both zero-initialised; absent tokens keep 0, 0) ------------
@@ -357,7 +364,7 @@ static Ws carve(void* base, long long n, int V, int E) {
   Ws w;
   size_t off = 0;
   auto take = [&](size_t b) { size_t o = off; off = (off + b + 255) & ~(size_t)255; return (char*)base + o; };
-  const long long nblk = (n + SORT_CH - 1) / SORT_CH;
+  const long long nblk = sort_blocks(n);
   const long long c1 = n_chunks(n > 0 ? n : 1), c2 = n_chunks(2 * c1);     // chunks of level 1 / level 2 (ping-pong buffers)
   w.keys_a = (int*)take(n * 4); w.keys_b = (int*)take(n * 4); w.pos_a = (int*)take(n * 4); w.pos_b = (int*)take(n * 4);
   w.ghist = (int*)take((size_t)RADIX * nblk * 4); w.bintot = (int*)take(RADIX * 4);
@@ -381,18 +388,8 @@ static int run(SRC src, long long n, int L, int KS, int V, int E, const int* tok
   LSTUR_CHECK_LAUNCH(name);
   int bits = 1;
   while ((1LL << bits) <= V) ++bits;              // keys are 0 .. V inclusive
-  const int nblk = (int)((n + SORT_CH - 1) / SORT_CH);
   int *ka = w.keys_a, *kb = w.keys_b, *pa = w.pos_a, *pb = w.pos_b;
-  for (int shift = 0; shift < bits; shift += RB) {
-    radix_hist_kernel<<<nblk, SORT_THREADS, 0, st>>>(ka, n, shift, nblk, w.ghist);
-    LSTUR_CHECK_LAUNCH(name);
-    radix_rowscan_kernel<<<RADIX, 256, 0, st>>>(w.ghist, nblk, w.bintot);
-    LSTUR_CHECK_LAUNCH(name);
-    radix_scatter_kernel<<<nblk, SORT_THREADS, 0, st>>>(ka, pa, kb, pb, n, shift, nblk, w.ghist, w.bintot);
-    LSTUR_CHECK_LAUNCH(name);
-    int* t = ka; ka = kb; kb = t;
-    t = pa; pa = pb; pb = t;
-  }
+  if (int rc = radix_sort_pairs(&ka, &pa, &kb, &pb, n, bits, w.ghist, w.bintot, st, name)) return rc;
   cudaMemsetAsync(w.seg_beg, 0, (size_t)V * 4 * 2, st);
   bounds_kernel<<<cdiv(n, 256), 256, 0, st>>>(n, V, ka, w.seg_beg, w.seg_end);
   LSTUR_CHECK_LAUNCH(name);

@@ -125,11 +125,16 @@ class LsturEngine:
         # is re-packed only when the table was written (lstur_plan_invalidate_tables)
         self._emb_version = [0] if src is None else src._emb_version
         self._emb_seen = -1
+        def i32dev(a):              # host arrays are uploaded; device tensors (e.g. an interned table) are used in place
+            if a is None:
+                return None
+            if torch.is_tensor(a):
+                return a.to(dev, dtype=torch.int32).contiguous()
+            return torch.as_tensor(np.ascontiguousarray(a, dtype=np.int32)).to(dev)
         if doc_tokens is None and src is not None:
             self.doc_tokens = src.doc_tokens
         else:
-            self.doc_tokens = None if doc_tokens is None else torch.as_tensor(np.ascontiguousarray(doc_tokens, dtype=np.int32)).to(dev)
-        i32dev = lambda a: None if a is None else torch.as_tensor(np.ascontiguousarray(a, dtype=np.int32)).to(dev)
+            self.doc_tokens = i32dev(doc_tokens)
         self.doc_vert = i32dev(doc_vert) if src is None or doc_vert is not None else src.doc_vert
         self.doc_subvert = i32dev(doc_subvert) if src is None or doc_subvert is not None else src.doc_subvert
         if src is None:
@@ -377,11 +382,12 @@ class LsturEngine:
                 _ptr(table), None, None, self._stream()))
         return table
 
-    def score_impressions(self, user, hist_doc, cand_off, cand_doc, table, out=None):
+    def score_impressions(self, user, hist_doc, cand_off, cand_doc, table, out=None, user_scale=None, user_scale2=None):
         """Test-head scores of whole impressions (lstur_score_impressions): user (n,), hist_doc (n, W), cand_doc (pairs,)
         int32 device tensors, cand_off (n + 1,) host int32 offsets into cand_doc, table = eval_doc_table().  The user
-        encoder runs once per impression.  -> (cand_off[-1],) float32 device tensor of sigmoid scores (entries before
-        cand_off[0] are left as they were in `out`)."""
+        encoder runs once per impression.  user_scale / user_scale2: optional (n,) float32 device multipliers of the
+        impression's user embedding, as the batch entries of the same names in forward().  -> (cand_off[-1],) float32
+        device tensor of sigmoid scores (entries before cand_off[0] are left as they were in `out`)."""
         off = np.ascontiguousarray(cand_off, dtype=np.int32)
         n = len(off) - 1
         assert table.dtype == torch.float32 and table.is_contiguous() and table.shape[1] == self.D
@@ -389,8 +395,11 @@ class LsturEngine:
             out = torch.empty(int(off[-1]) if n >= 0 else 0, dtype=torch.float32, device=self.device)
         for t in (user, hist_doc, cand_doc):
             assert t.dtype == torch.int32 and t.is_contiguous() and t.device == self.device
+        for t in (user_scale, user_scale2):
+            assert t is None or (t.dtype == torch.float32 and t.is_contiguous() and t.device == self.device and t.numel() >= n)
         _lib.check(self.lib.lstur_score_impressions(self.plan, ctypes.byref(self._w), _ptr(self.ws), n, _ptr(user),
-                                                    _ptr(hist_doc), off.ctypes.data_as(ctypes.c_void_p), _ptr(cand_doc),
+                                                    _ptr(user_scale), _ptr(user_scale2), _ptr(hist_doc),
+                                                    off.ctypes.data_as(ctypes.c_void_p), _ptr(cand_doc),
                                                     _ptr(table), int(table.shape[0]), _ptr(out), self._stream()))
         return out
 

@@ -55,6 +55,14 @@ def aggregate(users, imprs, mask, y_true, y_pred, metric_fn=None):
     starts, ends = impression_bounds(users, imprs)
     metric_fn = metric_fn or metrics.ranking_metrics
     m = metric_fn([y_pred[a:b] for a, b in zip(starts, ends)], [y_true[a:b] for a, b in zip(starts, ends)]) if len(starts) else np.zeros((0, 4))
+    return aggregate_metrics(users, mask, y_true, starts, ends, m)
+
+
+def aggregate_metrics(users, mask, y_true, starts, ends, m):
+    """The averaging of aggregate() over precomputed per-impression metrics: starts / ends = impression_bounds(users,
+    imprs), m (len(starts), 4) = [auc, ndcg@10, ndcg@5, mrr] of each of those impressions."""
+    users, mask = np.asarray(users), np.asarray(mask)
+    y_true = np.asarray(y_true, dtype=np.float32).reshape(-1)
     impr_results = [Result(float(m[i, 0]), float(m[i, 3]), float(m[i, 2]), float(m[i, 1]), float(y_true[a:b].sum()), int(b - a), i)
                     for i, (a, b) in enumerate(zip(starts, ends))]           # ndcgv = nDCG@5, ndcgx = nDCG@10 (main.py:262-263)
     user_results, iv, oov = [], [], []

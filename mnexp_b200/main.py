@@ -84,27 +84,38 @@ def train(config, on_build=None, device_batches=False, device_eval=False):
     return handler, log.records
 
 
-def cook(config, on_build=None):
-    """main.py:147-297 (the non-generator branch the reference's Cook handler supports)."""
+def cook(config, on_build=None, device_batches=False, device_eval=False):
+    """main.py:147-297 (the non-generator branch the reference's Cook handler supports).
+    device_batches: fit on handler.device_train (the titles interned on the GPU, batches gathered there; the host loop's
+    sampling exactly) where the loop fits on handler.train.
+    device_eval: evaluate handler.device_valid and score and aggregate the test file on the GPU (Cook.aggregate_test with
+    device=True; the scores differ by rounding only) where the loop does it on the host; independent of device_batches."""
     log = _Log()
     handler = task.get(config)
+    if (device_batches or device_eval) and not isinstance(handler, task.Cook):
+        raise NotImplementedError('%s has no interned device rows (Cook has)' % config.task)
+    training_data = handler.device_train if device_batches else handler.train
+    valid = handler.device_valid if device_eval else handler.valid
     for epoch in range(config.epochs):
         logging.info('[+] start epoch {}'.format(epoch))
         model = handler.build_model(epoch)
         if epoch == 0 and on_build is not None:
             on_build(handler)
-        history = model.fit(*handler.train(), config.batch_size, epochs=epoch + 1, initial_epoch=epoch, shuffle=True, verbose=2)
+        history = model.fit(*training_data(), config.batch_size, epochs=epoch + 1, initial_epoch=epoch, shuffle=True, verbose=2)
         log.history(history)
         if hasattr(handler, 'callback'):
             _with_captured_evaluations(log, handler.callback, epoch)
         try:
-            evaluations = handler.test_model.evaluate(*handler.valid(), config.batch_size, verbose=0)
+            evaluations = handler.test_model.evaluate(*valid(), config.batch_size, verbose=0)
             log.evaluation(dict(zip(handler.test_model.metrics_names, evaluations)))
         except Exception as e:
             print(e)
         if hasattr(handler, 'callback_valid'):
             handler.callback_valid(epoch)
         logging.info('[-] finish epoch {}'.format(epoch))
+    if device_eval:
+        handler.aggregate_test(config.batch_size, device=True, log=log.evaluation)
+        return handler, log.records
     feature, (users, imprs, mask, y_true) = handler.test()
     y_pred = handler.test_model.predict(feature, batch_size=config.batch_size, verbose=0).reshape((-1,))
     res = evaluation.aggregate(users, imprs, mask.reshape(-1), y_true, y_pred)

@@ -329,6 +329,57 @@ def write_cook_npz(dirname, shape, n_train=24, n_test=30, seed=0, days=30):
     np.save(os.path.join(dirname, 'Vocab.tsv.npy'), make_vocab(shape.vocab, shape.E))
 
 
+def write_cook_npz_shared(dirname, shape, n_train=23, n_impr=10, long_impr=40, seed=0, days=30):
+    """Cook .npz files (write_cook_npz's layout) whose test file is laid out as the reference's data is: every candidate
+    row of an impression repeats the impression's user, idx_mask and history.  Impressions have 2..8 candidates, one has
+    `long_impr`; users have one or two impressions; about a third of the users are out of vocabulary (idx_mask 0, in the
+    training file too); the title of document 0 (all zero) is a candidate in both files; titles recur across rows with
+    other verticals: a slot carries its document's vertical and subvertical, one slot in ten other ones.  n_train is
+    meant not to divide the batch size (a ragged last batch)."""
+    import os
+    g = np.random.default_rng(seed)
+    tok, dvert, dsub = make_docs(shape.n_news, shape.L, shape.vocab)
+
+    def verts(docs, lo):
+        other = g.random(docs.shape) < 0.1
+        v = np.where(other, g.integers(lo, 16, docs.shape), dvert[docs])
+        s = np.where(other, g.integers(lo, 307, docs.shape), dsub[docs])
+        return v * (docs > 0), s * (docs > 0)
+
+    def hist(n):
+        hd = g.integers(0, shape.n_news + 1, (n, shape.W))
+        hd[:, :2] = 0
+        return hd
+    hd, cd = hist(n_train), g.integers(1, shape.n_news + 1, (n_train, 5))
+    cd[0, 2] = 0
+    (hv, hs), (cv, cs) = verts(hd, 0), verts(cd, 1)
+    tr = dict(idx=g.integers(0, 50, (n_train, 1)), idx_mask=(g.random((n_train, 1)) < 0.7).astype(np.float32),
+              ch_title=tok[hd], ch_vert=hv, ch_subvert=hs, cd_title=tok[cd], cd_vert=cv, cd_subvert=cs,
+              cd_label=np.eye(5, dtype=np.float32)[np.zeros(n_train, dtype=int)])
+    sizes = g.integers(2, 9, n_impr)
+    sizes[n_impr // 2] = long_impr
+    imp = np.repeat(np.arange(n_impr), sizes)
+    h = n_impr // 2
+    u_of = np.where(np.arange(n_impr) < h, np.arange(n_impr) // 2, np.arange(n_impr) - h + (h + 1) // 2)
+    user = u_of[imp]                                      # users of two impressions, then users of one
+    n = len(imp)
+    iv = (g.random(int(user.max()) + 1) < 0.65).astype(np.float32)
+    iv[:2] = [1.0, 0.0]
+    hi = hist(n_impr)[imp]
+    cdt = g.integers(1, shape.n_news + 1, n)
+    cdt[np.cumsum(sizes)[:3] - 1] = 0                     # the all-zero title as a candidate
+    label = np.zeros(n, dtype=np.float32)
+    label[np.cumsum(sizes) - sizes + g.integers(0, sizes)] = 1.0
+    hv, hs = (a[imp] for a in verts(hi[np.cumsum(sizes) - sizes], 0))
+    cv, cs = verts(cdt, 1)
+    te = dict(idx=(user % 50).reshape(n, 1), idx_mask=iv[user].reshape(n, 1), ch_title=tok[hi], ch_vert=hv, ch_subvert=hs,
+              cd_title=tok[cdt], cd_vert=cv, cd_subvert=cs, label=label, user=user, impr=imp)
+    os.makedirs(dirname, exist_ok=True)
+    np.savez(os.path.join(dirname, 'train_%ddays_%dwindow.npz' % (days, shape.W)), **tr)
+    np.savez(os.path.join(dirname, 'test_%ddays_%dwindow.npz' % (days, shape.W)), **te)
+    np.save(os.path.join(dirname, 'Vocab.tsv.npy'), make_vocab(shape.vocab, shape.E))
+
+
 # ---- a LEARNABLE synthetic click task (training-parity / AUC checks; BASELINE.json north_star: "AUC within 0.002 after
 # a fixed step count").  make_batches() above draws positives at random, so nothing can be learnt from it; here every
 # document carries a latent topic visible in its title tokens and every user prefers one topic, so a model that reads

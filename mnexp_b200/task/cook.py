@@ -21,6 +21,49 @@ FEATURES = ['idx', 'idx_mask', 'ch_title', 'ch_vert', 'ch_subvert', 'cd_title', 
 N_USER_ROWS = 25000                                       # keras.layers.Embedding(25000, ...), task/cook.py:137
 
 
+class CookDeviceData:
+    """The rows of one Cook .npz file on the device, titles interned (mnexp_b200/intern.py): user (n,) int32 (`idx`),
+    mask (n,) float32 (`idx_mask`), hist_doc (n, W) and cand_doc (n, C) int32 document ids, label (n, C) float32; plus
+    host_mask, the host copy of `mask` the training draws read.  Cook.device_train / device_valid / device_test return
+    it where train / valid / test return the feature lists."""
+    __slots__ = ('user', 'mask', 'hist_doc', 'cand_doc', 'label', 'host_mask')
+
+    def __init__(self, user, mask, hist_doc, cand_doc, label, host_mask):
+        self.user, self.mask, self.hist_doc, self.cand_doc, self.label = user, mask, hist_doc, cand_doc, label
+        self.host_mask = host_mask
+
+    @property
+    def n(self):
+        return int(self.user.numel())
+
+    def head(self, k):
+        """the first k rows"""
+        return CookDeviceData(self.user[:k], self.mask[:k], self.hist_doc[:k], self.cand_doc[:k], self.label[:k],
+                              self.host_mask[:k])
+
+
+def epoch_scales(mask, order, batch_size, keep, two):
+    """The id-embedding multipliers of one epoch of CookModel.fit, drawn from numpy's global stream exactly as the host
+    loop draws them batch by batch (CookModel._batch on the rows of each batch, the ragged last one padded with its first
+    row): -> (scale, scale2) float32 arrays of ceil(n / B) * B entries, entry s*B + b for row b of batch s (scale2 None
+    unless `two`, the archs with a second id table)."""
+    n, B = len(order), batch_size
+    nb = -(-n // B)
+    slot = np.arange(nb * B)
+    rows = np.asarray(order)[np.where(slot < n, slot, slot // B * B)]
+    scale = np.asarray(mask, dtype=np.float32).reshape(-1)[rows]
+    scale2 = scale.copy() if two else None
+    if keep < 1.0:               # Dropout(1 - id_keep) on the mask (task/cook.py:141-142): random(B) per table per batch
+        r = np.empty((nb, 2 if two else 1, B))
+        for s in range(nb):
+            for t in range(r.shape[1]):
+                r[s, t] = np.random.random(B)
+        scale = scale * (r[:, 0].reshape(-1) < keep).astype(np.float32) / keep
+        if two:
+            scale2 = scale2 * (r[:, 1].reshape(-1) < keep).astype(np.float32) / keep
+    return scale, scale2
+
+
 class CookModel:
     """train_model (train=True) or test_model of Cook._build_model, task/cook.py:214-277."""
 
@@ -59,6 +102,8 @@ class CookModel:
 
     def fit(self, x, y, batch_size=32, epochs=1, initial_epoch=0, shuffle=True, verbose=0, **_):
         assert self.is_train
+        if isinstance(x, CookDeviceData):
+            return self._fit_device(x, batch_size, epochs, initial_epoch, shuffle)
         y = np.asarray(y[0] if isinstance(y, (list, tuple)) else y, dtype=np.float32)
         n, C = y.shape
         h = keras_like.History()
@@ -89,7 +134,90 @@ class CookModel:
                 h.history.setdefault(name, []).append(float(v))
         return h
 
+    def _fit_device(self, x, batch_size, epochs, initial_epoch, shuffle):
+        """fit on interned device rows (Cook.device_train): the host loop's permutation and id_keep draws, once per epoch
+        (epoch_scales), batches gathered on the device (lstur_gather_samples), and loss / accuracy summed on the device
+        in step order and read once per epoch.  The kernels see the same token rows as in the host loop."""
+        import torch
+        n = x.n
+        two = self.owner.config.arch in ('inigru', 'inagru')
+        h = keras_like.History()
+        for epoch in range(initial_epoch, epochs):
+            order = np.random.permutation(n) if shuffle else np.arange(n)
+            scale, scale2 = epoch_scales(x.host_mask, order, batch_size, self.owner.config.id_keep, two)
+            eng = self.owner.engine(batch_size, x.cand_doc.shape[1], training=True)
+            eng.lr = self.optimizer.lr.value
+            up = lambda a: None if a is None else torch.as_tensor(a).to(eng.device)
+            tot = self._device_steps(eng, x, up(order.astype(np.int32)), up(scale), up(scale2))
+            h.epoch.append(epoch)
+            for name, v in zip(self.metrics_names, tot.cpu().numpy() / max(1, n)):
+                h.history.setdefault(name, []).append(float(v))
+        return h
+
+    @staticmethod
+    def _device_steps(eng, x, order, scale, scale2):
+        """One epoch of train steps over the rows `order` (device int32), batch s taking its id multipliers from entries
+        s*B .. (s+1)*B of scale / scale2 (device float32; scale2 None for one id table).  Nothing waits for the device:
+        -> (2,) float64 device tensor [sum of loss * B, count of correct argmaxes], summed in step order."""
+        import ctypes
+        import torch
+        from .. import _lib
+        n, B, C, W = int(order.numel()), eng.B, eng.C, x.hist_doc.shape[1]
+        dev = eng.device
+        user = torch.empty(B, dtype=torch.int32, device=dev)
+        hist = torch.empty((B, W), dtype=torch.int32, device=dev)
+        cand = torch.empty((B, C), dtype=torch.int32, device=dev)
+        lab = torch.empty((B, C), dtype=torch.float32, device=dev)
+        tot = torch.zeros(2, dtype=torch.float64, device=dev)
+        probs = eng.view('probs').reshape(B, C)
+        p = lambda t: ctypes.c_void_p(None if t is None else t.data_ptr())
+        for step, s in enumerate(range(0, n, B)):
+            m = min(B, n - s)
+            _lib.check(eng.lib.lstur_gather_samples(B, m, W, C, ctypes.c_void_p(order.data_ptr() + 4 * s), p(x.user), None,
+                                                    p(x.hist_doc), p(x.cand_doc), p(x.label), p(user), None, p(hist),
+                                                    p(cand), p(lab), eng._stream()))
+            db = dict(user=user, user_scale=scale[step * B:(step + 1) * B], hist_doc=hist, cand_doc=cand, label=lab)
+            if scale2 is not None:
+                db['user_scale2'] = scale2[step * B:(step + 1) * B]
+            loss = eng.train_step(db, grad_scale=1.0 / m)
+            tot[0] += loss[0].double() * B           # the host loop's float(loss) * batch_size, in float64
+            tot[1] += (probs[:m].argmax(1) == lab[:m].argmax(1)).double().sum()
+        return tot
+
+    def _predict_device(self, x):
+        """test_model scores of interned test rows (Cook.device_valid / device_test) -> (n,) float32 device tensor.
+        Consecutive rows with the same user, mask and history form one impression of lstur_score_impressions (one user
+        vector; split where it exceeds the plan's rows * candidates), every document is encoded once."""
+        import ctypes
+        import torch
+        from .. import _lib, intern
+        assert not self.is_train and x.cand_doc.shape[1] == 1, 'device scoring is the one-candidate test model'
+        n = x.n
+        starts = intern.group_rows(x.user, x.mask, x.hist_doc)
+        sizes = np.diff(np.append(starts, n))
+        C = int(min(32, max(1, np.ceil(sizes.mean())))) if n else 1
+        eng = self.owner.engine(self.owner.predict_rows, C, training=False)
+        cap = eng.B * eng.C
+        pieces = np.concatenate([np.arange(a, a + k, cap) for a, k in zip(starts, sizes)]) if n else np.zeros(0, np.int64)
+        off = np.append(pieces, n).astype(np.int32)
+        P, W, dev = len(pieces), x.hist_doc.shape[1], eng.device
+        out = torch.empty(n, dtype=torch.float32, device=dev)
+        if n == 0:
+            return out
+        pos = torch.as_tensor(pieces.astype(np.int32)).to(dev)
+        user = torch.empty(P, dtype=torch.int32, device=dev)
+        scale = torch.empty(P, dtype=torch.float32, device=dev)
+        hist = torch.empty((P, W), dtype=torch.int32, device=dev)
+        p = lambda t: ctypes.c_void_p(None if t is None else t.data_ptr())
+        _lib.check(eng.lib.lstur_gather_samples(P, P, W, 0, p(pos), p(x.user), p(x.mask), p(x.hist_doc), None, None,
+                                                p(user), p(scale), p(hist), None, None, eng._stream()))
+        two = self.owner.config.arch in ('inigru', 'inagru')        # the second table's Dropout sees the same mask
+        return eng.score_impressions(user, hist, off, x.cand_doc.reshape(-1), eng.eval_doc_table(), out=out,
+                                     user_scale=scale, user_scale2=scale if two else None)
+
     def predict(self, x, batch_size=None, verbose=0, **_):
+        if isinstance(x, CookDeviceData):
+            return self._predict_device(x).cpu().numpy().reshape(-1, 1)
         n = len(np.asarray(x[0]))
         C = np.asarray(x[5]).shape[1] if self.is_train else 1
         R = self.owner.predict_rows
@@ -108,7 +236,7 @@ class CookModel:
 
     def evaluate(self, x, y, batch_size=None, verbose=0, **_):
         y = np.asarray(y[0] if isinstance(y, (list, tuple)) else y, dtype=np.float64)
-        p = self.predict(x).astype(np.float64)
+        p = self.predict(x).astype(np.float64)          # interned rows: one read-back of the scores
         if self.is_train:
             q = np.clip(p / p.sum(-1, keepdims=True), 1e-7, 1 - 1e-7)
             return [float((-(y * np.log(q)).sum(-1)).mean()), float((p.argmax(1) == y.argmax(1)).mean())]
@@ -135,6 +263,7 @@ class Cook:
         logging.info('[-] loaded testing data')
         self.predict_rows = 256
         self._train_engine, self._infer = None, {}
+        self._doc_table, self._device_data = None, None
 
     def train(self):
         return [self.training_data[x] for x in FEATURES], [self.training_data[x] for x in ['cd_label']]
@@ -146,15 +275,72 @@ class Cook:
     def test(self):
         return [self.test_data[x] for x in FEATURES], [self.test_data[x] for x in ['user', 'impr', 'idx_mask', 'label']]
 
-    def aggregate_test(self, batch_size=None):
+    # ---- interned rows on the device: training batches gathered there, test rows scored per user group ---------------
+    def _interned(self):
+        """Intern the titles of both files into one document table (once; needs the built model, whose vertical
+        embeddings decide whether the vertical / subvertical ids are part of the key) and keep each file's rows on the
+        device as CookDeviceData.  The engines are rebuilt on the table (Cook.engine)."""
+        import torch
+        from .. import intern
+        if self._device_data is None:
+            assert hasattr(self, 'dv'), 'build_model(0) first'
+            dev = torch.device('cuda', torch.cuda.current_device())
+            parts = []
+            for d in (self.training_data, self.test_data):
+                for t in ('ch', 'cd'):
+                    parts.append((d[t + '_title'], d[t + '_vert'] if self.dv else None, d[t + '_subvert'] if self.ds else None))
+            ids, self._doc_table = intern.intern(parts, self.L, dev)
+            out = {}
+            for i, (name, d) in enumerate((('train', self.training_data), ('test', self.test_data))):
+                hist, cand = ids[2 * i], ids[2 * i + 1]
+                n = hist.shape[0]
+                lab = d['cd_label'] if name == 'train' else d['label']
+                mask = np.asarray(d['idx_mask'], dtype=np.float32).reshape(n)
+                out[name] = CookDeviceData(intern._upload(d['idx'], dev).reshape(n), torch.as_tensor(mask).to(dev),
+                                           hist, cand.reshape(n, -1),
+                                           torch.as_tensor(np.asarray(lab, dtype=np.float32).reshape(n, -1)).to(dev), mask)
+            self._device_data = out
+        return self._device_data
+
+    def device_train(self):
+        """train() with the features interned on the device: (CookDeviceData, [cd_label]) for CookModel.fit"""
+        return self._interned()['train'], [self.training_data['cd_label']]
+
+    def device_valid(self):
+        """valid() interned: the first validation_step test rows, for test_model.evaluate"""
+        k = self.config.validation_step
+        return self._interned()['test'].head(k), [self.test_data['label'][:k]]
+
+    def device_test(self):
+        """test() interned: (CookDeviceData, [user, impr, idx_mask, label])"""
+        return self._interned()['test'], [self.test_data[x] for x in ['user', 'impr', 'idx_mask', 'label']]
+
+    def aggregate_test(self, batch_size=None, device=False, log=None):
         """The evaluation tail of `main.py cook` (main.py:216-297): score the test set with test_model and average the
         ranking metrics per impression, per user, and per in-vocabulary / out-of-vocabulary user.  Returns the four
-        Result objects of mnexp_b200.evaluation.aggregate and logs them like the reference."""
+        Result objects of mnexp_b200.evaluation.aggregate and logs them like the reference (through `log`, default
+        utils.logging_evaluation).  device: score the interned rows (device_test) and compute every impression's
+        metrics in one launch on the device scores."""
         from .. import evaluation, utils
-        feature, (users, imprs, mask, y_true) = self.test()
-        y_pred = self.test_model.predict(feature, batch_size=batch_size or self.config.batch_size).reshape(-1)
-        res = evaluation.aggregate(users, imprs, np.asarray(mask).reshape(-1), y_true, y_pred)
-        evaluation.log_aggregate(res, utils.logging_evaluation)
+        if not device:
+            feature, (users, imprs, mask, y_true) = self.test()
+            y_pred = self.test_model.predict(feature, batch_size=batch_size or self.config.batch_size).reshape(-1)
+            res = evaluation.aggregate(users, imprs, np.asarray(mask).reshape(-1), y_true, y_pred)
+        else:
+            import ctypes
+            import torch
+            from .. import _lib
+            x, (users, imprs, mask, y_true) = self.device_test()
+            scores = self.test_model._predict_device(x)
+            starts, ends = evaluation.impression_bounds(users, imprs)
+            m = torch.empty((len(starts), 4), dtype=torch.float32, device=scores.device)
+            if len(starts):             # the closed impressions are contiguous from row 0
+                off = torch.as_tensor(np.append(starts, ends[-1]).astype(np.int32)).to(scores.device)
+                p = lambda t: ctypes.c_void_p(t.data_ptr())
+                _lib.check(_lib.load().lstur_ranking_metrics(len(starts), p(off), p(scores), p(x.label), p(m),
+                                                             ctypes.c_void_p(torch.cuda.current_stream(scores.device).cuda_stream)))
+            res = evaluation.aggregate_metrics(users, np.asarray(mask).reshape(-1), y_true, starts, ends, m.cpu().numpy())
+        evaluation.log_aggregate(res, log or utils.logging_evaluation)
         return res
 
     def build_model(self, epoch):
@@ -211,14 +397,17 @@ class Cook:
         c = self.config
         kw = dict(arch=c.arch, flavour='cook', recurrent_activation=c.recurrent_activation, score_model=c.score_model,
                   precision=self._precision())
-        if training or self._train_engine is None:
-            e = self._train_engine
-            if e is None or ((e.B != B or e.C != C) and training):
+        e = self._train_engine
+        table = self._doc_table or {}
+        stale = e is not None and self._doc_table is not None and e.doc_tokens is not table['doc_tokens']
+        if training or e is None or stale:
+            if e is None or stale or ((e.B != B or e.C != C) and training):
+                tB, tC = (e.B, e.C) if e is not None and not training else (B, C)     # a rebuild on the table keeps its shape
                 if e is not None:
                     self.params = e.get_weights_dict()
-                self._train_engine = LsturEngine(self.params, B, self.W, C, self.L, dropout=c.dropout, lr=c.learning_rate,
+                self._train_engine = LsturEngine(self.params, tB, self.W, tC, self.L, dropout=c.dropout, lr=c.learning_rate,
                                                  training=True, sparse_user_adam=bool(c.sparse_user_adam),
-                                                 trainable_word_emb=bool(c.textual_embedding_trainable), **kw)
+                                                 trainable_word_emb=bool(c.textual_embedding_trainable), **table, **kw)
                 if e is not None:
                     self._train_engine.adopt_state_from(e)      # keep Adam moments / step count / dropout seed counter
                 self._infer = {}
