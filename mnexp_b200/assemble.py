@@ -109,6 +109,22 @@ def build_tables(data, W=None, window=None):
     return out
 
 
+def assemble_samples(t, sample_click, sample_hist_end, idx, W, K, expire=0, seed=0, row0=0):
+    """lstur_assemble_samples over the device copies t of build_tables: samples idx ((B,) int32 device tensor) of the
+    click table sample_click, histories ending at sample_hist_end (None: at the click), Days window `expire` seconds,
+    K negatives drawn with seed / row0.  -> dict(user (B), hist_doc (B, W), cand_doc (B, 1 + K)) int32 device tensors."""
+    B, dev = int(idx.numel()), idx.device
+    user = torch.empty(B, dtype=torch.int32, device=dev)
+    hist = torch.empty((B, W), dtype=torch.int32, device=dev)
+    cand = torch.empty((B, 1 + K), dtype=torch.int32, device=dev)
+    p = lambda x: ctypes.c_void_p(None if x is None else x.data_ptr())
+    _lib.check(_lib.load().lstur_assemble_samples(
+        B, W, K, p(sample_click), p(sample_hist_end), p(idx), p(t['click_user']), p(t.get('click_time')), expire,
+        p(t['stream_off']), p(t['stream_docs']), p(t['neg_off']), p(t['neg_docs']), ctypes.c_uint(seed), row0,
+        p(user), p(hist), p(cand), ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+    return dict(user=user, hist_doc=hist, cand_doc=cand)
+
+
 class DeviceBatch:
     """One assembled batch on the device: user (B), hist_doc (B,W), cand_doc (B,1+K) int32; the positive is column 0 of
     cand_doc.  keras_like.Model accepts it wherever it accepts a host (inputs, targets) pair."""
@@ -144,7 +160,6 @@ class DeviceBatcher:
         if split not in ('train', 'valid'):
             raise ValueError(split)
         assert 0 <= rank < world
-        self.lib = _lib.load()
         self.device = torch.device('cuda', torch.cuda.current_device()) if device is None else torch.device(device)
         self.B, self.W, self.K, self.seed = B, W, K, seed
         self.split, self.rank, self.world = split, rank, world
@@ -181,19 +196,9 @@ class DeviceBatcher:
 
     def assemble(self, idx, row0=0):
         """idx: (B) int32 device tensor of sample numbers -> device batch dict for LsturEngine."""
-        B, W, K = int(idx.numel()), self.W, self.K
-        user = torch.empty(B, dtype=torch.int32, device=self.device)
-        hist = torch.empty((B, W), dtype=torch.int32, device=self.device)
-        cand = torch.empty((B, 1 + K), dtype=torch.int32, device=self.device)
-        p = lambda x: ctypes.c_void_p(None if x is None else x.data_ptr())
-        t = self.t
         self.step += 1
-        _lib.check(self.lib.lstur_assemble_samples(
-            B, W, K, p(self._click), p(self._hist_end), p(idx), p(t['click_user']), p(t.get('click_time')), self.expire,
-            p(t['stream_off']), p(t['stream_docs']), p(t['neg_off']), p(t['neg_docs']),
-            ctypes.c_uint((self.seed * 1000003 + self.step) & 0xffffffff), row0, p(user), p(hist), p(cand),
-            ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
-        return dict(user=user, hist_doc=hist, cand_doc=cand)
+        return assemble_samples(self.t, self._click, self._hist_end, idx, self.W, self.K, self.expire,
+                                (self.seed * 1000003 + self.step) & 0xffffffff, row0)
 
     def next_batch(self):
         assert self.n_samples > 0, 'no %s samples' % self.split

@@ -14,6 +14,14 @@ import torch
 from . import _lib
 
 
+def _ptr(t):
+    return ctypes.c_void_p(None if t is None else t.data_ptr())
+
+
+def _stream(device):
+    return ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+
+
 def _upload(a, device):
     """int32 on the device, converted as LsturEngine.to_device_batch converts host token arrays"""
     t = a if torch.is_tensor(a) else torch.from_numpy(np.ascontiguousarray(a))
@@ -53,8 +61,7 @@ def intern(parts, L, device=None):
         if s is not None:
             subvert[r0:r0 + k] = _upload(s, dev).reshape(k)
         r0 += k
-    p = lambda t: ctypes.c_void_p(None if t is None else t.data_ptr())
-    st = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+    p, st = _ptr, _stream(dev)
     ids = torch.empty(n, dtype=torch.int32, device=dev)
     first_row = torch.empty(n + 1, dtype=torch.int32, device=dev)
     ws = torch.empty(int(lib.lstur_intern_workspace_bytes(n, L)), dtype=torch.uint8, device=dev)
@@ -84,7 +91,19 @@ def group_rows(user, scale, hist_doc):
     starts = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
     ws = torch.empty(int(lib.lstur_intern_workspace_bytes(n, 0)), dtype=torch.uint8, device=dev)
     n_groups = ctypes.c_int()
-    p = lambda t: ctypes.c_void_p(None if t is None else t.data_ptr())
+    p = _ptr
     _lib.check(lib.lstur_group_rows(n, W, p(user), p(scale), p(hist_doc), p(starts), ctypes.byref(n_groups), p(ws),
-                                    ws.numel(), ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+                                    ws.numel(), _stream(dev)))
     return starts[:n_groups.value].cpu().numpy().astype(np.int64)
+
+
+def gather_samples(pos, m, src, out):
+    """lstur_gather_samples: row b < m of each B-row device buffer in `out` <- sample pos[b] (int32 device tensor) of the
+    same-named table in `src` (user, scale, hist_doc, cand_doc, label; 'user' and 'hist_doc' required, the others read
+    only when `out` has them); rows b >= m (a ragged last batch) repeat pos[0] with an all-zero label row."""
+    B, W = out['hist_doc'].shape
+    C = out['cand_doc'].shape[1] if 'cand_doc' in out else 0
+    names = ('user', 'scale', 'hist_doc', 'cand_doc', 'label')
+    tables = [_ptr(src[k] if k in out else None) for k in names]
+    bufs = [_ptr(out.get(k)) for k in names]
+    _lib.check(_lib.load().lstur_gather_samples(B, m, W, C, _ptr(pos), *tables, *bufs, _stream(pos.device)))

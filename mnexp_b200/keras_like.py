@@ -41,6 +41,13 @@ class Adam:
         self.lr = Variable(lr)
 
 
+def categorical_loss_accuracy(p, y):
+    """Keras categorical_crossentropy (rows renormalised, clipped to [1e-7, 1 - 1e-7]) and categorical_accuracy of the
+    float64 probabilities p (n, C) against the one-hot targets y (n, C) -> [loss, accuracy]"""
+    q = np.clip(p / p.sum(-1, keepdims=True), 1e-7, 1 - 1e-7)
+    return [float((-(y * np.log(q)).sum(-1)).mean()), float((p.argmax(1) == y.argmax(1)).mean())]
+
+
 class History:
     def __init__(self):
         self.history = {}
@@ -48,20 +55,25 @@ class History:
 
 
 class _Core:
-    """Weights + engines shared by `model` (softmax/CE training graph) and `test_model` (sigmoid scoring graph)."""
+    """Weights + engines shared by `model` (softmax/CE training graph) and `test_model` (sigmoid scoring graph).  W / L:
+    history and title length of the plans, n_cand: candidates per training row (defaults from the config)."""
 
     def __init__(self, params, cfg, doc_tokens, has_user, arch, predict_rows=256, score_model='dot', loss='softmax',
-                 flavour='paper', has_vert=False):
-        self.params, self.cfg, self.doc_tokens, self.has_user, self.arch = params, cfg, doc_tokens, has_user, arch
+                 flavour='paper', has_vert=False, W=None, L=None, n_cand=None):
+        self.params, self.cfg, self.has_user, self.arch = params, cfg, has_user, arch
         self.score_model, self.loss, self.flavour = score_model, loss, flavour
         self.has_vert = has_vert        # inputs carry vertical ids next to the titles (task/paper.py:1205-1232)
+        self.W = cfg.window_size if W is None else W
+        self.L = cfg.title_shape if L is None else L
+        self.n_cand = n_cand
         self.optimizer = Adam(cfg.learning_rate)
         self.train_engine = None
         self.infer_engines = {}
         self.predict_rows = predict_rows
         self.step_seed = 0
         self.freeze_encoder = False     # --enable-pretrain-encoder without --pretrain-encoder-trainable (task/paper.py:103-106)
-        self.doc_vert = None            # (n_docs,) vertical of every document: vertical ids of device-assembled batches
+        # the document table that device batches address by id (set_doc_table): titles, vertical, subvertical
+        self.doc_tokens, self.doc_vert, self.doc_subvert = doc_tokens, None, None
 
     def precision(self):
         p = getattr(self.cfg, 'precision', 'auto')
@@ -69,28 +81,37 @@ class _Core:
             return p
         from . import _lib
         ks, E, F = self.params['conv_w'].shape
-        ok = _lib.load().lstur_tc_supported(self.cfg.title_shape, E, F, ks)
+        ok = _lib.load().lstur_tc_supported(self.L, E, F, ks)
         return 'fp16_tc' if ok else 'fp32'
 
+    def set_doc_table(self, doc_tokens, doc_vert=None, doc_subvert=None):
+        """Install a document table.  A training engine is rebuilt at its batch size on the new table and keeps its
+        weights and optimizer state; the inference engines are rebuilt when next asked for."""
+        self.doc_tokens, self.doc_vert, self.doc_subvert = doc_tokens, doc_vert, doc_subvert
+        if self.train_engine is not None:
+            self._build_train(self.train_engine.B)
+
     def engine_train(self, B):
-        e = self.train_engine
-        if e is None or e.B != B:
-            old = e
-            if e is not None:                      # batch size changed: carry the weights (and optimizer state, below) over
-                self.params = e.get_weights_dict()
-            c = self.cfg
-            self.train_engine = LsturEngine(
-                self.params, B, c.window_size, self.n_train_cand(), c.title_shape, arch=self.arch,
-                dropout=c.dropout, lr=c.learning_rate, recurrent_activation=c.recurrent_activation,
-                precision=self.precision(), doc_tokens=self.doc_tokens, training=True,
-                sparse_user_adam=bool(c.sparse_user_adam), score_model=self.score_model,
-                trainable_word_emb=bool(getattr(c, 'textual_embedding_trainable', False)), doc_vert=self.doc_vert,
-                **self.head_kw())
-            if old is not None:
-                self.train_engine.adopt_state_from(old)
-            self.train_engine.freeze_encoder = self.freeze_encoder
-            self.infer_engines = {}
+        if self.train_engine is None or self.train_engine.B != B:
+            self._build_train(B)
         return self.train_engine
+
+    def _build_train(self, B):
+        old = self.train_engine
+        if old is not None:                        # carry the weights (and optimizer state, below) over
+            self.params = old.get_weights_dict()
+        c = self.cfg
+        self.train_engine = LsturEngine(
+            self.params, B, self.W, self.n_train_cand(), self.L, arch=self.arch,
+            dropout=c.dropout, lr=c.learning_rate, recurrent_activation=c.recurrent_activation,
+            precision=self.precision(), doc_tokens=self.doc_tokens, training=True,
+            sparse_user_adam=bool(c.sparse_user_adam), score_model=self.score_model,
+            trainable_word_emb=bool(getattr(c, 'textual_embedding_trainable', False)), doc_vert=self.doc_vert,
+            doc_subvert=self.doc_subvert, **self.head_kw())
+        if old is not None:
+            self.train_engine.adopt_state_from(old)
+        self.train_engine.freeze_encoder = self.freeze_encoder
+        self.infer_engines = {}
 
     def engine_infer(self, C, rows=None):
         rows = rows or self.predict_rows
@@ -101,7 +122,7 @@ class _Core:
             # that would discard its optimizer state); create one only if training has not started
             base = self.train_engine if self.train_engine is not None else self.engine_train(c.batch_size)
             self.infer_engines[key] = LsturEngine(
-                self.params, rows, c.window_size, C, c.title_shape, arch=self.arch, dropout=0.0,
+                self.params, rows, self.W, C, self.L, arch=self.arch, dropout=0.0,
                 recurrent_activation=c.recurrent_activation, precision=self.precision(), training=False,
                 share_weights_from=base, score_model=self.score_model, **self.head_kw())
         return self.infer_engines[key]
@@ -134,7 +155,7 @@ class _Core:
         return cached
 
     def n_train_cand(self):
-        return 1 if self.loss == 'bce' else 1 + self.cfg.negative_samples
+        return self.n_cand or (1 if self.loss == 'bce' else 1 + self.cfg.negative_samples)
 
     def head_kw(self):
         kw = dict(flavour=self.flavour, loss=self.loss, gain=self.cfg.gain, bce_neg=self.cfg.negative_samples)
@@ -435,8 +456,7 @@ class Model:
             l = -0.5 * (1 + K) * np.mean(yy * np.log(q + 1e-8) * self.core.cfg.gain + (1 - yy) * np.log(1 - q + 1e-8) / K)
             return [float(l), metrics.auc_roc(q, yy)]
         if self.is_train:
-            q = np.clip(p / p.sum(-1, keepdims=True), 1e-7, 1 - 1e-7)
-            return [float((-(y * np.log(q)).sum(-1)).mean()), float((p.argmax(1) == y.argmax(1)).mean())]
+            return categorical_loss_accuracy(p, y)
         q = np.clip(p.reshape(-1), 1e-7, 1 - 1e-7)
         yy = y.reshape(-1)
         return [float(-(yy * np.log(q) + (1 - yy) * np.log(1 - q)).mean())]
@@ -630,9 +650,7 @@ class VertModel:
 
     def evaluate(self, x, y, batch_size=None, verbose=0, **_):
         y = np.asarray(y[0] if isinstance(y, (list, tuple)) else y, dtype=np.float64)
-        p = self.predict(x).astype(np.float64)
-        q = np.clip(p / p.sum(-1, keepdims=True), 1e-7, 1 - 1e-7)
-        return [float((-(y * np.log(q)).sum(-1)).mean()), float((p.argmax(1) == y.argmax(1)).mean())]
+        return categorical_loss_accuracy(self.predict(x).astype(np.float64), y)
 
     def evaluate_generator(self, generator, steps, verbose=0, **_):
         tot = np.zeros(2)
@@ -673,9 +691,7 @@ class DocEncoderModel:
             if self.core.train_engine is not None:
                 self.core.train_engine.freeze_encoder = not v
 
-    def _current(self):
-        e = self.core.train_engine
-        return e.get_weights_dict() if e is not None else self.core.params
+    _current = Model._current
 
     def get_weights(self):
         w = self._current()

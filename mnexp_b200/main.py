@@ -18,7 +18,7 @@ with the one the reference's own main.py produced).
 """
 import logging
 
-from . import evaluation, task, utils
+from . import task, utils
 
 
 class _Log:
@@ -113,11 +113,5 @@ def cook(config, on_build=None, device_batches=False, device_eval=False):
         if hasattr(handler, 'callback_valid'):
             handler.callback_valid(epoch)
         logging.info('[-] finish epoch {}'.format(epoch))
-    if device_eval:
-        handler.aggregate_test(config.batch_size, device=True, log=log.evaluation)
-        return handler, log.records
-    feature, (users, imprs, mask, y_true) = handler.test()
-    y_pred = handler.test_model.predict(feature, batch_size=config.batch_size, verbose=0).reshape((-1,))
-    res = evaluation.aggregate(users, imprs, mask.reshape(-1), y_true, y_pred)
-    evaluation.log_aggregate(res, log.evaluation)
+    handler.aggregate_test(config.batch_size, device=device_eval, log=log.evaluation)
     return handler, log.records

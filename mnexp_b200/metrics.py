@@ -16,23 +16,29 @@ def ranking_metrics(scores, labels, device=None):
     auc, ndcg@10, ndcg@5, mrr (NaN where the host formulas divide by zero)."""
     if not torch.cuda.is_available():
         raise _lib.LsturError('ranking_metrics needs a CUDA device (no CPU fallback; use mnexp_b200.utils on the host)')
-    lib = _lib.load()
     dev = torch.device('cuda', torch.cuda.current_device()) if device is None else torch.device(device)
     lens = np.array([len(s) for s in scores], dtype=np.int64)
     assert all(len(a) == len(b) for a, b in zip(scores, labels))
     off = np.zeros(len(lens) + 1, dtype=np.int32)
     off[1:] = np.cumsum(lens)
-    n = len(lens)
-    if n == 0:
+    if len(lens) == 0:
         return np.zeros((0, 4), dtype=np.float32)
     s = torch.as_tensor(np.concatenate([np.asarray(x, dtype=np.float32).reshape(-1) for x in scores])).to(dev)
     y = torch.as_tensor(np.concatenate([np.asarray(x, dtype=np.float32).reshape(-1) for x in labels])).to(dev)
-    o = torch.as_tensor(off).to(dev)
-    out = torch.empty((n, 4), dtype=torch.float32, device=dev)
-    p = lambda t: ctypes.c_void_p(t.data_ptr())
-    _lib.check(lib.lstur_ranking_metrics(n, p(o), p(s), p(y), p(out),
-                                         ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
-    return out.cpu().numpy()
+    return device_ranking_metrics(torch.as_tensor(off).to(dev), s, y).cpu().numpy()
+
+
+def device_ranking_metrics(offsets, scores, labels):
+    """ranking_metrics of impressions already on the device: offsets (n_impr + 1,) int32, scores / labels float32
+    device tensors, impression i = entries offsets[i] .. offsets[i+1].  -> (n_impr, 4) float32 device tensor; nothing
+    waits for the device."""
+    n = int(offsets.numel()) - 1
+    out = torch.empty((n, 4), dtype=torch.float32, device=offsets.device)
+    if n:
+        p = lambda t: ctypes.c_void_p(t.data_ptr())
+        _lib.check(_lib.load().lstur_ranking_metrics(n, p(offsets), p(scores), p(labels), p(out),
+                                                     ctypes.c_void_p(torch.cuda.current_stream(offsets.device).cuda_stream)))
+    return out
 
 
 def auc_roc(scores, labels):

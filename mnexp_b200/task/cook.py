@@ -15,10 +15,11 @@ import logging
 import numpy as np
 
 from .. import keras_like, metrics, settings, synth
-from ..engine import COOK_ARCH, LsturEngine
+from ..engine import COOK_ARCH
 
 FEATURES = ['idx', 'idx_mask', 'ch_title', 'ch_vert', 'ch_subvert', 'cd_title', 'cd_vert', 'cd_subvert']
 N_USER_ROWS = 25000                                       # keras.layers.Embedding(25000, ...), task/cook.py:137
+TWO_ID_ARCHS = ('inigru', 'inagru')     # a second id embedding with its own Dropout layer (task/cook.py:169-183)
 
 
 class CookDeviceData:
@@ -65,15 +66,23 @@ def epoch_scales(mask, order, batch_size, keep, two):
 
 
 class CookModel:
-    """train_model (train=True) or test_model of Cook._build_model, task/cook.py:214-277."""
+    """train_model (train=True) or test_model of Cook._build_model, task/cook.py:214-277, over the engines, weights and
+    optimizer of the handler's keras_like._Core."""
 
     def __init__(self, owner, train):
         self.owner, self.is_train = owner, train
         self.metrics_names = ['loss', 'categorical_accuracy'] if train else ['loss', 'auc_roc']
 
     @property
+    def core(self):
+        return self.owner._core
+
+    @property
     def optimizer(self):
-        return self.owner.optimizer
+        return self.core.optimizer
+
+    _current = get_weights_dict = keras_like.Model._current
+    summary = keras_like.Model.summary
 
     def _batch(self, x, rows, C, training):
         idx, idx_mask, ch_title, ch_vert, ch_subvert, cd_title, cd_vert, cd_subvert = [np.asarray(a)[rows] for a in x]
@@ -81,7 +90,7 @@ class CookModel:
         scale = np.asarray(idx_mask, dtype=np.float32).reshape(n)
         keep = self.owner.config.id_keep
         scale2 = None
-        two = self.owner.config.arch in ('inigru', 'inagru')    # second id embedding with its own Dropout layer (:169-183)
+        two = self.owner.config.arch in TWO_ID_ARCHS
         if two:
             scale2 = scale.copy()
         if training and keep < 1.0:                       # Dropout(1 - id_keep) on the mask (task/cook.py:141-142)
@@ -110,7 +119,7 @@ class CookModel:
         for epoch in range(initial_epoch, epochs):
             order = np.random.permutation(n) if shuffle else np.arange(n)
             tot, k = np.zeros(2), 0
-            eng = self.owner.engine(batch_size, C, training=True)
+            eng = self.core.engine_train(batch_size)
             eng.lr = self.optimizer.lr.value
             for s in range(0, n, batch_size):
                 rows = order[s:s + batch_size]
@@ -136,16 +145,16 @@ class CookModel:
 
     def _fit_device(self, x, batch_size, epochs, initial_epoch, shuffle):
         """fit on interned device rows (Cook.device_train): the host loop's permutation and id_keep draws, once per epoch
-        (epoch_scales), batches gathered on the device (lstur_gather_samples), and loss / accuracy summed on the device
+        (epoch_scales), batches gathered on the device (intern.gather_samples), and loss / accuracy summed on the device
         in step order and read once per epoch.  The kernels see the same token rows as in the host loop."""
         import torch
         n = x.n
-        two = self.owner.config.arch in ('inigru', 'inagru')
+        two = self.owner.config.arch in TWO_ID_ARCHS
         h = keras_like.History()
         for epoch in range(initial_epoch, epochs):
             order = np.random.permutation(n) if shuffle else np.arange(n)
             scale, scale2 = epoch_scales(x.host_mask, order, batch_size, self.owner.config.id_keep, two)
-            eng = self.owner.engine(batch_size, x.cand_doc.shape[1], training=True)
+            eng = self.core.engine_train(batch_size)
             eng.lr = self.optimizer.lr.value
             up = lambda a: None if a is None else torch.as_tensor(a).to(eng.device)
             tot = self._device_steps(eng, x, up(order.astype(np.int32)), up(scale), up(scale2))
@@ -159,44 +168,39 @@ class CookModel:
         """One epoch of train steps over the rows `order` (device int32), batch s taking its id multipliers from entries
         s*B .. (s+1)*B of scale / scale2 (device float32; scale2 None for one id table).  Nothing waits for the device:
         -> (2,) float64 device tensor [sum of loss * B, count of correct argmaxes], summed in step order."""
-        import ctypes
         import torch
-        from .. import _lib
+        from .. import intern
         n, B, C, W = int(order.numel()), eng.B, eng.C, x.hist_doc.shape[1]
         dev = eng.device
-        user = torch.empty(B, dtype=torch.int32, device=dev)
-        hist = torch.empty((B, W), dtype=torch.int32, device=dev)
-        cand = torch.empty((B, C), dtype=torch.int32, device=dev)
-        lab = torch.empty((B, C), dtype=torch.float32, device=dev)
+        src = dict(user=x.user, hist_doc=x.hist_doc, cand_doc=x.cand_doc, label=x.label)
+        i32 = dict(dtype=torch.int32, device=dev)
+        out = dict(user=torch.empty(B, **i32), hist_doc=torch.empty((B, W), **i32), cand_doc=torch.empty((B, C), **i32),
+                   label=torch.empty((B, C), dtype=torch.float32, device=dev))
         tot = torch.zeros(2, dtype=torch.float64, device=dev)
         probs = eng.view('probs').reshape(B, C)
-        p = lambda t: ctypes.c_void_p(None if t is None else t.data_ptr())
         for step, s in enumerate(range(0, n, B)):
             m = min(B, n - s)
-            _lib.check(eng.lib.lstur_gather_samples(B, m, W, C, ctypes.c_void_p(order.data_ptr() + 4 * s), p(x.user), None,
-                                                    p(x.hist_doc), p(x.cand_doc), p(x.label), p(user), None, p(hist),
-                                                    p(cand), p(lab), eng._stream()))
-            db = dict(user=user, user_scale=scale[step * B:(step + 1) * B], hist_doc=hist, cand_doc=cand, label=lab)
+            intern.gather_samples(order[s:], m, src, out)
+            db = dict(out, user_scale=scale[step * B:(step + 1) * B])
             if scale2 is not None:
                 db['user_scale2'] = scale2[step * B:(step + 1) * B]
             loss = eng.train_step(db, grad_scale=1.0 / m)
             tot[0] += loss[0].double() * B           # the host loop's float(loss) * batch_size, in float64
-            tot[1] += (probs[:m].argmax(1) == lab[:m].argmax(1)).double().sum()
+            tot[1] += (probs[:m].argmax(1) == out['label'][:m].argmax(1)).double().sum()
         return tot
 
     def _predict_device(self, x):
         """test_model scores of interned test rows (Cook.device_valid / device_test) -> (n,) float32 device tensor.
         Consecutive rows with the same user, mask and history form one impression of lstur_score_impressions (one user
         vector; split where it exceeds the plan's rows * candidates), every document is encoded once."""
-        import ctypes
         import torch
-        from .. import _lib, intern
+        from .. import intern
         assert not self.is_train and x.cand_doc.shape[1] == 1, 'device scoring is the one-candidate test model'
         n = x.n
         starts = intern.group_rows(x.user, x.mask, x.hist_doc)
         sizes = np.diff(np.append(starts, n))
         C = int(min(32, max(1, np.ceil(sizes.mean())))) if n else 1
-        eng = self.owner.engine(self.owner.predict_rows, C, training=False)
+        eng = self.core.engine_infer(C)
         cap = eng.B * eng.C
         pieces = np.concatenate([np.arange(a, a + k, cap) for a, k in zip(starts, sizes)]) if n else np.zeros(0, np.int64)
         off = np.append(pieces, n).astype(np.int32)
@@ -205,23 +209,20 @@ class CookModel:
         if n == 0:
             return out
         pos = torch.as_tensor(pieces.astype(np.int32)).to(dev)
-        user = torch.empty(P, dtype=torch.int32, device=dev)
-        scale = torch.empty(P, dtype=torch.float32, device=dev)
-        hist = torch.empty((P, W), dtype=torch.int32, device=dev)
-        p = lambda t: ctypes.c_void_p(None if t is None else t.data_ptr())
-        _lib.check(eng.lib.lstur_gather_samples(P, P, W, 0, p(pos), p(x.user), p(x.mask), p(x.hist_doc), None, None,
-                                                p(user), p(scale), p(hist), None, None, eng._stream()))
-        two = self.owner.config.arch in ('inigru', 'inagru')        # the second table's Dropout sees the same mask
-        return eng.score_impressions(user, hist, off, x.cand_doc.reshape(-1), eng.eval_doc_table(), out=out,
-                                     user_scale=scale, user_scale2=scale if two else None)
+        g = dict(user=torch.empty(P, dtype=torch.int32, device=dev), scale=torch.empty(P, dtype=torch.float32, device=dev),
+                 hist_doc=torch.empty((P, W), dtype=torch.int32, device=dev))
+        intern.gather_samples(pos, P, dict(user=x.user, scale=x.mask, hist_doc=x.hist_doc), g)
+        two = self.owner.config.arch in TWO_ID_ARCHS        # the second table's Dropout sees the same mask
+        return eng.score_impressions(g['user'], g['hist_doc'], off, x.cand_doc.reshape(-1), eng.eval_doc_table(), out=out,
+                                     user_scale=g['scale'], user_scale2=g['scale'] if two else None)
 
     def predict(self, x, batch_size=None, verbose=0, **_):
         if isinstance(x, CookDeviceData):
             return self._predict_device(x).cpu().numpy().reshape(-1, 1)
         n = len(np.asarray(x[0]))
         C = np.asarray(x[5]).shape[1] if self.is_train else 1
-        R = self.owner.predict_rows
-        eng = self.owner.engine(R, C, training=False)
+        eng = self.core.engine_infer(C)
+        R = eng.B
         out = np.zeros((n, C), dtype=np.float32)
         for s in range(0, n, R):
             rows = np.arange(s, min(n, s + R))
@@ -238,18 +239,13 @@ class CookModel:
         y = np.asarray(y[0] if isinstance(y, (list, tuple)) else y, dtype=np.float64)
         p = self.predict(x).astype(np.float64)          # interned rows: one read-back of the scores
         if self.is_train:
-            q = np.clip(p / p.sum(-1, keepdims=True), 1e-7, 1 - 1e-7)
-            return [float((-(y * np.log(q)).sum(-1)).mean()), float((p.argmax(1) == y.argmax(1)).mean())]
+            return keras_like.categorical_loss_accuracy(p, y)
         q, yy = np.clip(p.reshape(-1), 1e-7, 1 - 1e-7), y.reshape(-1)     # binary_crossentropy + utils.auc_roc
         return [float(-(yy * np.log(q) + (1 - yy) * np.log(1 - q)).mean()), metrics.auc_roc(q, yy)]
 
-    def get_weights_dict(self):
-        return self.owner.current_params()
 
-    def summary(self):
-        w = self.owner.current_params()
-        print('\n'.join('%-12s %-18s %d' % (k, tuple(np.asarray(v).shape), np.asarray(v).size) for k, v in w.items()))
-        print('Total params: %d' % sum(np.asarray(v).size for v in w.values()))
+def _core_attr(name):
+    return property(lambda self: getattr(self._core, name), lambda self, v: setattr(self._core, name, v))
 
 
 class Cook:
@@ -261,9 +257,7 @@ class Cook:
         logging.info('[+] loading testing data')
         self.test_data = dict(np.load(self.config.test_npz_input))
         logging.info('[-] loaded testing data')
-        self.predict_rows = 256
-        self._train_engine, self._infer = None, {}
-        self._doc_table, self._device_data = None, None
+        self._device_data = None
 
     def train(self):
         return [self.training_data[x] for x in FEATURES], [self.training_data[x] for x in ['cd_label']]
@@ -279,7 +273,7 @@ class Cook:
     def _interned(self):
         """Intern the titles of both files into one document table (once; needs the built model, whose vertical
         embeddings decide whether the vertical / subvertical ids are part of the key) and keep each file's rows on the
-        device as CookDeviceData.  The engines are rebuilt on the table (Cook.engine)."""
+        device as CookDeviceData.  The engines are rebuilt on the table (keras_like._Core.set_doc_table)."""
         import torch
         from .. import intern
         if self._device_data is None:
@@ -289,7 +283,8 @@ class Cook:
             for d in (self.training_data, self.test_data):
                 for t in ('ch', 'cd'):
                     parts.append((d[t + '_title'], d[t + '_vert'] if self.dv else None, d[t + '_subvert'] if self.ds else None))
-            ids, self._doc_table = intern.intern(parts, self.L, dev)
+            ids, table = intern.intern(parts, self.L, dev)
+            self._core.set_doc_table(**table)
             out = {}
             for i, (name, d) in enumerate((('train', self.training_data), ('test', self.test_data))):
                 hist, cand = ids[2 * i], ids[2 * i + 1]
@@ -327,18 +322,13 @@ class Cook:
             y_pred = self.test_model.predict(feature, batch_size=batch_size or self.config.batch_size).reshape(-1)
             res = evaluation.aggregate(users, imprs, np.asarray(mask).reshape(-1), y_true, y_pred)
         else:
-            import ctypes
             import torch
-            from .. import _lib
             x, (users, imprs, mask, y_true) = self.device_test()
             scores = self.test_model._predict_device(x)
             starts, ends = evaluation.impression_bounds(users, imprs)
-            m = torch.empty((len(starts), 4), dtype=torch.float32, device=scores.device)
-            if len(starts):             # the closed impressions are contiguous from row 0
-                off = torch.as_tensor(np.append(starts, ends[-1]).astype(np.int32)).to(scores.device)
-                p = lambda t: ctypes.c_void_p(t.data_ptr())
-                _lib.check(_lib.load().lstur_ranking_metrics(len(starts), p(off), p(scores), p(x.label), p(m),
-                                                             ctypes.c_void_p(torch.cuda.current_stream(scores.device).cuda_stream)))
+            # the closed impressions are contiguous from row 0
+            off = np.append(starts, ends[-1] if len(ends) else 0).astype(np.int32)
+            m = metrics.device_ranking_metrics(torch.as_tensor(off).to(scores.device), scores, x.label)
             res = evaluation.aggregate_metrics(users, np.asarray(mask).reshape(-1), y_true, starts, ends, m.cpu().numpy())
         evaluation.log_aggregate(res, log or utils.logging_evaluation)
         return res
@@ -376,48 +366,26 @@ class Cook:
             P.pop('vert_emb', None)
         if not self.ds:
             P.pop('subvert_emb', None)
-        self.params = P
-        self.optimizer = keras_like.Adam(c.learning_rate)
+        self._core = keras_like._Core(P, c, None, True, c.arch, score_model=c.score_model, flavour='cook', W=self.W,
+                                      L=self.L, n_cand=self.training_data['cd_title'].shape[1])
+        self.optimizer = self._core.optimizer             # callback decays the learning rate the engines read
         self.train_model = CookModel(self, True)
         self.test_model = CookModel(self, False)
         self.title_encoder = None
 
-    def current_params(self):
-        return self._train_engine.get_weights_dict() if self._train_engine is not None else self.params
+    # the core's weights, plan rows and engines under the handler's names
+    params = _core_attr('params')
+    predict_rows = _core_attr('predict_rows')
 
-    def _precision(self):
-        p = getattr(self.config, 'precision', 'auto')
-        if p != 'auto':
-            return p
-        from .. import _lib
-        ks, E, F = self.params['conv_w'].shape
-        return 'fp16_tc' if _lib.load().lstur_tc_supported(self.L, E, F, ks) else 'fp32'
+    def current_params(self):
+        return self.train_model.get_weights_dict()
 
     def engine(self, B, C, training):
-        c = self.config
-        kw = dict(arch=c.arch, flavour='cook', recurrent_activation=c.recurrent_activation, score_model=c.score_model,
-                  precision=self._precision())
-        e = self._train_engine
-        table = self._doc_table or {}
-        stale = e is not None and self._doc_table is not None and e.doc_tokens is not table['doc_tokens']
-        if training or e is None or stale:
-            if e is None or stale or ((e.B != B or e.C != C) and training):
-                tB, tC = (e.B, e.C) if e is not None and not training else (B, C)     # a rebuild on the table keeps its shape
-                if e is not None:
-                    self.params = e.get_weights_dict()
-                self._train_engine = LsturEngine(self.params, tB, self.W, tC, self.L, dropout=c.dropout, lr=c.learning_rate,
-                                                 training=True, sparse_user_adam=bool(c.sparse_user_adam),
-                                                 trainable_word_emb=bool(c.textual_embedding_trainable), **table, **kw)
-                if e is not None:
-                    self._train_engine.adopt_state_from(e)      # keep Adam moments / step count / dropout seed counter
-                self._infer = {}
-            if training:
-                return self._train_engine
-        key = (B, C)
-        if key not in self._infer:
-            self._infer[key] = LsturEngine(self.params, B, self.W, C, self.L, dropout=0.0, training=False,
-                                           share_weights_from=self._train_engine, **kw)
-        return self._infer[key]
+        """the core's training engine of B rows, or its inference engine of B rows and C candidates"""
+        if training:
+            assert C == self._core.n_train_cand(), (C, self._core.n_train_cand())
+            return self._core.engine_train(B)
+        return self._core.engine_infer(C, rows=B)
 
     def callback(self, epoch):
         if epoch in self.config.lrd_on_epochs:             # task/cook.py:282-285

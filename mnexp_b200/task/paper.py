@@ -311,9 +311,8 @@ class Seq2VecPaperSoftmax(Seq2VecPaper):
         GPU by test_model's head -> (offsets (m + 1,), scores (offsets[-1],), labels (offsets[-1],)) device tensors; the
         candidates of impression i are entries offsets[i] .. offsets[i+1] in test_gen order, positives (label 1) first.
         Every document is encoded once, the user encoder runs once per impression (LsturEngine.score_impressions)."""
-        import ctypes
         import torch
-        from .. import _lib
+        from .. import assemble
         host, dev = self._uploaded_tables()
         m = min(int(n), len(host['eval_first_click']))
         off = host['eval_cand_off'][:m + 1]
@@ -323,34 +322,20 @@ class Seq2VecPaperSoftmax(Seq2VecPaper):
             self._eval_label = torch.as_tensor((rank < np.repeat(host['eval_npos'], sizes)).astype(np.float32)).to(
                 dev['eval_cand_off'].device)
         eng = self._eval_engine()
-        W = self.config.window_size
-        user = torch.empty(m, dtype=torch.int32, device=eng.device)
-        hist = torch.empty((m, W), dtype=torch.int32, device=eng.device)
-        pos = torch.empty((m, 1), dtype=torch.int32, device=eng.device)
         idx = torch.arange(m, dtype=torch.int32, device=eng.device)
         w = self._w_device()
-        p = lambda x: ctypes.c_void_p(None if x is None else x.data_ptr())
         # the history of impression i: the W stream entries before its first click (K = 0: no negatives are drawn)
-        _lib.check(eng.lib.lstur_assemble_samples(
-            m, W, 0, p(dev['eval_first_click']), p(dev['eval_first_click']), p(idx), p(dev['click_user']),
-            p(dev.get('click_time')), 0 if w is None else int(w[1]), p(dev['stream_off']), p(dev['stream_docs']),
-            p(dev['neg_off']), p(dev['neg_docs']), 0, 0, p(user), p(hist), p(pos), eng._stream()))
+        b = assemble.assemble_samples(dev, dev['eval_first_click'], dev['eval_first_click'], idx, self.config.window_size,
+                                      0, 0 if w is None else int(w[1]))
         table = eng.eval_doc_table()
-        scores = eng.score_impressions(user, hist, off, dev['eval_cand_docs'], table)
+        scores = eng.score_impressions(b['user'], b['hist_doc'], off, dev['eval_cand_docs'], table)
         P = int(off[-1])
         return dev['eval_cand_off'][:m + 1], scores[:P], self._eval_label[:P]
 
     def _device_rows(self, x):
-        import ctypes
-        import torch
-        from .. import _lib
         off, scores, labels = self.device_test(x)
-        n = int(off.numel()) - 1
-        out = torch.empty((n, 4), dtype=torch.float32, device=off.device)
-        if n:
-            _lib.check(_lib.load().lstur_ranking_metrics(
-                n, ctypes.c_void_p(off.data_ptr()), ctypes.c_void_p(scores.data_ptr()), ctypes.c_void_p(labels.data_ptr()),
-                ctypes.c_void_p(out.data_ptr()), ctypes.c_void_p(torch.cuda.current_stream(off.device).cuda_stream)))
+        out = metrics.device_ranking_metrics(off, scores, labels)
+        n = int(out.shape[0])
         host = self._host_tables()
         return out.cpu().numpy(), host['eval_npos'][:n].tolist(), np.diff(host['eval_cand_off'][:n + 1]).tolist()
 
@@ -606,7 +591,8 @@ class Seq2VecPaperSoftmaxDaysIdVert(Seq2VecPaperSoftmaxDaysId):
     def _build_model(self):
         super(Seq2VecPaperSoftmaxDaysIdVert, self)._build_model()
         self._core.has_vert = True
-        self._core.doc_vert = self.device_doc_vert()     # vertical ids of device batches (host batches carry their own)
+        # vertical ids of device batches (host batches carry their own)
+        self._core.set_doc_table(self._core.doc_tokens, self.device_doc_vert())
 
 
 def _to_categorical(ids, num_classes):
@@ -668,7 +654,8 @@ class Seq2VecPaperSoftmaxDaysIdVertSup(Seq2VecPaperSoftmaxDaysId):
 
     def _build_model(self):
         super(Seq2VecPaperSoftmaxDaysIdVertSup, self)._build_model()
-        self._core.doc_vert = self.device_doc_vert()     # vertical labels of device batches (host batches carry their own)
+        # vertical labels of device batches (host batches carry their own)
+        self._core.set_doc_table(self._core.doc_tokens, self.device_doc_vert())
         layers = self.model.layers
         self.model = keras_like.VertSupModel(self._core, name='model')
         self.model.layers.update(layers)

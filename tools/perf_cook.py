@@ -73,7 +73,7 @@ def run(args, d):
     t_first, _ = timed(h._interned)
     parts = [(dd[t + '_title'], dd[t + '_vert'], dd[t + '_subvert']) for dd in (h.training_data, h.test_data) for t in ('ch', 'cd')]
     t_intern = [timed(intern.intern, parts, h.L)[0] for _ in range(args.reps)]
-    n_docs = int(h._doc_table['doc_tokens'].shape[0])
+    n_docs = int(h._core.doc_tokens.shape[0])
     print('interning: first call %.1f ms (with the upload), again %s ms; %d documents from %d rows'
           % (1e3 * t_first, ', '.join('%.1f' % (1e3 * t) for t in t_intern), n_docs,
              sum(int(np.prod(np.shape(p[0])[:-1])) for p in parts)))
